@@ -4,6 +4,7 @@ synthetic 1280x1280 pages, 1/2/4/8 GPUs).
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the reference algorithm on host cores
+    python bench.py ... --dump-outputs DIR                    # also writes the last timed step's items as DIR/*.npy
 
 One process per GPU (torchrun sets RANK / LOCAL_RANK / WORLD_SIZE for N > 1).  A *step* is one pass
 of the whole path (CRAFT -> post-process -> crop/resize -> PARSeq -> decode) over BASELINE configs[4]'s
@@ -168,11 +169,38 @@ class ClockSampler:
                     reasons=sorted(reasons), samples=len(sel), source=self.source)
 
 
-def ensure_weights():
-    """Seeded random-init weights of the named architectures (no checkpoints offline)."""
+def ensure_weights(out_dir):
+    """Seeded random-init weights of the named architectures (no checkpoints offline), written under `out_dir`: the
+    benchmark writes nothing into the source tree, which may be read-only."""
     from tuatara_b200 import weights
 
-    return weights.export_random(ROOT / "tests" / "_cache" / "weights_bench_seed0", seed=0)
+    return weights.export_random(Path(out_dir) / "weights_seed0", seed=0)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+TEXT_WIDTH = 26  # one character per PARSeq position at most
+
+
+def dump_outputs(out_dir, pages):
+    """Writes what one step returned to its caller, `pages` being per page a list of (text, bbox) items:
+    page_index.npy (which of this rank's pages are written), items_per_page.npy, bbox.npy [items, 4] and text.npy
+    [items, width] (latin-1 codes, zero-padded).  Above 64 MiB a seeded sample of whole pages is written instead."""
+    width = max([TEXT_WIDTH] + [len(t) for p in pages for t, _ in p])
+    page_bytes = max([len(p) for p in pages] + [1]) * (4 + width) * 4 + 16
+    idx = np.arange(len(pages))
+    if len(pages) * page_bytes > DUMP_LIMIT_BYTES:
+        k = max(1, DUMP_LIMIT_BYTES // page_bytes)
+        idx = np.sort(np.random.default_rng(0).choice(len(pages), k, replace=False))
+    items = [it for i in idx for it in pages[i]]
+    text = np.zeros((len(items), width), np.float32)
+    for r, (t, _) in enumerate(items):
+        text[r, :len(t)] = np.frombuffer(t, np.uint8)
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "page_index.npy", idx.astype(np.float64))
+    np.save(out / "items_per_page.npy", np.array([len(pages[i]) for i in idx], np.float64))
+    np.save(out / "bbox.npy", np.array([b for _, b in items], np.float32).reshape(-1, 4))
+    np.save(out / "text.npy", text)
 
 
 # ------------------------------------------------------------------------------ CPU reference arm
@@ -279,10 +307,9 @@ def run_native(args, rank, local_rank, world):
     if not _native.LIB_PATH.exists():
         build.build()
     lib = tb.lib()
-    wdir = ensure_weights() if rank == 0 else None
-    if world > 1:
-        dist.barrier()
-    wdir = ensure_weights()
+    import tempfile
+    tmp = tempfile.TemporaryDirectory(prefix="tuatara_bench_")
+    wdir = ensure_weights(tmp.name)
     cfg = tb.default_config()
     cfg.max_batch_pages = args.batch_pages
     cfg.slots_per_gpu = env_int("TT_SLOTS", 3)  # three execution slots per GPU (the library default)
@@ -307,11 +334,15 @@ def run_native(args, rank, local_rank, world):
         opt = _native.tt_ocr_options(int(on_dev), 1, ptrs, int(detect_only))
         h = (engine or eng)._h
 
-        def call():
+        def call(keep=None):
+            """-> the number of items; with a list `keep`, the result is appended to it instead of freed."""
             res = C.POINTER(_native.tt_result)()
             tb.check(lib.tt_ocr_pages_ex(h, arr, k, C.byref(opt), C.byref(res)), "tt_ocr_pages_ex")
             items = sum(res.contents.pages[i].n_items for i in range(res.contents.n_pages))
-            lib.tt_result_free(res)
+            if keep is None:
+                lib.tt_result_free(res)
+            else:
+                keep.append(res)
             return items
         call.keep = (arr, ptrs, opt, tensors, maps)
         return call
@@ -329,7 +360,8 @@ def run_native(args, rank, local_rank, world):
     sampler = ClockSampler(local_rank)  # one nvidia-smi for the whole run (it needs ~1 s to start); windows are cut by time
     sampler.start()
 
-    def timed(step, steps, profile=False):
+    def timed(step, steps, profile=False, keep_last=None):
+        """keep_last: a list that receives the last step's result (read and freed after the timed region)."""
         barrier()
         w0 = datetime.now()
         l0 = tb.launch_count()
@@ -340,8 +372,8 @@ def run_native(args, rank, local_rank, world):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
         items = 0
-        for _ in range(steps):
-            items += step()
+        for i in range(steps):
+            items += step(keep_last if i == steps - 1 else None)
         e1.record(stream)
         barrier()
         ms = e0.elapsed_time(e1)
@@ -375,7 +407,13 @@ def run_native(args, rank, local_rank, world):
 
     for _ in range(args.warmup):
         step_dev()
-    r_dev = timed(step_dev, args.steps)                    # headline: 2 slots per GPU, kernels of two batches interleave
+    last = []
+    r_dev = timed(step_dev, args.steps, keep_last=last if args.dump_outputs else None)  # headline: all slots busy
+    if last:
+        res = last[0].contents
+        outputs = [[(res.pages[p].items[i].text, tuple(res.pages[p].items[i].bbox)) for i in range(res.pages[p].n_items)]
+                   for p in range(res.n_pages)]
+        lib.tt_result_free(last[0])
     step_host()
     r_host = timed(step_host, args.steps)                  # same through host buffers
     lib.tt_engine_set_slots(eng._h, 1)                     # roofline pass: one slot => kernels strictly serial, so the
@@ -508,9 +546,12 @@ def run_native(args, rank, local_rank, world):
         line["cpu_baseline"] = {"value": npg / sec, "unit": "pages/s", "cores": os.cpu_count(), "kind": "port",
                                 "sample": f"{npg} page (300 crops), oracle (torch CPU + cv2, upstream AR early exit per 4-crop chunk), torch threads {threads}, "
                                           "PARSeq chunks of 4 on 6 threads (tuatara.cpp:452-475), models pre-loaded"}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     if rank == 0:
         print(json.dumps(line), flush=True)
     eng.close()
+    tmp.cleanup()
     if world > 1:
         dist.destroy_process_group()
 
@@ -606,6 +647,8 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the configs #1/#2/#4 block and the engine_dp_check")
     ap.add_argument("--batch-pages", type=int, default=32)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the items the last headline step returned (rank 0's pages) "
+                    "as DIR/*.npy, for comparing the outputs of two builds")
     args = ap.parse_args()
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
     if args.impl == "reference":

@@ -1,6 +1,7 @@
 """The C-ABI library loads and exports every symbol include/tuatara_c.h declares; the C++ header
 compiles without OpenCV; pytuatara keeps the reference's module/function/keyword names.  No compute
 calls that need a GPU."""
+import os
 import re
 import subprocess
 import sys
@@ -30,15 +31,16 @@ def test_every_declared_symbol_is_exported(native_lib):
 
 
 def test_no_gpu_fails_loudly(native_lib, tmp_path):
-    """Without a CUDA device the product path must refuse, not fall back to anything."""
-    import torch
-
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    import tuatara_b200 as tb
-
-    with pytest.raises(tb.TuataraError, match="no CUDA device|cannot open|CUDA"):
-        tb.Engine(str(tmp_path))
+    """Without a CUDA device the product path must refuse, not fall back to anything.  The engine is created in a
+    child process that sees no device, so the refusal is checked on GPU machines too."""
+    code = ("import sys\nimport tuatara_b200 as tb\n"
+            "try:\n    tb.Engine(sys.argv[1])\n"
+            "except tb.TuataraError as e:\n    print(e)\n    raise SystemExit(0)\n"
+            "raise SystemExit('tt_engine_create succeeded without a device')\n")
+    r = subprocess.run([sys.executable, "-c", code, str(tmp_path)], cwd=ROOT, capture_output=True, text=True,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0, r.stdout + r.stderr
+    assert re.search("no CUDA device|cannot open|CUDA", r.stdout), r.stdout
 
 
 def test_product_never_imports_oracle():
