@@ -47,6 +47,15 @@ struct ImageView {  // 8-bit, 3 channels, row-major (what cv::imread / np.uint8[
   size_t step = 0;  // bytes per row; 0 = cols * channels
 };
 
+// An OutputItem with its scores (image_to_data_scored), all on a 0..1 scale; definitions at tt_item_scores.
+struct ScoredItem {
+  std::string text;
+  std::vector<float> bbox;               // [min_x, min_y, max_x, max_y]
+  float confidence = -1.f;               // word confidence; -1 when the word was not recognised
+  float detection_score = 0.f;           // the box's maximum normalised text score (>= text_threshold)
+  std::vector<float> char_confidence;    // one probability per character of text
+};
+
 namespace detail {
 inline tt_engine* engine_for(const std::string& weights_dir) {
   static std::mutex mu;
@@ -67,26 +76,39 @@ inline tt_engine* engine_for(const std::string& weights_dir) {
 }
 }  // namespace detail
 
+namespace detail {
+// The checks, soft failures and engine call shared by the batch entry points: nullptr after printing the reason.
+// opt == nullptr: plain tt_ocr_pages.
+inline tt_result* ocr_pages(const std::vector<ImageView>& images, const std::string& weights_dir,
+                            const std::string& outputs_dir, const tt_ocr_options* opt) {
+  if (weights_dir.empty()) { std::cerr << "Please provide a value for weights_dir" << std::endl; return nullptr; }
+  if (outputs_dir.empty()) { std::cerr << "Please provide a value for outputs_dir" << std::endl; return nullptr; }
+  std::vector<tt_image> pages(images.size());
+  for (size_t i = 0; i < images.size(); ++i) {
+    const ImageView& v = images[i];
+    if (!v.data || v.rows <= 0 || v.cols <= 0) { std::cerr << "Error reading image from file"; return nullptr; }
+    pages[i] = tt_image{v.data, v.rows, v.cols, v.channels, v.step ? v.step : static_cast<size_t>(v.cols) * v.channels};
+  }
+  tt_engine* e = engine_for(weights_dir);
+  if (!e) { std::cerr << "error loading the models: " << tt_last_error() << std::endl; return nullptr; }
+  tt_result* r = nullptr;
+  const int rc = opt ? tt_ocr_pages_ex(e, pages.data(), static_cast<int>(pages.size()), opt, &r)
+                     : tt_ocr_pages(e, pages.data(), static_cast<int>(pages.size()), &r);
+  if (rc != 0) {
+    std::cerr << "tuatara: " << tt_last_error() << std::endl;
+    return nullptr;
+  }
+  return r;
+}
+}  // namespace detail
+
 // Additive batch API: many pages in one call, spread over the engine's GPUs (all visible ones, or TT_DEVICES).
 inline std::vector<std::vector<OutputItem>> image_to_data_batch(const std::vector<ImageView>& images,
                                                                 const std::string& weights_dir,
                                                                 const std::string& outputs_dir) {
   std::vector<std::vector<OutputItem>> out;
-  if (weights_dir.empty()) { std::cerr << "Please provide a value for weights_dir" << std::endl; return out; }
-  if (outputs_dir.empty()) { std::cerr << "Please provide a value for outputs_dir" << std::endl; return out; }
-  std::vector<tt_image> pages(images.size());
-  for (size_t i = 0; i < images.size(); ++i) {
-    const ImageView& v = images[i];
-    if (!v.data || v.rows <= 0 || v.cols <= 0) { std::cerr << "Error reading image from file"; return out; }
-    pages[i] = tt_image{v.data, v.rows, v.cols, v.channels, v.step ? v.step : static_cast<size_t>(v.cols) * v.channels};
-  }
-  tt_engine* e = detail::engine_for(weights_dir);
-  if (!e) { std::cerr << "error loading the models: " << tt_last_error() << std::endl; return out; }
-  tt_result* r = nullptr;
-  if (tt_ocr_pages(e, pages.data(), static_cast<int>(pages.size()), &r) != 0) {
-    std::cerr << "tuatara: " << tt_last_error() << std::endl;
-    return out;
-  }
+  tt_result* r = detail::ocr_pages(images, weights_dir, outputs_dir, nullptr);
+  if (!r) return out;
   out.resize(r->n_pages);
   for (int p = 0; p < r->n_pages; ++p)
     for (int k = 0; k < r->pages[p].n_items; ++k) {
@@ -95,6 +117,42 @@ inline std::vector<std::vector<OutputItem>> image_to_data_batch(const std::vecto
     }
   tt_result_free(r);
   return out;
+}
+
+// image_to_data_batch with scores: same items (text, bbox) and the same soft failures, plus each item's scores.
+inline std::vector<std::vector<ScoredItem>> image_to_data_scored_batch(const std::vector<ImageView>& images,
+                                                                       const std::string& weights_dir,
+                                                                       const std::string& outputs_dir) {
+  std::vector<std::vector<ScoredItem>> out;
+  tt_ocr_options opt = {};
+  opt.with_scores = 1;
+  tt_result* r = detail::ocr_pages(images, weights_dir, outputs_dir, &opt);
+  if (!r) return out;
+  out.resize(r->n_pages);
+  for (int p = 0; p < r->n_pages; ++p)
+    for (int k = 0; k < r->pages[p].n_items; ++k) {
+      const tt_item& it = r->pages[p].items[k];
+      ScoredItem s;
+      s.text = it.text;
+      s.bbox.assign(it.bbox, it.bbox + 4);
+      const float* cc = nullptr;
+      int n = 0;
+      if (tt_item_scores(r, p, k, &s.confidence, &s.detection_score, &cc, &n) != 0) {
+        std::cerr << "tuatara: " << tt_last_error() << std::endl;
+        tt_result_free(r);
+        return std::vector<std::vector<ScoredItem>>{};
+      }
+      if (n > 0) s.char_confidence.assign(cc, cc + n);
+      out[p].push_back(s);
+    }
+  tt_result_free(r);
+  return out;
+}
+
+inline std::vector<ScoredItem> image_to_data_scored(const ImageView& image, const std::string& weights_dir,
+                                                    const std::string& outputs_dir) {
+  std::vector<std::vector<ScoredItem>> pages = image_to_data_scored_batch({image}, weights_dir, outputs_dir);
+  return pages.empty() ? std::vector<ScoredItem>{} : pages[0];
 }
 
 }  // namespace tuatara

@@ -97,9 +97,21 @@ typedef struct tt_ocr_options {
   const float* const* score_override;
   int detect_only;   /* 1: stop after the word boxes (tuatara.cpp:349-418): items carry bbox and an empty text
                         (BASELINE config "CRAFT detection only") */
+  int with_scores;   /* 1: the result also holds per-item scores, read with tt_item_scores (0: none, the default) */
 } tt_ocr_options;
 TT_API int tt_ocr_pages_ex(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt, tt_result** out);
 TT_API void tt_result_free(tt_result* r);
+/* Scores of item `item` of page `page` of a result made with tt_ocr_options.with_scores = 1 (an error otherwise).
+ * Scale 0..1.  p[t] is the largest softmax probability of the refinement logits at position t (t = 0..25), the
+ * position's id being its argmax; the end position e is the first t whose id is 0 (where the text stops), else 25.
+ *  conf       = p[0] * ... * p[e] (the end position and positions of id 88 included), multiplied in double and
+ *               rounded once to float; may underflow to 0.  -1 when the item was not recognised (detect_only).
+ *  det_score  = the component's maximum normalised text score (tuatara.cpp:151-152), >= text_threshold.
+ *  char_conf  = p[t] of each position that produced a character of the item's text, in order (*n_chars == strlen(text));
+ *               memory owned by the result, valid until tt_result_free.  NULL (and 0) when not recognised.
+ * Every output pointer may be NULL. */
+TT_API int tt_item_scores(const tt_result* r, int page, int item, float* conf, float* det_score, const float** char_conf,
+                          int* n_chars);
 /* Kernel launches issued by this library so far (bench.py's gpu_launches). */
 TT_API unsigned long long tt_launch_count(void);
 
@@ -161,8 +173,15 @@ TT_API int tt_rect_to_quad(const float rect[5], float quad_out[8]);
  * logits_out (nullable) [n][26][95] fp32; ids_out (nullable) [n][26] argmax (== softmax + max, :486,:103). */
 TT_API int tt_parseq_forward(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens, float* logits_out,
                       int32_t* ids_out);
+/* tt_parseq_forward's ids together with pmax_out [n][26]: the largest softmax probability of the refinement logits at
+ * each position (the p[t] of tt_item_scores), from the same kernel that picks the ids.  ids_out [n][26]. */
+TT_API int tt_parseq_forward_scores(tt_engine* e, const uint8_t* crops, int n, int32_t* ids_out, float* pmax_out);
 /* Tokenizer::decode + truncation (tuatara.cpp:61-116, :497-502). ids [n][len]; out [n][out_stride] chars. */
 TT_API int tt_decode(const int32_t* ids, int n, int len, char* out, int out_stride);
+/* tt_decode with the scores of tt_item_scores (host only).  pmax [n][len]; conf_out (nullable) [n];
+ * char_conf_out (nullable) [n][len]: row i starts with the char_conf of string i, the rest of the row is 0. */
+TT_API int tt_decode_scores(const int32_t* ids, const float* pmax, int n, int len, char* out, int out_stride, float* conf_out,
+                            float* char_conf_out);
 /* itos_out: >= 99 bytes. */
 TT_API int tt_tokenizer_table(char* itos_out, int* eos_id, int* bos_id, int* pad_id);
 

@@ -16,8 +16,8 @@ from . import _native
 from ._native import TuataraError, check, lib, ptr
 
 __all__ = [
-    "TuataraError", "Engine", "image_to_data", "images_to_data", "default_config", "resize_plan", "preprocess",
-    "postprocess", "crop_resize", "decode_ids", "tokenizer_table", "min_area_rect", "convex_hull",
+    "TuataraError", "Engine", "image_to_data", "images_to_data", "image_to_data_scored", "images_to_data_scored",
+    "default_config", "resize_plan", "preprocess", "postprocess", "crop_resize", "decode_ids", "decode_scores", "tokenizer_table", "min_area_rect", "convex_hull",
     "rect_points", "rect_bounding", "adjust_rect", "rect_to_bbox", "launch_count",
 ]
 
@@ -54,6 +54,22 @@ def decode_ids(ids: np.ndarray) -> list[str]:
     out = np.zeros((n, 64), np.uint8)
     check(lib().tt_decode(ptr(ids), n, ln, ptr(out), 64), "tt_decode")
     return [bytes(row).split(b"\0", 1)[0].decode("latin-1") for row in out]
+
+
+def decode_scores(ids: np.ndarray, pmax: np.ndarray):
+    """decode_ids with scores (host only): ids int32 [n, len], pmax float32 [n, len] (the largest softmax probability
+    per position) -> (texts, conf float32 [n], char_conf: list of float32 arrays, one value per character)."""
+    ids = np.ascontiguousarray(ids, np.int32)
+    pmax = np.ascontiguousarray(pmax, np.float32)
+    n, ln = ids.shape
+    if pmax.shape != ids.shape:
+        raise ValueError("decode_scores: ids and pmax differ in shape")
+    out = np.zeros((n, 64), np.uint8)
+    conf = np.empty(n, np.float32)
+    cc = np.empty((n, ln), np.float32)
+    check(lib().tt_decode_scores(ptr(ids), ptr(pmax), n, ln, ptr(out), 64, ptr(conf), ptr(cc)), "tt_decode_scores")
+    texts = [bytes(row).split(b"\0", 1)[0].decode("latin-1") for row in out]
+    return texts, conf, [cc[i, :len(t)].copy() for i, t in enumerate(texts)]
 
 
 def convex_hull(points: np.ndarray) -> np.ndarray:
@@ -193,10 +209,13 @@ class Engine:
 
     __del__ = close
 
-    def ocr_pages(self, images: list, score_override: list | None = None, detect_only: bool = False) -> list[list[dict]]:
+    def ocr_pages(self, images: list, score_override: list | None = None, detect_only: bool = False,
+                  scores: bool = False) -> list[list[dict]]:
         """images: uint8 [H,W,3] numpy arrays (host) or torch CUDA tensors (already on the device).
         score_override: optional per-page float32 [h32/2, w32/2, 2] maps (numpy or CUDA tensors, or
-        None entries) that replace CRAFT's output after CRAFT has run (benchmark / parity tests)."""
+        None entries) that replace CRAFT's output after CRAFT has run (benchmark / parity tests).
+        scores: every item also carries conf (word confidence 0..1, None when not recognised), det_score (the
+        detection score of its box) and char_conf (one probability per character of text); see tt_item_scores."""
         n = len(images)
         on_dev = n > 0 and not isinstance(images[0], np.ndarray)
         if on_dev:
@@ -206,7 +225,7 @@ class Engine:
         arr = (_native.tt_image * n)(*structs)
         if n and any(isinstance(im, np.ndarray) == on_dev for im in images):
             raise TuataraError("ocr_pages: host and device pages cannot be mixed in one call")
-        opt = _native.tt_ocr_options(int(on_dev), 0, None, int(detect_only))
+        opt = _native.tt_ocr_options(int(on_dev), 0, None, int(detect_only), int(scores))
         keep = []
         if score_override is not None:
             ov_dev = any(m is not None and not isinstance(m, np.ndarray) for m in score_override)
@@ -229,6 +248,9 @@ class Engine:
                 page = res.contents.pages[p]
                 out.append([dict(text=page.items[i].text.decode("latin-1"), bbox=[float(v) for v in page.items[i].bbox])
                             for i in range(page.n_items)])
+                if scores:
+                    for i, item in enumerate(out[-1]):
+                        item.update(_item_scores(res, p, i))
             return out
         finally:
             lib().tt_result_free(res)
@@ -249,6 +271,16 @@ class Engine:
         check(lib().tt_craft_tap(self._h, name.encode(), ptr(out), out.size, dims), "tt_craft_tap")
         return out
 
+    def parseq_forward_scores(self, crops_u8: np.ndarray):
+        """crops_u8: uint8 [n, 32, 128, 3] -> (ids int32 [n, 26], pmax float32 [n, 26]): parseq_forward's ids and the
+        largest softmax probability of the refinement logits at each position."""
+        x = np.ascontiguousarray(crops_u8, np.uint8)
+        n = x.shape[0]
+        ids = np.empty((n, 26), np.int32)
+        pmax = np.empty((n, 26), np.float32)
+        check(lib().tt_parseq_forward_scores(self._h, ptr(x), n, ptr(ids), ptr(pmax)), "tt_parseq_forward_scores")
+        return ids, pmax
+
     def parseq_forward(self, crops_u8: np.ndarray, forced_tokens: np.ndarray | None = None):
         """crops_u8: uint8 [n, 32, 128, 3] -> (logits float32 [n, 26, 95], ids int32 [n, 26])."""
         x = np.ascontiguousarray(crops_u8, np.uint8)
@@ -258,6 +290,14 @@ class Engine:
         ft = None if forced_tokens is None else np.ascontiguousarray(forced_tokens, np.int32)
         check(lib().tt_parseq_forward(self._h, ptr(x), n, ptr(ft), ptr(logits), ptr(ids)), "tt_parseq_forward")
         return logits, ids
+
+
+def _item_scores(res, page: int, item: int) -> dict:
+    conf, det = C.c_float(), C.c_float()
+    cc, n = C.POINTER(C.c_float)(), C.c_int()
+    check(lib().tt_item_scores(res, page, item, C.byref(conf), C.byref(det), C.byref(cc), C.byref(n)), "tt_item_scores")
+    return dict(conf=None if conf.value < 0 else conf.value, det_score=det.value,
+                char_conf=[cc[k] for k in range(n.value)])
 
 
 _engines: dict = {}
@@ -292,3 +332,25 @@ def image_to_data(image: np.ndarray, weights_dir: str, outputs_dir: str) -> list
 def images_to_data(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".") -> list[list[dict]]:
     """Additive batch API: one call, many pages (sharded over the engine's GPUs)."""
     return _engine_for(weights_dir).ocr_pages(list(images))
+
+
+def image_to_data_scored(image: np.ndarray, weights_dir: str, outputs_dir: str) -> list[dict]:
+    """image_to_data whose items also carry ``conf`` (word confidence 0..1), ``det_score`` (the detection score of the
+    box) and ``char_conf`` (one probability per character of ``text``).  Same inputs, errors and soft failures;
+    ``text`` and ``bbox`` are what image_to_data returns."""
+    import sys
+
+    if not weights_dir:
+        print("Please provide a value for weights_dir", file=sys.stderr)
+        return []
+    if not outputs_dir:
+        print("Please provide a value for outputs_dir", file=sys.stderr)
+        return []
+    if image.ndim != 3:
+        raise RuntimeError("Input array should have 3 dimensions")
+    return _engine_for(weights_dir).ocr_pages([image], scores=True)[0]
+
+
+def images_to_data_scored(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".") -> list[list[dict]]:
+    """Batch variant of image_to_data_scored."""
+    return _engine_for(weights_dir).ocr_pages(list(images), scores=True)

@@ -30,7 +30,7 @@ class tt_config(C.Structure):
 
 class tt_ocr_options(C.Structure):
     _fields_ = [("pages_on_device", C.c_int), ("override_on_device", C.c_int),
-                ("score_override", C.POINTER(C.c_void_p)), ("detect_only", C.c_int)]
+                ("score_override", C.POINTER(C.c_void_p)), ("detect_only", C.c_int), ("with_scores", C.c_int)]
 
 
 class tt_item(C.Structure):
@@ -61,6 +61,7 @@ SIGNATURES = {
     "tt_ocr_pages": (_I, [_P, C.POINTER(tt_image), _I, C.POINTER(C.POINTER(tt_result))]),
     "tt_ocr_pages_ex": (_I, [_P, C.POINTER(tt_image), _I, C.POINTER(tt_ocr_options), C.POINTER(C.POINTER(tt_result))]),
     "tt_result_free": (None, [C.POINTER(tt_result)]),
+    "tt_item_scores": (_I, [C.POINTER(tt_result), _I, _I, _PF, _PF, C.POINTER(_PF), _PI]),
     "tt_launch_count": (C.c_ulonglong, []),
     "tt_engine_set_slots": (None, [_P, _I]),
     "tt_engine_stream": (_P, [_P, _I]),
@@ -79,7 +80,9 @@ SIGNATURES = {
     "tt_crop_warp": (_I, [C.POINTER(tt_image), _P, _I, _P]),
     "tt_rect_to_quad": (_I, [_P, _P]),
     "tt_parseq_forward": (_I, [_P, _P, _I, _P, _P, _P]),
+    "tt_parseq_forward_scores": (_I, [_P, _P, _I, _P, _P]),
     "tt_decode": (_I, [_P, _I, _I, _P, _I]),
+    "tt_decode_scores": (_I, [_P, _P, _I, _I, _P, _I, _P, _P]),
     "tt_tokenizer_table": (_I, [C.c_char_p, _PI, _PI, _PI]),
     "tt_convex_hull_i32": (_I, [_P, _I, _P, _PI]),
     "tt_convex_hull_f32": (_I, [_P, _I, _P, _PI]),

@@ -31,6 +31,17 @@ static py::dict output_item_to_dict(const OutputItem& item) {  // python.cpp:36-
   return d;
 }
 
+// conf is None for a word that was not recognised (ScoredItem::confidence == -1)
+static py::dict scored_item_to_dict(const tuatara::ScoredItem& item) {
+  py::dict d;
+  d["text"] = item.text;
+  d["bbox"] = item.bbox;
+  d["conf"] = item.confidence < 0.f ? py::object(py::none()) : py::object(py::float_(item.confidence));
+  d["det_score"] = item.detection_score;
+  d["char_conf"] = item.char_confidence;
+  return d;
+}
+
 static py::list image_to_data_wrapper(py::array_t<unsigned char, py::array::c_style | py::array::forcecast> image_data,
                                       std::string weights_dir, std::string output_dir) {
   const tuatara::ImageView img = buffer_to_view(image_data);
@@ -62,10 +73,45 @@ static py::list images_to_data_wrapper(std::vector<py::array_t<unsigned char, py
   return result;
 }
 
+static py::list image_to_data_scored_wrapper(py::array_t<unsigned char, py::array::c_style | py::array::forcecast> image_data,
+                                             std::string weights_dir, std::string output_dir) {
+  const tuatara::ImageView img = buffer_to_view(image_data);
+  std::vector<tuatara::ScoredItem> items;
+  {
+    py::gil_scoped_release release;
+    items = tuatara::image_to_data_scored(img, weights_dir, output_dir);
+  }
+  py::list result;
+  for (const auto& item : items) result.append(scored_item_to_dict(item));
+  return result;
+}
+
+static py::list images_to_data_scored_wrapper(std::vector<py::array_t<unsigned char, py::array::c_style | py::array::forcecast>> images,
+                                              std::string weights_dir, std::string output_dir) {
+  std::vector<tuatara::ImageView> views;
+  for (auto& a : images) views.push_back(buffer_to_view(a));
+  std::vector<std::vector<tuatara::ScoredItem>> pages;
+  {
+    py::gil_scoped_release release;
+    pages = tuatara::image_to_data_scored_batch(views, weights_dir, output_dir);
+  }
+  py::list result;
+  for (const auto& page : pages) {
+    py::list items;
+    for (const auto& item : page) items.append(scored_item_to_dict(item));
+    result.append(items);
+  }
+  return result;
+}
+
 PYBIND11_MODULE(pytuatara, m) {
   m.doc() = "Tuatara ocr";
   m.def("image_to_data", &image_to_data_wrapper, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"),
         "Extract text and bounding boxes from an image");
   m.def("images_to_data", &images_to_data_wrapper, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"),
         "Batch variant: list of images -> list of per-page results");
+  m.def("image_to_data_scored", &image_to_data_scored_wrapper, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"),
+        "image_to_data whose items also carry conf (word confidence 0..1, None when not recognised), det_score and char_conf");
+  m.def("images_to_data_scored", &images_to_data_scored_wrapper, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"),
+        "Batch variant of image_to_data_scored");
 }

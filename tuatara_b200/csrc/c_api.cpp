@@ -251,6 +251,27 @@ int tt_decode(const int32_t* ids, int n, int len, char* out, int out_stride) {
   });
 }
 
+int tt_decode_scores(const int32_t* ids, const float* pmax, int n, int len, char* out, int out_stride, float* conf_out,
+                     float* char_conf_out) {
+  return guarded([&]() -> int {
+    std::string s;
+    std::vector<float> cc;
+    for (int i = 0; i < n; ++i) {
+      float conf = 0.f;
+      decode_ids_scored(ids + static_cast<size_t>(i) * len, pmax + static_cast<size_t>(i) * len, len, &s, &cc, &conf);
+      if (static_cast<int>(s.size()) + 1 > out_stride) { set_error("tt_decode_scores: out_stride too small"); return 1; }
+      std::memcpy(out + static_cast<size_t>(i) * out_stride, s.c_str(), s.size() + 1);
+      if (conf_out) conf_out[i] = conf;
+      if (char_conf_out) {
+        float* row = char_conf_out + static_cast<size_t>(i) * len;
+        std::fill(row, row + len, 0.f);
+        std::copy(cc.begin(), cc.end(), row);
+      }
+    }
+    return 0;
+  });
+}
+
 int tt_tokenizer_table(char* itos_out, int* eos_id, int* bos_id, int* pad_id) {
   const TokenizerTable& t = tokenizer_table();
   std::memcpy(itos_out, t.itos.c_str(), t.itos.size() + 1);

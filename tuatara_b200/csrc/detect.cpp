@@ -18,7 +18,7 @@ bool collect_boxes(const uint8_t* block, int comp_cap, int row_cap, int H, int W
     if (!component_rect(ci, reinterpret_cast<const int*>(rows + c.row_off), W, H, cfg.min_area, cfg.text_threshold,
                         &rr, &scratch))
       continue;
-    out->push_back(DetBox{j + 1, rr});
+    out->push_back(DetBox{j + 1, rr, c.max_text});
   }
   return true;
 }

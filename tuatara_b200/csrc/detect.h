@@ -12,6 +12,7 @@ namespace tt {
 struct DetBox {
   int label;        // cv label of the component (1-based)
   RotatedRect rect; // in score-map coordinates
+  float score;      // the component's maximum normalised text score (>= text_threshold, tuatara.cpp:151-154)
 };
 
 // `block` = one page's result block copied from PostWorkspace::result (header | comps | rows).

@@ -44,6 +44,17 @@ constexpr int kCraftSubBatch = 8;   // pages per CRAFT / post-processing pass in
 struct PageOut {
   std::vector<std::string> text;
   std::vector<std::array<float, 4>> bbox;
+  // tt_ocr_options.with_scores only (empty otherwise); definitions at tt_item_scores
+  std::vector<float> det;                        // per item: the component's maximum normalised text score
+  std::vector<float> conf;                       // per item: word confidence, -1 until recognised
+  std::vector<std::vector<float>> char_conf;     // per item: one probability per character of text
+};
+
+// What tt_ocr_pages_ex returns: the public tt_result first (the caller only ever sees its address), the scores in a
+// block of their own so that tt_item / tt_page_result / tt_result keep their layout.
+struct ResultBlock {
+  tt_result r;
+  std::vector<PageOut>* scores;   // null without with_scores; text / bbox already copied into r
 };
 
 cudaError_t ensure_post(DeviceCtx& d, int batch, int H, int W, int comp_cap, int row_cap) {
@@ -190,6 +201,7 @@ int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const
       std::array<float, 4> bb;
       rect_to_bbox(adj, bb.data());
       po.bbox.push_back(bb);
+      if (opt.with_scores) po.det.push_back(db.score);
       const RectI r = rect_bounding(adj);  // the reference throws when this leaves the image; we clamp
       const int x0 = std::max(r.x, 0), y0 = std::max(r.y, 0);
       const int x1 = std::min(r.x + r.w, im.cols), y1 = std::min(r.y + r.h, im.rows);
@@ -204,6 +216,10 @@ int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const
       pend->owner.push_back(CropOwner{u.pages[b], k++});
     }
     po.text.resize(po.bbox.size());   // zero boxes: the reference crashes in torch::cat({}) (tuatara.cpp:485); we return no items
+    if (opt.with_scores) {
+      po.conf.assign(po.bbox.size(), -1.f);
+      po.char_conf.resize(po.bbox.size());
+    }
   }
   const int n = static_cast<int>(crops.size());
   if (opt.detect_only) {   // boxes only: nothing joins the recognition batch
@@ -236,28 +252,41 @@ int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const
   return 0;
 }
 
-// PARSeq + tokenizer over the slot's recognition batch (tuatara.cpp:450-505).
-int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend) {
+// PARSeq + tokenizer over the slot's recognition batch (tuatara.cpp:450-505).  scores: the refinement head also
+// writes each position's largest softmax probability, copied back next to the ids and decoded into conf / char_conf.
+int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, bool scores) {
   const int n = static_cast<int>(pend->owner.size());
   const int L = d.w->pd.L;
   for (int c0 = 0; c0 < n; c0 += kMaxCropsPerPass) {
     const int nc = std::min(kMaxCropsPerPass, n - c0);
-    const size_t need = d.parseq_bytes(nc) + (4u << 20);
+    const size_t bytes = sizeof(int) * static_cast<size_t>(nc) * L;   // ids; with scores as many bytes of pmax follow
+    const size_t need = d.parseq_bytes(nc) + (4u << 20) + (scores ? bytes : 0);
     if (need > d.arena.capacity()) E_TRY(stream_sync(d.stream));
     E_TRY(d.arena.reserve(need));
     d.arena.reset();
+    float* pmax = scores ? d.arena.get<float>(static_cast<size_t>(nc) * L) : nullptr;
+    if (scores && !pmax) { set_error("arena exhausted (pmax)"); return 1; }
     float* logits = nullptr;
     int* ids = nullptr;
-    E_TRY(d.parseq_forward(d.patch_buf + static_cast<size_t>(c0) * 128 * 96, nc, nullptr, &logits, &ids));
-    const size_t bytes = sizeof(int) * static_cast<size_t>(nc) * L;
-    E_TRY(d.ensure_pinned(bytes));
+    E_TRY(d.parseq_forward(d.patch_buf + static_cast<size_t>(c0) * 128 * 96, nc, nullptr, &logits, &ids, pmax));
+    E_TRY(d.ensure_pinned(scores ? 2 * bytes : bytes));
     E_CUDA(cudaMemcpyAsync(d.pinned, ids, bytes, cudaMemcpyDeviceToHost, d.stream));
     g_d2h_bytes += bytes;
+    if (scores) {
+      E_CUDA(cudaMemcpyAsync(d.pinned + bytes, pmax, bytes, cudaMemcpyDeviceToHost, d.stream));
+      g_d2h_bytes += bytes;
+    }
     E_TRY(stream_sync(d.stream));
     const int* host_ids = reinterpret_cast<const int*>(d.pinned);
+    const float* host_p = reinterpret_cast<const float*>(d.pinned + bytes);
     for (int c = 0; c < nc; ++c) {   // tokenizer (tuatara.cpp:492-505)
       const CropOwner& o = pend->owner[c0 + c];
-      (*results)[o.page].text[o.box] = decode_ids(host_ids + static_cast<size_t>(c) * L, L);
+      PageOut& po = (*results)[o.page];
+      if (scores)
+        decode_ids_scored(host_ids + static_cast<size_t>(c) * L, host_p + static_cast<size_t>(c) * L, L, &po.text[o.box],
+                          &po.char_conf[o.box], &po.conf[o.box]);
+      else
+        po.text[o.box] = decode_ids(host_ids + static_cast<size_t>(c) * L, L);
     }
   }
   pend->owner.clear();
@@ -303,9 +332,9 @@ void slot_worker(tt_engine& e, int g, int sidx, int want, const tt_image* pages,
   Pending pend;
   for (int ui = q->pop(g); ui >= 0; ui = q->pop(g)) {
     if (detect_unit(d, cfg, pages, q->units[ui], opt, results, &pend)) { *err = last_error(); *rc = 1; return; }
-    if (pend.pages >= max_b && recognise(d, results, &pend)) { *err = last_error(); *rc = 1; return; }
+    if (pend.pages >= max_b && recognise(d, results, &pend, opt.with_scores != 0)) { *err = last_error(); *rc = 1; return; }
   }
-  if (recognise(d, results, &pend)) { *err = last_error(); *rc = 1; return; }
+  if (recognise(d, results, &pend, opt.with_scores != 0)) { *err = last_error(); *rc = 1; return; }
 }
 
 }  // namespace
@@ -403,7 +432,7 @@ int tt_ocr_pages(tt_engine* e, const tt_image* pages, int n_pages, tt_result** o
 
 int tt_ocr_pages_ex(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt_in, tt_result** out) {
   try {
-    tt_ocr_options opt{0, 0, nullptr, 0};
+    tt_ocr_options opt{0, 0, nullptr, 0, 0};
     if (opt_in) opt = *opt_in;
     if (!e || !out) { set_error("tt_ocr_pages: null argument"); return 1; }
     if (n_pages < 0 || (n_pages > 0 && !pages)) { set_error("tt_ocr_pages: bad page array"); return 1; }
@@ -457,7 +486,8 @@ int tt_ocr_pages_ex(tt_engine* e, const tt_image* pages, int n_pages, const tt_o
     for (size_t w = 0; w < ws.size(); ++w)
       if (rcs[w]) { set_error("device " + std::to_string(e->devs[ws[w].g * kSlotsPerDevice]->device) + ": " + errs[w]); return 1; }
     // host-side gather into the C result
-    tt_result* r = new tt_result;
+    ResultBlock* rb = new ResultBlock{};
+    tt_result* r = &rb->r;
     r->n_pages = n_pages;
     r->pages = new tt_page_result[n_pages];
     for (int i = 0; i < n_pages; ++i) {
@@ -470,6 +500,13 @@ int tt_ocr_pages_ex(tt_engine* e, const tt_image* pages, int n_pages, const tt_o
         std::memcpy(pr.items[k].text, po.text[k].c_str(), po.text[k].size() + 1);
         std::memcpy(pr.items[k].bbox, po.bbox[k].data(), sizeof(float) * 4);
       }
+    }
+    if (opt.with_scores) {
+      for (PageOut& po : results) {   // only the scores are kept
+        po.text.clear();
+        po.bbox.clear();
+      }
+      rb->scores = new std::vector<PageOut>(std::move(results));
     }
     *out = r;
     return 0;
@@ -486,7 +523,27 @@ void tt_result_free(tt_result* r) {
     delete[] r->pages[i].items;
   }
   delete[] r->pages;
-  delete r;
+  ResultBlock* rb = reinterpret_cast<ResultBlock*>(r);   // r is its first member (tt_ocr_pages_ex)
+  delete rb->scores;
+  delete rb;
+}
+
+int tt_item_scores(const tt_result* r, int page, int item, float* conf, float* det_score, const float** char_conf,
+                   int* n_chars) {
+  if (!r) { set_error("tt_item_scores: null result"); return 1; }
+  const ResultBlock* rb = reinterpret_cast<const ResultBlock*>(r);
+  if (!rb->scores) { set_error("tt_item_scores: the result was made without tt_ocr_options.with_scores"); return 1; }
+  if (page < 0 || page >= r->n_pages || item < 0 || item >= r->pages[page].n_items) {
+    set_error("tt_item_scores: page or item out of range");
+    return 1;
+  }
+  const PageOut& po = (*rb->scores)[page];
+  const std::vector<float>& cc = po.char_conf[item];
+  if (conf) *conf = po.conf[item];
+  if (det_score) *det_score = po.det[item];
+  if (char_conf) *char_conf = cc.empty() ? nullptr : cc.data();
+  if (n_chars) *n_chars = static_cast<int>(cc.size());
+  return 0;
 }
 
 int tt_craft_forward(tt_engine* e, const uint8_t* craft_input, int h32, int w32, float* maps_out) {
@@ -536,8 +593,12 @@ int tt_craft_tap(tt_engine* e, const char* name, float* out, long long capacity,
   }
 }
 
-int tt_parseq_forward(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens, float* logits_out,
-                      int32_t* ids_out) {
+}  // extern "C"
+
+namespace {
+// tt_parseq_forward and tt_parseq_forward_scores (pmax_out != null: the refinement head also writes the probabilities)
+int parseq_stage(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens, float* logits_out,
+                 int32_t* ids_out, float* pmax_out) {
   try {
     if (!e) { set_error("tt_parseq_forward: null engine"); return 1; }
     if (n <= 0) return 0;
@@ -548,8 +609,10 @@ int tt_parseq_forward(tt_engine* e, const uint8_t* crops, int n, const int32_t* 
     for (int c0 = 0; c0 < n; c0 += kMaxCropsPerPass) {
       const int nc = std::min(kMaxCropsPerPass, n - c0);
       const size_t crop_bytes = static_cast<size_t>(nc) * 32 * 128 * 3;
-      E_TRY(d.arena.reserve(d.parseq_bytes(nc) + crop_bytes + static_cast<size_t>(nc) * (128 * 96 * 2 + 4 * L) + (8u << 20)));
+      E_TRY(d.arena.reserve(d.parseq_bytes(nc) + crop_bytes + static_cast<size_t>(nc) * (128 * 96 * 2 + 4 * L) + (8u << 20) +
+                            (pmax_out ? sizeof(float) * nc * L : 0)));
       d.arena.reset();
+      float* pmax = pmax_out ? d.arena.get<float>(static_cast<size_t>(nc) * L) : nullptr;
       uint8_t* cu8 = d.arena.get<uint8_t>(crop_bytes);
       __nv_bfloat16* patches = d.arena.get<__nv_bfloat16>(static_cast<size_t>(nc) * 128 * 96);
       int* forced = forced_tokens ? d.arena.get<int>(static_cast<size_t>(nc) * (L - 1)) : nullptr;
@@ -560,13 +623,15 @@ int tt_parseq_forward(tt_engine* e, const uint8_t* crops, int n, const int32_t* 
       E_TRY(patchify_u8(cu8, nc, patches, d.stream));
       float* logits = nullptr;
       int* ids = nullptr;
-      E_TRY(d.parseq_forward(patches, nc, forced, &logits, &ids));
+      E_TRY(d.parseq_forward(patches, nc, forced, &logits, &ids, pmax));
       if (logits_out)
         E_CUDA(cudaMemcpy2DAsync(logits_out + static_cast<size_t>(c0) * L * d.w->pd.n_cls, sizeof(float) * d.w->pd.n_cls, logits,
                                  sizeof(float) * NC, sizeof(float) * d.w->pd.n_cls, static_cast<size_t>(nc) * L,
                                  cudaMemcpyDeviceToHost, d.stream));
       if (ids_out)
         E_CUDA(cudaMemcpyAsync(ids_out + static_cast<size_t>(c0) * L, ids, sizeof(int) * nc * L, cudaMemcpyDeviceToHost, d.stream));
+      if (pmax_out)
+        E_CUDA(cudaMemcpyAsync(pmax_out + static_cast<size_t>(c0) * L, pmax, sizeof(float) * nc * L, cudaMemcpyDeviceToHost, d.stream));
       E_TRY(stream_sync(d.stream));
     }
     return 0;
@@ -574,6 +639,19 @@ int tt_parseq_forward(tt_engine* e, const uint8_t* crops, int n, const int32_t* 
     set_error(std::string("tt_parseq_forward: ") + ex.what());
     return 1;
   }
+}
+}  // namespace
+
+extern "C" {
+
+int tt_parseq_forward(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens, float* logits_out,
+                      int32_t* ids_out) {
+  return parseq_stage(e, crops, n, forced_tokens, logits_out, ids_out, nullptr);
+}
+
+int tt_parseq_forward_scores(tt_engine* e, const uint8_t* crops, int n, int32_t* ids_out, float* pmax_out) {
+  if (!pmax_out) { set_error("tt_parseq_forward_scores: null pmax_out"); return 1; }
+  return parseq_stage(e, crops, n, nullptr, nullptr, ids_out, pmax_out);
 }
 
 int tt_postprocess_dev(tt_engine* e, const float* maps_dev, int batch, int H, int W, int* n_rects_total, void*) {

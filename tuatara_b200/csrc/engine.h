@@ -108,9 +108,10 @@ struct DeviceCtx {
   // CRAFT: device u8 [B][H][W][3] (already swapped/padded) -> device fp32 maps [B][H/2][W/2][2] (arena memory)
   cudaError_t craft_forward(const uint8_t* input_dev, int B, int H, int W, float** maps_out);
   size_t craft_bytes(int B, int H, int W) const;
-  // PARSeq: device bf16 patches [n*128][96] -> device fp32 logits [n][L][n_cls_pad] + int ids [n][L] (arena)
+  // PARSeq: device bf16 patches [n*128][96] -> device fp32 logits [n][L][n_cls_pad] + int ids [n][L] (arena).
+  // pmax_dev (nullable, device [n][L]): also the largest softmax probability of each refinement position.
   cudaError_t parseq_forward(const __nv_bfloat16* patches_dev, int n, const int* forced_dev, float** logits_out,
-                             int** ids_out);
+                             int** ids_out, float* pmax_dev = nullptr);
   size_t parseq_bytes(int n) const;
 };
 

@@ -267,7 +267,7 @@ static cudaError_t lin(cudaStream_t s, const __nv_bfloat16* A, int lda, int M, i
 }
 
 cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const int* forced, float** logits_out,
-                                      int** ids_out) {
+                                      int** ids_out, float* pmax_dev) {
   using bf = __nv_bfloat16;
   const ParseqDims& pd = w->pd;
   const WeightFile& wf = w->parseq;
@@ -492,7 +492,10 @@ cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const
   }
   DecoderStep st{n, D, pd.dec_heads, L, 0, L, 1};
   RUN(stream_tail(st, R, logits, NC));
-  RUN(argmax_rows(logits, R, pd.n_cls, NC, ids, 1, nullptr, 0, nullptr, 0, s));
+  if (pmax_dev)   // scores requested: the same ids plus each position's largest softmax probability, in the same launch
+    RUN(argmax_conf_rows(logits, R, pd.n_cls, NC, ids, pmax_dev, s));
+  else
+    RUN(argmax_rows(logits, R, pd.n_cls, NC, ids, 1, nullptr, 0, nullptr, 0, s));
   // decoder: 2 x 0.153 GMAC per crop over L + 1 passes; its floor is one read of the crop's memory K|V (128 x 768 bf16) per
   // pass the crop takes part in: L AR steps (fewer with the early exit) + the refinement
   {

@@ -994,6 +994,37 @@ __global__ void k_argmax(const float* __restrict__ logits, int rows, int n_cls, 
   }
 }
 
+// Refinement head with scores: the argmax of k_argmax (same per-lane and cross-lane rules, so the ids are bit-identical)
+// and the row's largest softmax probability p = 1 / sum_c exp(l[c] - max), summed per lane in class order and then over
+// a fixed xor butterfly (every lane ends with the same bits), accurate expf: p is deterministic.  A row with a NaN
+// gets p = NaN.  The second pass re-reads the row from L1.
+__global__ void k_argmax_conf(const float* __restrict__ logits, int rows, int n_cls, int ld, int* __restrict__ ids,
+                              float* __restrict__ pmax) {
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (row >= rows) return;
+  const float* l = logits + static_cast<long long>(row) * ld;
+  float best = -INFINITY;
+  int bi = 0x7fffffff;
+  for (int c = lane; c < n_cls; c += 32) {
+    const float v = l[c];
+    if (v > best) { best = v; bi = c; }  // strictly greater: first max per lane
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    const float ov = __shfl_xor_sync(0xffffffffu, best, o);
+    const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+    if (ov > best || (ov == best && oi < bi)) { best = ov; bi = oi; }  // ties -> lowest index (at::max on CPU)
+  }
+  if (bi >= n_cls) bi = 0;  // all-NaN row
+  float sum = 0.f;
+  for (int c = lane; c < n_cls; c += 32) sum += expf(l[c] - best);
+  for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
+  if (lane == 0) {
+    ids[row] = bi;
+    pmax[row] = 1.f / sum;
+  }
+}
+
 // fp32 -> (hi, lo) bf16 pair with x ~= hi + lo (the split residual stream of gemm_tc.cuh, RES_SPLIT)
 __global__ void k_split_f32(const float* __restrict__ x, long long n, __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo) {
   const long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
@@ -1213,6 +1244,13 @@ cudaError_t argmax_rows(const float* logits, int rows, int n_cls, int ld, int* i
   if (rows <= 0) return cudaSuccess;
   k_argmax<<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, ids_stride, next, next_stride, forced,
                                           forced_stride);
+  TT_LAUNCH_CHECK();
+  return cudaSuccess;
+}
+
+cudaError_t argmax_conf_rows(const float* logits, int rows, int n_cls, int ld, int* ids, float* pmax, cudaStream_t s) {
+  if (rows <= 0) return cudaSuccess;
+  k_argmax_conf<<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, pmax);
   TT_LAUNCH_CHECK();
   return cudaSuccess;
 }

@@ -62,6 +62,9 @@ cudaError_t dec_cross_attn(const DecoderStep& st, const __nv_bfloat16* q, const 
 // `forced` != null the value written to next_tokens comes from forced instead of the argmax.
 cudaError_t argmax_rows(const float* logits, int rows, int n_cls, int ld, int* ids, int ids_stride,
                         int* next_tokens, int next_stride, const int* forced, int forced_stride, cudaStream_t s);
+// argmax_rows' ids (same tie and NaN rules, bit-identical) fused with the largest softmax probability of the row,
+// pmax[row] = 1 / sum_c exp(logits[row][c] - max) in fp32 (deterministic; NaN for a row holding a NaN).  ids, pmax [rows].
+cudaError_t argmax_conf_rows(const float* logits, int rows, int n_cls, int ld, int* ids, float* pmax, cudaStream_t s);
 // u8 crops [n][32][128][3] -> bf16 patch rows [n*128][96] (raw 0..255), k = c*32 + (y%4)*8 + x%8
 cudaError_t tokens_init(int* tokens, int n, int L, int bos, int pad, cudaStream_t s);
 // AR early exit: the crops of (active_in, *n_in) -- null: all n crops -- whose token at position `pos` is not EOS, in the

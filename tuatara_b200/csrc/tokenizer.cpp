@@ -37,4 +37,24 @@ std::string decode_ids(const int32_t* ids, int len) {
   return s;
 }
 
+void decode_ids_scored(const int32_t* ids, const float* p, int len, std::string* text, std::vector<float>* char_conf,
+                       float* conf) {
+  const TokenizerTable& t = tokenizer_table();
+  text->clear();
+  char_conf->clear();
+  int end = len - 1;   // no end class: every position is a factor
+  for (int i = 0; i < len; ++i) {   // decode_ids' loop, keeping the probability of each character it emits
+    const int id = ids[i];
+    if (id == t.eos_id) continue;
+    if (id < 0 || id >= static_cast<int>(t.itos.size())) continue;
+    const char ch = t.itos[id];
+    if (ch == ']') { end = i; break; }
+    text->push_back(ch);
+    char_conf->push_back(p[i]);
+  }
+  double prod = 1.0;
+  for (int i = 0; i <= end; ++i) prod *= static_cast<double>(p[i]);
+  *conf = static_cast<float>(prod);
+}
+
 }  // namespace tt

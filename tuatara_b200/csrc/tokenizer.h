@@ -3,6 +3,7 @@
 #include <stdint.h>
 
 #include <string>
+#include <vector>
 
 namespace tt {
 
@@ -16,5 +17,14 @@ const TokenizerTable& tokenizer_table();
 // Drops every id == eos_id (tuatara.cpp:108-116), maps through itos (:93-99), cuts at the first
 // ']' character (:497-502).
 std::string decode_ids(const int32_t* ids, int len);
+
+// decode_ids with scores.  p[i]: the largest softmax probability at position i.  The end position e is the first
+// position whose id is 0 (itos[0] = ']', where decode_ids stops; upstream PARSeq's EOS class), else len - 1.
+//   text      == decode_ids(ids, len)
+//   char_conf  = p[i] of each position that emits a character of text, in order: positions before the first id 0
+//                (every position when there is none) whose id is not eos_id, so char_conf.size() == text.size()
+//   conf       = prod_{i=0..e} p[i], multiplied in double in position order and rounded once to float
+void decode_ids_scored(const int32_t* ids, const float* p, int len, std::string* text, std::vector<float>* char_conf,
+                       float* conf);
 
 }  // namespace tt
