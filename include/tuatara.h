@@ -56,6 +56,13 @@ struct ScoredItem {
   std::vector<float> char_confidence;    // one probability per character of text
 };
 
+// Character filter (tt_char_filter, INTEGRATION.md section 7): recognition only produces characters that are in `allow`
+// (when not null) and not in `block` (when not null).  E.g. CharFilter{"0123456789"} for digits only.
+struct CharFilter {
+  const char* allow = nullptr;
+  const char* block = nullptr;
+};
+
 namespace detail {
 inline tt_engine* engine_for(const std::string& weights_dir) {
   static std::mutex mu;
@@ -78,9 +85,10 @@ inline tt_engine* engine_for(const std::string& weights_dir) {
 
 namespace detail {
 // The checks, soft failures and engine call shared by the batch entry points: nullptr after printing the reason.
-// opt == nullptr: plain tt_ocr_pages.
+// opt == nullptr: plain tt_ocr_pages.  filters != nullptr: tt_ocr_pages_filtered (one filter, or one per page).
 inline tt_result* ocr_pages(const std::vector<ImageView>& images, const std::string& weights_dir,
-                            const std::string& outputs_dir, const tt_ocr_options* opt) {
+                            const std::string& outputs_dir, const tt_ocr_options* opt,
+                            const std::vector<CharFilter>* filters = nullptr) {
   if (weights_dir.empty()) { std::cerr << "Please provide a value for weights_dir" << std::endl; return nullptr; }
   if (outputs_dir.empty()) { std::cerr << "Please provide a value for outputs_dir" << std::endl; return nullptr; }
   std::vector<tt_image> pages(images.size());
@@ -92,22 +100,28 @@ inline tt_result* ocr_pages(const std::vector<ImageView>& images, const std::str
   tt_engine* e = engine_for(weights_dir);
   if (!e) { std::cerr << "error loading the models: " << tt_last_error() << std::endl; return nullptr; }
   tt_result* r = nullptr;
-  const int rc = opt ? tt_ocr_pages_ex(e, pages.data(), static_cast<int>(pages.size()), opt, &r)
-                     : tt_ocr_pages(e, pages.data(), static_cast<int>(pages.size()), &r);
+  int rc = 0;
+  if (filters) {
+    std::vector<tt_char_filter> f;
+    for (const CharFilter& cf : *filters) f.push_back(tt_char_filter{cf.allow, cf.block});
+    const tt_ocr_options none = {};
+    rc = tt_ocr_pages_filtered(e, pages.data(), static_cast<int>(pages.size()), opt ? opt : &none, f.data(),
+                               static_cast<int>(f.size()), &r);
+  } else {
+    rc = opt ? tt_ocr_pages_ex(e, pages.data(), static_cast<int>(pages.size()), opt, &r)
+             : tt_ocr_pages(e, pages.data(), static_cast<int>(pages.size()), &r);
+  }
   if (rc != 0) {
     std::cerr << "tuatara: " << tt_last_error() << std::endl;
     return nullptr;
   }
   return r;
 }
-}  // namespace detail
 
-// Additive batch API: many pages in one call, spread over the engine's GPUs (all visible ones, or TT_DEVICES).
-inline std::vector<std::vector<OutputItem>> image_to_data_batch(const std::vector<ImageView>& images,
-                                                                const std::string& weights_dir,
-                                                                const std::string& outputs_dir) {
+inline std::vector<std::vector<OutputItem>> batch_items(const std::vector<ImageView>& images, const std::string& weights_dir,
+                                                        const std::string& outputs_dir, const std::vector<CharFilter>* filters) {
   std::vector<std::vector<OutputItem>> out;
-  tt_result* r = detail::ocr_pages(images, weights_dir, outputs_dir, nullptr);
+  tt_result* r = ocr_pages(images, weights_dir, outputs_dir, nullptr, filters);
   if (!r) return out;
   out.resize(r->n_pages);
   for (int p = 0; p < r->n_pages; ++p)
@@ -119,14 +133,12 @@ inline std::vector<std::vector<OutputItem>> image_to_data_batch(const std::vecto
   return out;
 }
 
-// image_to_data_batch with scores: same items (text, bbox) and the same soft failures, plus each item's scores.
-inline std::vector<std::vector<ScoredItem>> image_to_data_scored_batch(const std::vector<ImageView>& images,
-                                                                       const std::string& weights_dir,
-                                                                       const std::string& outputs_dir) {
+inline std::vector<std::vector<ScoredItem>> scored_items(const std::vector<ImageView>& images, const std::string& weights_dir,
+                                                         const std::string& outputs_dir, const std::vector<CharFilter>* filters) {
   std::vector<std::vector<ScoredItem>> out;
   tt_ocr_options opt = {};
   opt.with_scores = 1;
-  tt_result* r = detail::ocr_pages(images, weights_dir, outputs_dir, &opt);
+  tt_result* r = ocr_pages(images, weights_dir, outputs_dir, &opt, filters);
   if (!r) return out;
   out.resize(r->n_pages);
   for (int p = 0; p < r->n_pages; ++p)
@@ -148,10 +160,49 @@ inline std::vector<std::vector<ScoredItem>> image_to_data_scored_batch(const std
   tt_result_free(r);
   return out;
 }
+}  // namespace detail
+
+// Additive batch API: many pages in one call, spread over the engine's GPUs (all visible ones, or TT_DEVICES).
+inline std::vector<std::vector<OutputItem>> image_to_data_batch(const std::vector<ImageView>& images,
+                                                                const std::string& weights_dir,
+                                                                const std::string& outputs_dir) {
+  return detail::batch_items(images, weights_dir, outputs_dir, nullptr);
+}
+
+// image_to_data_batch with character filters: `filters` holds one filter for every page, or one per page.
+inline std::vector<std::vector<OutputItem>> image_to_data_batch(const std::vector<ImageView>& images,
+                                                                const std::string& weights_dir,
+                                                                const std::string& outputs_dir,
+                                                                const std::vector<CharFilter>& filters) {
+  return detail::batch_items(images, weights_dir, outputs_dir, &filters);
+}
+
+// image_to_data_batch with scores: same items (text, bbox) and the same soft failures, plus each item's scores.
+inline std::vector<std::vector<ScoredItem>> image_to_data_scored_batch(const std::vector<ImageView>& images,
+                                                                       const std::string& weights_dir,
+                                                                       const std::string& outputs_dir) {
+  return detail::scored_items(images, weights_dir, outputs_dir, nullptr);
+}
+
+// image_to_data_scored_batch with character filters (one for every page, or one per page); the scores are renormalised
+// over each page's allowed characters (tt_item_scores).
+inline std::vector<std::vector<ScoredItem>> image_to_data_scored_batch(const std::vector<ImageView>& images,
+                                                                       const std::string& weights_dir,
+                                                                       const std::string& outputs_dir,
+                                                                       const std::vector<CharFilter>& filters) {
+  return detail::scored_items(images, weights_dir, outputs_dir, &filters);
+}
 
 inline std::vector<ScoredItem> image_to_data_scored(const ImageView& image, const std::string& weights_dir,
                                                     const std::string& outputs_dir) {
   std::vector<std::vector<ScoredItem>> pages = image_to_data_scored_batch({image}, weights_dir, outputs_dir);
+  return pages.empty() ? std::vector<ScoredItem>{} : pages[0];
+}
+
+inline std::vector<ScoredItem> image_to_data_scored(const ImageView& image, const std::string& weights_dir,
+                                                    const std::string& outputs_dir, const CharFilter& filter) {
+  std::vector<std::vector<ScoredItem>> pages =
+      image_to_data_scored_batch({image}, weights_dir, outputs_dir, std::vector<CharFilter>{filter});
   return pages.empty() ? std::vector<ScoredItem>{} : pages[0];
 }
 
@@ -160,6 +211,13 @@ inline std::vector<ScoredItem> image_to_data_scored(const ImageView& image, cons
 inline std::vector<OutputItem> image_to_data(const tuatara::ImageView& image, std::string weights_dir,
                                              std::string outputs_dir) {
   auto pages = tuatara::image_to_data_batch({image}, weights_dir, outputs_dir);
+  return pages.empty() ? std::vector<OutputItem>{} : pages[0];
+}
+
+// image_to_data with a character filter: every character of every item's text obeys it.
+inline std::vector<OutputItem> image_to_data(const tuatara::ImageView& image, std::string weights_dir,
+                                             std::string outputs_dir, const tuatara::CharFilter& filter) {
+  auto pages = tuatara::image_to_data_batch({image}, weights_dir, outputs_dir, std::vector<tuatara::CharFilter>{filter});
   return pages.empty() ? std::vector<OutputItem>{} : pages[0];
 }
 

@@ -101,9 +101,29 @@ typedef struct tt_ocr_options {
 } tt_ocr_options;
 TT_API int tt_ocr_pages_ex(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt, tt_result** out);
 TT_API void tt_result_free(tt_result* r);
+/* Character filter (INTEGRATION.md section 7): restricts the characters recognition may produce.  allow / block are
+ * NUL-terminated byte strings or NULL (no restriction).  Class c of the 95 prints itos[c] (tt_tokenizer_table); classes 0
+ * (end of word) and 88 (dropped from the text) print nothing and are always allowed.  Any other class is allowed iff
+ * (allow == NULL or allow holds its character) and (block == NULL or block does not).  Characters no class prints are
+ * ignored; allow = "" is valid and gives every word an empty text.  The choice is made inside the greedy decode: at every
+ * AR step (the token fed back is the best allowed class) and at the refinement.  Boxes, bboxes, det_score, item order
+ * and detect_only results do not change; a filter that allows every class gives bit-identical results to no filter. */
+typedef struct tt_char_filter {
+  const char* allow;
+  const char* block;
+} tt_char_filter;
+/* The filter's class mask (host only): bit c & 31 of mask_out[c >> 5] is set when class c is allowed; mask_out[3] = 0. */
+TT_API int tt_char_filter_mask(const tt_char_filter* f, uint32_t mask_out[4]);
+/* tt_ocr_pages_ex with character filters.  n_filters == 1: filters[0] for every page; == n_pages: filters[i] for page i;
+ * == 0 (filters may be NULL): the same as tt_ocr_pages_ex.  Any other count, or filters == NULL with n_filters > 0, is an
+ * error.  Every character of every item's text is in its page's allow (when given) and not in its block (when given). */
+TT_API int tt_ocr_pages_filtered(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
+                                 const tt_char_filter* filters, int n_filters, tt_result** out);
 /* Scores of item `item` of page `page` of a result made with tt_ocr_options.with_scores = 1 (an error otherwise).
  * Scale 0..1.  p[t] is the largest softmax probability of the refinement logits at position t (t = 0..25), the
  * position's id being its argmax; the end position e is the first t whose id is 0 (where the text stops), else 25.
+ * With a character filter (tt_ocr_pages_filtered) the softmax is renormalised over the page's allowed classes:
+ * p[t] = 1 / sum_{c allowed} exp(l[t][c] - max_{c allowed} l[t][c]), the id being the argmax over those classes.
  *  conf       = p[0] * ... * p[e] (the end position and positions of id 88 included), multiplied in double and
  *               rounded once to float; may underflow to 0.  -1 when the item was not recognised (detect_only).
  *  det_score  = the component's maximum normalised text score (tuatara.cpp:151-152), >= text_threshold.
@@ -176,6 +196,12 @@ TT_API int tt_parseq_forward(tt_engine* e, const uint8_t* crops, int n, const in
 /* tt_parseq_forward's ids together with pmax_out [n][26]: the largest softmax probability of the refinement logits at
  * each position (the p[t] of tt_item_scores), from the same kernel that picks the ids.  ids_out [n][26]. */
 TT_API int tt_parseq_forward_scores(tt_engine* e, const uint8_t* crops, int n, int32_t* ids_out, float* pmax_out);
+/* tt_parseq_forward / tt_parseq_forward_scores with per-crop class masks (tt_char_filter_mask): class_masks [n][4]
+ * (NULL = none).  Every AR step feeds back the argmax over the crop's allowed classes (forced_tokens, when given, still
+ * win) and ids_out / pmax_out are the refinement's argmax and renormalised probability over them.  logits_out holds the
+ * raw, unmasked head output.  Every output pointer may be NULL. */
+TT_API int tt_parseq_forward_masked(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens,
+                                    const uint32_t* class_masks, float* logits_out, int32_t* ids_out, float* pmax_out);
 /* Tokenizer::decode + truncation (tuatara.cpp:61-116, :497-502). ids [n][len]; out [n][out_stride] chars. */
 TT_API int tt_decode(const int32_t* ids, int n, int len, char* out, int out_stride);
 /* tt_decode with the scores of tt_item_scores (host only).  pmax [n][len]; conf_out (nullable) [n];

@@ -17,7 +17,8 @@ from ._native import TuataraError, check, lib, ptr
 
 __all__ = [
     "TuataraError", "Engine", "image_to_data", "images_to_data", "image_to_data_scored", "images_to_data_scored",
-    "default_config", "resize_plan", "preprocess", "postprocess", "crop_resize", "decode_ids", "decode_scores", "tokenizer_table", "min_area_rect", "convex_hull",
+    "default_config", "resize_plan", "preprocess", "postprocess", "crop_resize", "decode_ids", "decode_scores", "tokenizer_table",
+    "char_filter_mask", "min_area_rect", "convex_hull",
     "rect_points", "rect_bounding", "adjust_rect", "rect_to_bbox", "launch_count",
 ]
 
@@ -46,6 +47,41 @@ def tokenizer_table():
     eos, bos, pad = C.c_int(), C.c_int(), C.c_int()
     check(lib().tt_tokenizer_table(buf, C.byref(eos), C.byref(bos), C.byref(pad)), "tt_tokenizer_table")
     return buf.value.decode("latin-1"), eos.value, bos.value, pad.value
+
+
+def _filter_bytes(v, name: str):
+    if v is None:
+        return None
+    if not isinstance(v, str):
+        raise TypeError(f"{name}: expected str or None")
+    return v.encode()
+
+
+def char_filter_mask(allow: str | None = None, block: str | None = None) -> np.ndarray:
+    """Class mask of a character filter (tt_char_filter_mask): uint32 [4], bit c & 31 of word c >> 5 set when class c may
+    be produced.  Classes 0 and 88 (they print nothing) are always set; word 3 is 0."""
+    f = _native.tt_char_filter(_filter_bytes(allow, "allow"), _filter_bytes(block, "block"))
+    out = np.zeros(4, np.uint32)
+    check(lib().tt_char_filter_mask(C.byref(f), ptr(out)), "tt_char_filter_mask")
+    return out
+
+
+def _filters(allowlist, blocklist, n_pages: int):
+    """allowlist / blocklist keywords -> a tt_char_filter array (None: no filter).  Each is None, a str for every page, or
+    a list with one str or None per page."""
+    if allowlist is None and blocklist is None:
+        return None
+    per_page = isinstance(allowlist, (list, tuple)) or isinstance(blocklist, (list, tuple))
+    n = n_pages if per_page else 1
+    cols = []
+    for v, name in ((allowlist, "allowlist"), (blocklist, "blocklist")):
+        if isinstance(v, (list, tuple)):
+            if len(v) != n_pages:
+                raise ValueError(f"{name}: expected one entry per page ({n_pages}), got {len(v)}")
+            cols.append([_filter_bytes(x, name) for x in v])
+        else:
+            cols.append([_filter_bytes(v, name)] * n)
+    return (_native.tt_char_filter * n)(*[_native.tt_char_filter(a, b) for a, b in zip(*cols)])
 
 
 def decode_ids(ids: np.ndarray) -> list[str]:
@@ -210,12 +246,14 @@ class Engine:
     __del__ = close
 
     def ocr_pages(self, images: list, score_override: list | None = None, detect_only: bool = False,
-                  scores: bool = False) -> list[list[dict]]:
+                  scores: bool = False, *, allowlist=None, blocklist=None) -> list[list[dict]]:
         """images: uint8 [H,W,3] numpy arrays (host) or torch CUDA tensors (already on the device).
         score_override: optional per-page float32 [h32/2, w32/2, 2] maps (numpy or CUDA tensors, or
         None entries) that replace CRAFT's output after CRAFT has run (benchmark / parity tests).
         scores: every item also carries conf (word confidence 0..1, None when not recognised), det_score (the
-        detection score of its box) and char_conf (one probability per character of text); see tt_item_scores."""
+        detection score of its box) and char_conf (one probability per character of text); see tt_item_scores.
+        allowlist / blocklist: character filters (tt_ocr_pages_filtered): recognition only produces characters in
+        allowlist and not in blocklist.  Each is None, a str for every page, or a list with one str or None per page."""
         n = len(images)
         on_dev = n > 0 and not isinstance(images[0], np.ndarray)
         if on_dev:
@@ -241,7 +279,12 @@ class Engine:
             opt.override_on_device = int(ov_dev)
             opt.score_override = ptrs
         res = C.POINTER(_native.tt_result)()
-        check(lib().tt_ocr_pages_ex(self._h, arr, n, C.byref(opt), C.byref(res)), "tt_ocr_pages_ex")
+        filters = _filters(allowlist, blocklist, n)
+        if filters is None:
+            check(lib().tt_ocr_pages_ex(self._h, arr, n, C.byref(opt), C.byref(res)), "tt_ocr_pages_ex")
+        else:
+            check(lib().tt_ocr_pages_filtered(self._h, arr, n, C.byref(opt), filters, len(filters), C.byref(res)),
+                  "tt_ocr_pages_filtered")
         try:
             out = []
             for p in range(res.contents.n_pages):
@@ -271,25 +314,46 @@ class Engine:
         check(lib().tt_craft_tap(self._h, name.encode(), ptr(out), out.size, dims), "tt_craft_tap")
         return out
 
-    def parseq_forward_scores(self, crops_u8: np.ndarray):
+    def parseq_forward_scores(self, crops_u8: np.ndarray, class_masks: np.ndarray | None = None):
         """crops_u8: uint8 [n, 32, 128, 3] -> (ids int32 [n, 26], pmax float32 [n, 26]): parseq_forward's ids and the
-        largest softmax probability of the refinement logits at each position."""
+        largest softmax probability of the refinement logits at each position.  class_masks: as in parseq_forward
+        (pmax is then renormalised over each crop's allowed classes)."""
         x = np.ascontiguousarray(crops_u8, np.uint8)
         n = x.shape[0]
         ids = np.empty((n, 26), np.int32)
         pmax = np.empty((n, 26), np.float32)
-        check(lib().tt_parseq_forward_scores(self._h, ptr(x), n, ptr(ids), ptr(pmax)), "tt_parseq_forward_scores")
+        if class_masks is None:
+            check(lib().tt_parseq_forward_scores(self._h, ptr(x), n, ptr(ids), ptr(pmax)), "tt_parseq_forward_scores")
+        else:
+            m = _class_masks(class_masks, n)
+            check(lib().tt_parseq_forward_masked(self._h, ptr(x), n, None, ptr(m), None, ptr(ids), ptr(pmax)),
+                  "tt_parseq_forward_masked")
         return ids, pmax
 
-    def parseq_forward(self, crops_u8: np.ndarray, forced_tokens: np.ndarray | None = None):
-        """crops_u8: uint8 [n, 32, 128, 3] -> (logits float32 [n, 26, 95], ids int32 [n, 26])."""
+    def parseq_forward(self, crops_u8: np.ndarray, forced_tokens: np.ndarray | None = None,
+                       class_masks: np.ndarray | None = None):
+        """crops_u8: uint8 [n, 32, 128, 3] -> (logits float32 [n, 26, 95], ids int32 [n, 26]).
+        class_masks: uint32 [n, 4] per-crop class masks (char_filter_mask): every greedy choice runs over the crop's
+        allowed classes (tt_parseq_forward_masked); the logits stay unmasked."""
         x = np.ascontiguousarray(crops_u8, np.uint8)
         n = x.shape[0]
         logits = np.empty((n, 26, 95), np.float32)
         ids = np.empty((n, 26), np.int32)
         ft = None if forced_tokens is None else np.ascontiguousarray(forced_tokens, np.int32)
-        check(lib().tt_parseq_forward(self._h, ptr(x), n, ptr(ft), ptr(logits), ptr(ids)), "tt_parseq_forward")
+        if class_masks is None:
+            check(lib().tt_parseq_forward(self._h, ptr(x), n, ptr(ft), ptr(logits), ptr(ids)), "tt_parseq_forward")
+        else:
+            m = _class_masks(class_masks, n)
+            check(lib().tt_parseq_forward_masked(self._h, ptr(x), n, ptr(ft), ptr(m), ptr(logits), ptr(ids), None),
+                  "tt_parseq_forward_masked")
         return logits, ids
+
+
+def _class_masks(class_masks, n: int) -> np.ndarray:
+    m = np.ascontiguousarray(class_masks, np.uint32)
+    if m.shape != (n, 4):
+        raise ValueError(f"class_masks: expected shape ({n}, 4), got {m.shape}")
+    return m
 
 
 def _item_scores(res, page: int, item: int) -> dict:
@@ -312,10 +376,12 @@ def _engine_for(weights_dir: str) -> Engine:
     return _engines[key]
 
 
-def image_to_data(image: np.ndarray, weights_dir: str, outputs_dir: str) -> list[dict]:
+def image_to_data(image: np.ndarray, weights_dir: str, outputs_dir: str, *, allowlist: str | None = None,
+                  blocklist: str | None = None) -> list[dict]:
     """Same call as the reference's ``pytuatara.image_to_data`` (bindings/python.cpp:43-57):
     uint8 [H, W, 3] in, list of ``dict(text=str, bbox=[4 floats])`` out.  Empty directory
-    strings print to stderr and return [] like tuatara.cpp:315-323."""
+    strings print to stderr and return [] like tuatara.cpp:315-323.  allowlist / blocklist: recognition only produces
+    characters in allowlist and not in blocklist (INTEGRATION.md section 7)."""
     import sys
 
     if not weights_dir:
@@ -326,15 +392,18 @@ def image_to_data(image: np.ndarray, weights_dir: str, outputs_dir: str) -> list
         return []
     if image.ndim != 3:
         raise RuntimeError("Input array should have 3 dimensions")
-    return _engine_for(weights_dir).ocr_pages([image])[0]
+    return _engine_for(weights_dir).ocr_pages([image], allowlist=allowlist, blocklist=blocklist)[0]
 
 
-def images_to_data(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".") -> list[list[dict]]:
-    """Additive batch API: one call, many pages (sharded over the engine's GPUs)."""
-    return _engine_for(weights_dir).ocr_pages(list(images))
+def images_to_data(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".", *, allowlist=None,
+                   blocklist=None) -> list[list[dict]]:
+    """Additive batch API: one call, many pages (sharded over the engine's GPUs).  allowlist / blocklist: None, a str
+    for every page, or a list with one str or None per page."""
+    return _engine_for(weights_dir).ocr_pages(list(images), allowlist=allowlist, blocklist=blocklist)
 
 
-def image_to_data_scored(image: np.ndarray, weights_dir: str, outputs_dir: str) -> list[dict]:
+def image_to_data_scored(image: np.ndarray, weights_dir: str, outputs_dir: str, *, allowlist: str | None = None,
+                         blocklist: str | None = None) -> list[dict]:
     """image_to_data whose items also carry ``conf`` (word confidence 0..1), ``det_score`` (the detection score of the
     box) and ``char_conf`` (one probability per character of ``text``).  Same inputs, errors and soft failures;
     ``text`` and ``bbox`` are what image_to_data returns."""
@@ -348,9 +417,10 @@ def image_to_data_scored(image: np.ndarray, weights_dir: str, outputs_dir: str) 
         return []
     if image.ndim != 3:
         raise RuntimeError("Input array should have 3 dimensions")
-    return _engine_for(weights_dir).ocr_pages([image], scores=True)[0]
+    return _engine_for(weights_dir).ocr_pages([image], scores=True, allowlist=allowlist, blocklist=blocklist)[0]
 
 
-def images_to_data_scored(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".") -> list[list[dict]]:
+def images_to_data_scored(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".", *, allowlist=None,
+                          blocklist=None) -> list[list[dict]]:
     """Batch variant of image_to_data_scored."""
-    return _engine_for(weights_dir).ocr_pages(list(images), scores=True)
+    return _engine_for(weights_dir).ocr_pages(list(images), scores=True, allowlist=allowlist, blocklist=blocklist)

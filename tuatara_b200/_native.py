@@ -33,6 +33,10 @@ class tt_ocr_options(C.Structure):
                 ("score_override", C.POINTER(C.c_void_p)), ("detect_only", C.c_int), ("with_scores", C.c_int)]
 
 
+class tt_char_filter(C.Structure):
+    _fields_ = [("allow", C.c_char_p), ("block", C.c_char_p)]
+
+
 class tt_item(C.Structure):
     _fields_ = [("text", C.c_char_p), ("bbox", C.c_float * 4)]
 
@@ -61,6 +65,9 @@ SIGNATURES = {
     "tt_ocr_pages": (_I, [_P, C.POINTER(tt_image), _I, C.POINTER(C.POINTER(tt_result))]),
     "tt_ocr_pages_ex": (_I, [_P, C.POINTER(tt_image), _I, C.POINTER(tt_ocr_options), C.POINTER(C.POINTER(tt_result))]),
     "tt_result_free": (None, [C.POINTER(tt_result)]),
+    "tt_char_filter_mask": (_I, [C.POINTER(tt_char_filter), _P]),
+    "tt_ocr_pages_filtered": (_I, [_P, C.POINTER(tt_image), _I, C.POINTER(tt_ocr_options), C.POINTER(tt_char_filter), _I,
+                                   C.POINTER(C.POINTER(tt_result))]),
     "tt_item_scores": (_I, [C.POINTER(tt_result), _I, _I, _PF, _PF, C.POINTER(_PF), _PI]),
     "tt_launch_count": (C.c_ulonglong, []),
     "tt_engine_set_slots": (None, [_P, _I]),
@@ -81,6 +88,7 @@ SIGNATURES = {
     "tt_rect_to_quad": (_I, [_P, _P]),
     "tt_parseq_forward": (_I, [_P, _P, _I, _P, _P, _P]),
     "tt_parseq_forward_scores": (_I, [_P, _P, _I, _P, _P]),
+    "tt_parseq_forward_masked": (_I, [_P, _P, _I, _P, _P, _P, _P, _P]),
     "tt_decode": (_I, [_P, _I, _I, _P, _I]),
     "tt_decode_scores": (_I, [_P, _P, _I, _I, _P, _I, _P, _P]),
     "tt_tokenizer_table": (_I, [C.c_char_p, _PI, _PI, _PI]),

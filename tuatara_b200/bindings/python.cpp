@@ -3,6 +3,8 @@
 //   pytuatara.image_to_data(image, weights_dir, outputs_dir) -> list[dict(text=str, bbox=list[float])]
 // The reference copies the buffer into a cv::Mat (buffer_to_mat, :12-28); here the numpy buffer is
 // passed straight to the C ABI as an ImageView.
+#include <memory>
+
 #include <pybind11/numpy.h>
 #include <pybind11/pybind11.h>
 #include <pybind11/stl.h>
@@ -42,13 +44,50 @@ static py::dict scored_item_to_dict(const tuatara::ScoredItem& item) {
   return d;
 }
 
+// allowlist / blocklist keywords -> character filters (tuatara::CharFilter).  Each is None, a str (every page) or, for
+// the batch functions, a list with one str or None per page.  No filter at all when both are None.
+struct FilterArgs {
+  std::vector<std::unique_ptr<std::string>> keep;   // the strings the filters point into
+  std::vector<tuatara::CharFilter> filters;          // empty: no filter
+};
+
+static const char* filter_str(const py::handle& v, FilterArgs* fa, const char* name) {
+  if (v.is_none()) return nullptr;
+  if (!py::isinstance<py::str>(v)) throw py::type_error(std::string(name) + ": expected str or None");
+  fa->keep.emplace_back(new std::string(v.cast<std::string>()));
+  return fa->keep.back()->c_str();
+}
+
+static FilterArgs filter_args(const py::object& allow, const py::object& block, size_t n_pages, bool batch) {
+  FilterArgs fa;
+  if (allow.is_none() && block.is_none()) return fa;
+  const bool al = batch && py::isinstance<py::list>(allow), bl = batch && py::isinstance<py::list>(block);
+  if (al && py::len(allow) != n_pages)
+    throw py::value_error("allowlist: expected one entry per page (" + std::to_string(n_pages) + "), got " +
+                          std::to_string(py::len(allow)));
+  if (bl && py::len(block) != n_pages)
+    throw py::value_error("blocklist: expected one entry per page (" + std::to_string(n_pages) + "), got " +
+                          std::to_string(py::len(block)));
+  const size_t n = (al || bl) ? n_pages : 1;
+  for (size_t i = 0; i < n; ++i) {
+    tuatara::CharFilter f;
+    f.allow = filter_str(al ? py::handle(allow.cast<py::list>()[i]) : py::handle(allow), &fa, "allowlist");
+    f.block = filter_str(bl ? py::handle(block.cast<py::list>()[i]) : py::handle(block), &fa, "blocklist");
+    fa.filters.push_back(f);
+  }
+  return fa;
+}
+
 static py::list image_to_data_wrapper(py::array_t<unsigned char, py::array::c_style | py::array::forcecast> image_data,
-                                      std::string weights_dir, std::string output_dir) {
+                                      std::string weights_dir, std::string output_dir, py::object allowlist,
+                                      py::object blocklist) {
   const tuatara::ImageView img = buffer_to_view(image_data);
+  const FilterArgs fa = filter_args(allowlist, blocklist, 1, false);
   std::vector<OutputItem> items;
   {
     py::gil_scoped_release release;
-    items = image_to_data(img, weights_dir, output_dir);
+    items = fa.filters.empty() ? image_to_data(img, weights_dir, output_dir)
+                               : image_to_data(img, weights_dir, output_dir, fa.filters[0]);
   }
   py::list result;
   for (const auto& item : items) result.append(output_item_to_dict(item));
@@ -56,13 +95,16 @@ static py::list image_to_data_wrapper(py::array_t<unsigned char, py::array::c_st
 }
 
 static py::list images_to_data_wrapper(std::vector<py::array_t<unsigned char, py::array::c_style | py::array::forcecast>> images,
-                                       std::string weights_dir, std::string output_dir) {
+                                       std::string weights_dir, std::string output_dir, py::object allowlist,
+                                       py::object blocklist) {
   std::vector<tuatara::ImageView> views;
   for (auto& a : images) views.push_back(buffer_to_view(a));
+  const FilterArgs fa = filter_args(allowlist, blocklist, views.size(), true);
   std::vector<std::vector<OutputItem>> pages;
   {
     py::gil_scoped_release release;
-    pages = tuatara::image_to_data_batch(views, weights_dir, output_dir);
+    pages = fa.filters.empty() ? tuatara::image_to_data_batch(views, weights_dir, output_dir)
+                               : tuatara::image_to_data_batch(views, weights_dir, output_dir, fa.filters);
   }
   py::list result;
   for (const auto& page : pages) {
@@ -74,12 +116,15 @@ static py::list images_to_data_wrapper(std::vector<py::array_t<unsigned char, py
 }
 
 static py::list image_to_data_scored_wrapper(py::array_t<unsigned char, py::array::c_style | py::array::forcecast> image_data,
-                                             std::string weights_dir, std::string output_dir) {
+                                             std::string weights_dir, std::string output_dir, py::object allowlist,
+                                             py::object blocklist) {
   const tuatara::ImageView img = buffer_to_view(image_data);
+  const FilterArgs fa = filter_args(allowlist, blocklist, 1, false);
   std::vector<tuatara::ScoredItem> items;
   {
     py::gil_scoped_release release;
-    items = tuatara::image_to_data_scored(img, weights_dir, output_dir);
+    items = fa.filters.empty() ? tuatara::image_to_data_scored(img, weights_dir, output_dir)
+                               : tuatara::image_to_data_scored(img, weights_dir, output_dir, fa.filters[0]);
   }
   py::list result;
   for (const auto& item : items) result.append(scored_item_to_dict(item));
@@ -87,13 +132,16 @@ static py::list image_to_data_scored_wrapper(py::array_t<unsigned char, py::arra
 }
 
 static py::list images_to_data_scored_wrapper(std::vector<py::array_t<unsigned char, py::array::c_style | py::array::forcecast>> images,
-                                              std::string weights_dir, std::string output_dir) {
+                                              std::string weights_dir, std::string output_dir, py::object allowlist,
+                                              py::object blocklist) {
   std::vector<tuatara::ImageView> views;
   for (auto& a : images) views.push_back(buffer_to_view(a));
+  const FilterArgs fa = filter_args(allowlist, blocklist, views.size(), true);
   std::vector<std::vector<tuatara::ScoredItem>> pages;
   {
     py::gil_scoped_release release;
-    pages = tuatara::image_to_data_scored_batch(views, weights_dir, output_dir);
+    pages = fa.filters.empty() ? tuatara::image_to_data_scored_batch(views, weights_dir, output_dir)
+                               : tuatara::image_to_data_scored_batch(views, weights_dir, output_dir, fa.filters);
   }
   py::list result;
   for (const auto& page : pages) {
@@ -106,12 +154,17 @@ static py::list images_to_data_scored_wrapper(std::vector<py::array_t<unsigned c
 
 PYBIND11_MODULE(pytuatara, m) {
   m.doc() = "Tuatara ocr";
-  m.def("image_to_data", &image_to_data_wrapper, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"),
+  // allowlist / blocklist (keyword only): recognition only produces characters in allowlist and not in blocklist
+  m.def("image_to_data", &image_to_data_wrapper, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"), py::kw_only(),
+        py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(),
         "Extract text and bounding boxes from an image");
-  m.def("images_to_data", &images_to_data_wrapper, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"),
+  m.def("images_to_data", &images_to_data_wrapper, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"), py::kw_only(),
+        py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(),
         "Batch variant: list of images -> list of per-page results");
   m.def("image_to_data_scored", &image_to_data_scored_wrapper, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"),
+        py::kw_only(), py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(),
         "image_to_data whose items also carry conf (word confidence 0..1, None when not recognised), det_score and char_conf");
   m.def("images_to_data_scored", &images_to_data_scored_wrapper, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"),
+        py::kw_only(), py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(),
         "Batch variant of image_to_data_scored");
 }

@@ -272,6 +272,12 @@ int tt_decode_scores(const int32_t* ids, const float* pmax, int n, int len, char
   });
 }
 
+int tt_char_filter_mask(const tt_char_filter* f, uint32_t mask_out[4]) {
+  if (!f || !mask_out) { set_error("tt_char_filter_mask: null argument"); return 1; }
+  char_filter_mask(f->allow, f->block, mask_out);
+  return 0;
+}
+
 int tt_tokenizer_table(char* itos_out, int* eos_id, int* bos_id, int* pad_id) {
   const TokenizerTable& t = tokenizer_table();
   std::memcpy(itos_out, t.itos.c_str(), t.itos.size() + 1);

@@ -50,6 +50,7 @@ struct DenseParams {
   const int* active;
   const int* n_act;
   unsigned long long* dbg;               // TT_DEC_DEBUG=1 (development): role cycle counters of CTA 0
+  const uint32_t* mask;                  // B, MASK only: [n][4] class masks, indexed by crop like tokens
 };
 
 struct alignas(16) Ctl {
@@ -80,7 +81,8 @@ struct Cfg {
   static_assert(kSmem <= 227 * 1024, "shared memory budget");
 };
 
-template <int D, int MLP, int MODE>
+// MASK (MODE_B only): the greedy token is the argmax over the classes allowed by the crop's class mask.
+template <int D, int MLP, int MODE, bool MASK>
 __global__ void __launch_bounds__(kThreads, 1) k_dec_dense(const __grid_constant__ DenseParams p) {
   using C = Cfg<D, MLP, MODE>;
   constexpr int KB = C::KB, kStages = C::kStages;
@@ -393,16 +395,22 @@ __global__ void __launch_bounds__(kThreads, 1) k_dec_dense(const __grid_constant
       {
         const long long crop = (valid && p.active) ? p.active[m] : m;
         float* lrow = p.logits + (crop * p.L + p.step) * p.ncp;
+        // MASK: the crop's class mask, one 16-byte load (rows past the live count compete unmasked: never stored)
+        uint4 mw = make_uint4(~0u, ~0u, ~0u, ~0u);
+        if constexpr (MASK) {
+          if (valid) mw = *reinterpret_cast<const uint4*>(p.mask + crop * 4);
+        }
         float best = -INFINITY;
         int bi = 0;
         const int nb = p.ncp / 32, hb0 = half ? (nb + 1) / 2 : 0, hb1 = half ? nb : (nb + 1) / 2;
         for_blocks(tl + D, hb0, hb1, [&](int blk, uint32_t (&raw)[32]) {
           float l[32];
           lds_f32x32(vec_s + (6 * D + MLP + blk * 32) * 4, l);
+          const uint32_t bits = MASK ? (blk == 0 ? mw.x : blk == 1 ? mw.y : blk == 2 ? mw.z : mw.w) : ~0u;
 #pragma unroll
           for (int j = 0; j < 32; ++j) {
             l[j] += __uint_as_float(raw[j]);
-            if (blk * 32 + j < p.n_cls && l[j] > best) { best = l[j]; bi = blk * 32 + j; }   // first max wins (at::max on CPU)
+            if (blk * 32 + j < p.n_cls && (!MASK || ((bits >> j) & 1u)) && l[j] > best) { best = l[j]; bi = blk * 32 + j; }   // first max wins (at::max on CPU)
           }
           if (valid) {
 #pragma unroll
@@ -454,10 +462,10 @@ int dense_priority() {
   return prio;
 }
 
-template <int D, int MLP, int MODE>
+template <int D, int MLP, int MODE, bool MASK = false>
 cudaError_t launch_dense(const DenseParams& p, cudaStream_t s) {
   using C = Cfg<D, MLP, MODE>;
-  TT_CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(k_dec_dense<D, MLP, MODE>), C::kSmem));
+  TT_CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(k_dec_dense<D, MLP, MODE, MASK>), C::kSmem));
   // Highest launch priority: a CTA needs a whole SM (216 KB smem, 512 TMEM columns).  Next to the other half-batch's
   // cross-attention grid (thousands of small blocks, launched earlier) it would otherwise wait for that grid to drain.
   cudaLaunchConfig_t cfg{};
@@ -478,7 +486,7 @@ cudaError_t launch_dense(const DenseParams& p, cudaStream_t s) {
     cudaMemsetAsync(dbg_buf, 0, 8 * sizeof(unsigned long long), s);
     pp.dbg = dbg_buf;
   }
-  TT_CUDA_TRY(cudaLaunchKernelEx(&cfg, k_dec_dense<D, MLP, MODE>, pp));
+  TT_CUDA_TRY(cudaLaunchKernelEx(&cfg, k_dec_dense<D, MLP, MODE, MASK>, pp));
   TT_LAUNCH_CHECK();
   if (dbg_env && p.step == 13) {
     unsigned long long h[8];
@@ -562,7 +570,8 @@ cudaError_t dec_dense_a2(const DecDenseWeights& w, const __nv_bfloat16* ab, int 
 }
 
 cudaError_t dec_dense_b(const DecDenseWeights& w, const __nv_bfloat16* ab2, int n, int step, const float* t_scratch,
-                        float* logits, int* tokens, const int* forced, cudaStream_t s, const int* active, const int* n_act) {
+                        float* logits, int* tokens, const int* forced, cudaStream_t s, const int* active, const int* n_act,
+                        const uint32_t* mask) {
   if (n <= 0) return cudaSuccess;
   if (!w.ready) { set_error("dec_dense_b: weights not initialised for this width"); return cudaErrorInvalidValue; }
   DenseParams p{};
@@ -570,9 +579,13 @@ cudaError_t dec_dense_b(const DecDenseWeights& w, const __nv_bfloat16* ab2, int 
   p.tm_w0 = w.tm_wco; p.tm_w1 = w.tm_w1; p.tm_w2 = w.tm_w2; p.tm_wh = w.tm_wh;
   p.vec_src = w.vec_b;
   p.t_scratch = const_cast<float*>(t_scratch);
-  p.logits = logits; p.tokens = tokens; p.forced = forced;
+  p.logits = logits; p.tokens = tokens; p.forced = forced; p.mask = mask;
   p.n = n; p.L = w.L; p.step = step; p.n_cls = w.n_cls; p.ncp = w.ncp;
   p.active = active; p.n_act = n_act;
+  if (mask) {
+    if (w.D == 384) return launch_dense<384, 1536, MODE_B, true>(p, s);
+    return launch_dense<192, 768, MODE_B, true>(p, s);
+  }
   if (w.D == 384) return launch_dense<384, 1536, MODE_B>(p, s);
   return launch_dense<192, 768, MODE_B>(p, s);
 }

@@ -16,6 +16,7 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
+#include <stdint.h>
 
 namespace tt {
 
@@ -53,8 +54,10 @@ cudaError_t dec_dense_a2(const DecDenseWeights& w, const __nv_bfloat16* ab, int 
                          __nv_bfloat16* q_out, cudaStream_t s, const int* active = nullptr, const int* n_act = nullptr);
 // ab2 [n][D] bf16 (cross-attention output of step `step`), t_scratch -> logits [n][L][ncp] row `step` (fp32) and the next
 // token: tokens[crop][step + 1] = forced ? forced[crop][step] : argmax over the first n_cls logits (first max wins).
+// mask (nullable): class masks [n][4] uint32 (16-byte aligned, indexed by crop like tokens): the argmax runs over the
+// classes whose bit (c & 31 of word c >> 5) is set; the logits are written unmasked.
 cudaError_t dec_dense_b(const DecDenseWeights& w, const __nv_bfloat16* ab2, int n, int step, const float* t_scratch,
                         float* logits, int* tokens, const int* forced, cudaStream_t s, const int* active = nullptr,
-                        const int* n_act = nullptr);
+                        const int* n_act = nullptr, const uint32_t* mask = nullptr);
 
 }  // namespace tt

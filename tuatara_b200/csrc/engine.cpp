@@ -112,6 +112,8 @@ struct Unit {
 
 struct CropOwner { int page, box; };
 
+using ClassMask = std::array<uint32_t, 4>;   // tt_char_filter_mask
+
 // crops waiting for recognition in one slot (device patch rows live in DeviceCtx::patch_buf)
 struct Pending {
   std::vector<CropOwner> owner;
@@ -254,22 +256,35 @@ int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const
 
 // PARSeq + tokenizer over the slot's recognition batch (tuatara.cpp:450-505).  scores: the refinement head also
 // writes each position's largest softmax probability, copied back next to the ids and decoded into conf / char_conf.
-int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, bool scores) {
+// page_masks (null: no page of the request has a character filter): the class mask of every page of the request; each
+// crop decodes under its page's mask, uploaded per pass as [nc][4] words.
+int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, bool scores,
+              const std::vector<ClassMask>* page_masks) {
   const int n = static_cast<int>(pend->owner.size());
   const int L = d.w->pd.L;
   for (int c0 = 0; c0 < n; c0 += kMaxCropsPerPass) {
     const int nc = std::min(kMaxCropsPerPass, n - c0);
     const size_t bytes = sizeof(int) * static_cast<size_t>(nc) * L;   // ids; with scores as many bytes of pmax follow
-    const size_t need = d.parseq_bytes(nc) + (4u << 20) + (scores ? bytes : 0);
+    const size_t mask_bytes = page_masks ? sizeof(ClassMask) * nc : 0;
+    const size_t need = d.parseq_bytes(nc) + (4u << 20) + (scores ? bytes : 0) + mask_bytes;
     if (need > d.arena.capacity()) E_TRY(stream_sync(d.stream));
     E_TRY(d.arena.reserve(need));
     d.arena.reset();
     float* pmax = scores ? d.arena.get<float>(static_cast<size_t>(nc) * L) : nullptr;
     if (scores && !pmax) { set_error("arena exhausted (pmax)"); return 1; }
+    uint32_t* mask = nullptr;
+    E_TRY(d.ensure_pinned(std::max(scores ? 2 * bytes : bytes, mask_bytes)));
+    if (page_masks) {
+      mask = d.arena.get<uint32_t>(4 * static_cast<size_t>(nc));
+      if (!mask) { set_error("arena exhausted (class masks)"); return 1; }
+      ClassMask* host_mask = reinterpret_cast<ClassMask*>(d.pinned);   // the ids' D2H below is ordered after this copy
+      for (int c = 0; c < nc; ++c) host_mask[c] = (*page_masks)[pend->owner[c0 + c].page];
+      E_CUDA(cudaMemcpyAsync(mask, host_mask, mask_bytes, cudaMemcpyHostToDevice, d.stream));
+      g_h2d_bytes += mask_bytes;
+    }
     float* logits = nullptr;
     int* ids = nullptr;
-    E_TRY(d.parseq_forward(d.patch_buf + static_cast<size_t>(c0) * 128 * 96, nc, nullptr, &logits, &ids, pmax));
-    E_TRY(d.ensure_pinned(scores ? 2 * bytes : bytes));
+    E_TRY(d.parseq_forward(d.patch_buf + static_cast<size_t>(c0) * 128 * 96, nc, nullptr, &logits, &ids, pmax, mask));
     E_CUDA(cudaMemcpyAsync(d.pinned, ids, bytes, cudaMemcpyDeviceToHost, d.stream));
     g_d2h_bytes += bytes;
     if (scores) {
@@ -312,8 +327,9 @@ struct WorkQueues {
 };
 
 // One execution slot draining the queues.
-void slot_worker(tt_engine& e, int g, int sidx, int want, const tt_image* pages, const tt_ocr_options& opt, WorkQueues* q,
-                 std::vector<PageOut>* results, int* rc, std::string* err) {
+void slot_worker(tt_engine& e, int g, int sidx, int want, const tt_image* pages, const tt_ocr_options& opt,
+                 const std::vector<ClassMask>* page_masks, WorkQueues* q, std::vector<PageOut>* results, int* rc,
+                 std::string* err) {
   // take an idle slot of this GPU if there is one (concurrent callers spread over the slots), else queue on our own
   DeviceCtx* dp = nullptr;
   for (int k = 0; k < want && dp == nullptr; ++k) {
@@ -332,10 +348,17 @@ void slot_worker(tt_engine& e, int g, int sidx, int want, const tt_image* pages,
   Pending pend;
   for (int ui = q->pop(g); ui >= 0; ui = q->pop(g)) {
     if (detect_unit(d, cfg, pages, q->units[ui], opt, results, &pend)) { *err = last_error(); *rc = 1; return; }
-    if (pend.pages >= max_b && recognise(d, results, &pend, opt.with_scores != 0)) { *err = last_error(); *rc = 1; return; }
+    if (pend.pages >= max_b && recognise(d, results, &pend, opt.with_scores != 0, page_masks)) {
+      *err = last_error();
+      *rc = 1;
+      return;
+    }
   }
-  if (recognise(d, results, &pend, opt.with_scores != 0)) { *err = last_error(); *rc = 1; return; }
+  if (recognise(d, results, &pend, opt.with_scores != 0, page_masks)) { *err = last_error(); *rc = 1; return; }
 }
+
+int ocr_pages(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt_in,
+              const std::vector<ClassMask>* page_masks, tt_result** out);
 
 }  // namespace
 
@@ -430,7 +453,38 @@ int tt_ocr_pages(tt_engine* e, const tt_image* pages, int n_pages, tt_result** o
   return tt_ocr_pages_ex(e, pages, n_pages, nullptr, out);
 }
 
-int tt_ocr_pages_ex(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt_in, tt_result** out) {
+int tt_ocr_pages_ex(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt, tt_result** out) {
+  return ocr_pages(e, pages, n_pages, opt, nullptr, out);
+}
+
+int tt_ocr_pages_filtered(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
+                          const tt_char_filter* filters, int n_filters, tt_result** out) {
+  try {
+    if (n_filters == 0) return ocr_pages(e, pages, n_pages, opt, nullptr, out);
+    if (!filters) { set_error("tt_ocr_pages_filtered: filters is NULL but n_filters is " + std::to_string(n_filters)); return 1; }
+    if (n_filters != 1 && n_filters != n_pages) {
+      set_error("tt_ocr_pages_filtered: n_filters must be 0, 1 or n_pages (" + std::to_string(n_pages) + "), got " +
+                std::to_string(n_filters));
+      return 1;
+    }
+    std::vector<ClassMask> masks(std::max(n_pages, 0));
+    for (int i = 0; i < n_pages; ++i) {
+      const tt_char_filter& f = filters[n_filters == 1 ? 0 : i];
+      char_filter_mask(f.allow, f.block, masks[i].data());
+    }
+    return ocr_pages(e, pages, n_pages, opt, &masks, out);
+  } catch (const std::exception& ex) {
+    set_error(std::string("tt_ocr_pages_filtered: ") + ex.what());
+    return 1;
+  }
+}
+
+}  // extern "C"
+
+namespace {
+// tt_ocr_pages_ex and tt_ocr_pages_filtered (page_masks: one class mask per page, null without filters)
+int ocr_pages(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt_in,
+              const std::vector<ClassMask>* page_masks, tt_result** out) {
   try {
     tt_ocr_options opt{0, 0, nullptr, 0, 0};
     if (opt_in) opt = *opt_in;
@@ -480,8 +534,10 @@ int tt_ocr_pages_ex(tt_engine* e, const tt_image* pages, int n_pages, const tt_o
     std::vector<int> rcs(ws.size(), 0);
     std::vector<std::thread> workers;
     for (size_t w = 1; w < ws.size(); ++w)
-      workers.emplace_back([&, w] { slot_worker(*e, ws[w].g, ws[w].sidx, want, pages, opt, &q, &results, &rcs[w], &errs[w]); });
-    if (!ws.empty()) slot_worker(*e, ws[0].g, ws[0].sidx, want, pages, opt, &q, &results, &rcs[0], &errs[0]);
+      workers.emplace_back([&, w] {
+        slot_worker(*e, ws[w].g, ws[w].sidx, want, pages, opt, page_masks, &q, &results, &rcs[w], &errs[w]);
+      });
+    if (!ws.empty()) slot_worker(*e, ws[0].g, ws[0].sidx, want, pages, opt, page_masks, &q, &results, &rcs[0], &errs[0]);
     for (auto& w : workers) w.join();
     for (size_t w = 0; w < ws.size(); ++w)
       if (rcs[w]) { set_error("device " + std::to_string(e->devs[ws[w].g * kSlotsPerDevice]->device) + ": " + errs[w]); return 1; }
@@ -515,6 +571,9 @@ int tt_ocr_pages_ex(tt_engine* e, const tt_image* pages, int n_pages, const tt_o
     return 1;
   }
 }
+}  // namespace
+
+extern "C" {
 
 void tt_result_free(tt_result* r) {
   if (!r) return;
@@ -596,9 +655,10 @@ int tt_craft_tap(tt_engine* e, const char* name, float* out, long long capacity,
 }  // extern "C"
 
 namespace {
-// tt_parseq_forward and tt_parseq_forward_scores (pmax_out != null: the refinement head also writes the probabilities)
-int parseq_stage(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens, float* logits_out,
-                 int32_t* ids_out, float* pmax_out) {
+// tt_parseq_forward, tt_parseq_forward_scores and tt_parseq_forward_masked (pmax_out != null: the refinement head also
+// writes the probabilities; class_masks != null: [n][4] per-crop class masks)
+int parseq_stage(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens, const uint32_t* class_masks,
+                 float* logits_out, int32_t* ids_out, float* pmax_out) {
   try {
     if (!e) { set_error("tt_parseq_forward: null engine"); return 1; }
     if (n <= 0) return 0;
@@ -610,9 +670,13 @@ int parseq_stage(tt_engine* e, const uint8_t* crops, int n, const int32_t* force
       const int nc = std::min(kMaxCropsPerPass, n - c0);
       const size_t crop_bytes = static_cast<size_t>(nc) * 32 * 128 * 3;
       E_TRY(d.arena.reserve(d.parseq_bytes(nc) + crop_bytes + static_cast<size_t>(nc) * (128 * 96 * 2 + 4 * L) + (8u << 20) +
-                            (pmax_out ? sizeof(float) * nc * L : 0)));
+                            (pmax_out ? sizeof(float) * nc * L : 0) + (class_masks ? 16 * static_cast<size_t>(nc) : 0)));
       d.arena.reset();
       float* pmax = pmax_out ? d.arena.get<float>(static_cast<size_t>(nc) * L) : nullptr;
+      uint32_t* mask = class_masks ? d.arena.get<uint32_t>(4 * static_cast<size_t>(nc)) : nullptr;
+      if (mask)
+        E_CUDA(cudaMemcpyAsync(mask, class_masks + 4 * static_cast<size_t>(c0), 16 * static_cast<size_t>(nc), cudaMemcpyHostToDevice,
+                               d.stream));
       uint8_t* cu8 = d.arena.get<uint8_t>(crop_bytes);
       __nv_bfloat16* patches = d.arena.get<__nv_bfloat16>(static_cast<size_t>(nc) * 128 * 96);
       int* forced = forced_tokens ? d.arena.get<int>(static_cast<size_t>(nc) * (L - 1)) : nullptr;
@@ -623,7 +687,7 @@ int parseq_stage(tt_engine* e, const uint8_t* crops, int n, const int32_t* force
       E_TRY(patchify_u8(cu8, nc, patches, d.stream));
       float* logits = nullptr;
       int* ids = nullptr;
-      E_TRY(d.parseq_forward(patches, nc, forced, &logits, &ids, pmax));
+      E_TRY(d.parseq_forward(patches, nc, forced, &logits, &ids, pmax, mask));
       if (logits_out)
         E_CUDA(cudaMemcpy2DAsync(logits_out + static_cast<size_t>(c0) * L * d.w->pd.n_cls, sizeof(float) * d.w->pd.n_cls, logits,
                                  sizeof(float) * NC, sizeof(float) * d.w->pd.n_cls, static_cast<size_t>(nc) * L,
@@ -646,12 +710,17 @@ extern "C" {
 
 int tt_parseq_forward(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens, float* logits_out,
                       int32_t* ids_out) {
-  return parseq_stage(e, crops, n, forced_tokens, logits_out, ids_out, nullptr);
+  return parseq_stage(e, crops, n, forced_tokens, nullptr, logits_out, ids_out, nullptr);
 }
 
 int tt_parseq_forward_scores(tt_engine* e, const uint8_t* crops, int n, int32_t* ids_out, float* pmax_out) {
   if (!pmax_out) { set_error("tt_parseq_forward_scores: null pmax_out"); return 1; }
-  return parseq_stage(e, crops, n, nullptr, nullptr, ids_out, pmax_out);
+  return parseq_stage(e, crops, n, nullptr, nullptr, nullptr, ids_out, pmax_out);
+}
+
+int tt_parseq_forward_masked(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens, const uint32_t* class_masks,
+                             float* logits_out, int32_t* ids_out, float* pmax_out) {
+  return parseq_stage(e, crops, n, forced_tokens, class_masks, logits_out, ids_out, pmax_out);
 }
 
 int tt_postprocess_dev(tt_engine* e, const float* maps_dev, int batch, int H, int W, int* n_rects_total, void*) {

@@ -110,8 +110,11 @@ struct DeviceCtx {
   size_t craft_bytes(int B, int H, int W) const;
   // PARSeq: device bf16 patches [n*128][96] -> device fp32 logits [n][L][n_cls_pad] + int ids [n][L] (arena).
   // pmax_dev (nullable, device [n][L]): also the largest softmax probability of each refinement position.
+  // mask_dev (nullable, device [n][4] uint32, 16-byte aligned): per-crop class masks (tt_char_filter_mask); every greedy
+  // choice -- each AR step's fed-back token and the refinement's ids -- and pmax run over the allowed classes only.  The
+  // logits are not masked.
   cudaError_t parseq_forward(const __nv_bfloat16* patches_dev, int n, const int* forced_dev, float** logits_out,
-                             int** ids_out, float* pmax_dev = nullptr);
+                             int** ids_out, float* pmax_dev = nullptr, const uint32_t* mask_dev = nullptr);
   size_t parseq_bytes(int n) const;
 };
 

@@ -267,7 +267,7 @@ static cudaError_t lin(cudaStream_t s, const __nv_bfloat16* A, int lda, int M, i
 }
 
 cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const int* forced, float** logits_out,
-                                      int** ids_out, float* pmax_dev) {
+                                      int** ids_out, float* pmax_dev, const uint32_t* mask_dev) {
   using bf = __nv_bfloat16;
   const ParseqDims& pd = w->pd;
   const WeightFile& wf = w->parseq;
@@ -448,6 +448,7 @@ cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const
       float* la_h = logits_ar + static_cast<size_t>(c0) * L * NC;
       const int* forced_h = forced ? forced + static_cast<size_t>(c0) * (L - 1) : nullptr;
       const bf* mkv_h = mem_kv + static_cast<size_t>(c0) * 128 * 2 * D;
+      const uint32_t* mask_h = mask_dev ? mask_dev + static_cast<size_t>(c0) * 4 : nullptr;
       // lists hold crop indices relative to the half; step 0 works on all of them (no list)
       int* const cnt = act_n + half * L;
       const int* cur = (early && i > 0) ? act + static_cast<size_t>(i & 1) * n + c0 : nullptr;
@@ -457,7 +458,7 @@ cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const
       RUN(dec_self_attn(st, w->q_sa_table, w->sc_table, kv_table, tok_h, pd.eos_id, pd.n_tok, ab_h, hs));
       RUN(dec_dense_a2(w->dd, ab_h, nc, i, ts_h, qc_h, hs, cur, cur_n));
       RUN(dec_cross_attn(st, qc_h, mkv_h, ab_h, hs));
-      RUN(dec_dense_b(w->dd, ab_h, nc, i, ts_h, la_h, tok_h, forced_h, hs, cur, cur_n));
+      RUN(dec_dense_b(w->dd, ab_h, nc, i, ts_h, la_h, tok_h, forced_h, hs, cur, cur_n, mask_h));
       if (early && i + 1 < L)
         RUN(dec_compact(cur, cur_n, nc, tok_h, L, i + 1, pd.eos_id, act + static_cast<size_t>((i + 1) & 1) * n + c0, cnt + i + 1, hs));
       return cudaSuccess;
@@ -487,15 +488,15 @@ cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const
       RUN(stream_tail(st, n, logits_ar + static_cast<size_t>(i) * NC, L * NC));
       if (i + 1 < L)
         RUN(argmax_rows(logits_ar + static_cast<size_t>(i) * NC, n, pd.n_cls, L * NC, nullptr, 0, tokens + i + 1, L,
-                        forced ? forced + i : nullptr, L - 1, s));
+                        forced ? forced + i : nullptr, L - 1, s, mask_dev, 1));
     }
   }
   DecoderStep st{n, D, pd.dec_heads, L, 0, L, 1};
   RUN(stream_tail(st, R, logits, NC));
   if (pmax_dev)   // scores requested: the same ids plus each position's largest softmax probability, in the same launch
-    RUN(argmax_conf_rows(logits, R, pd.n_cls, NC, ids, pmax_dev, s));
+    RUN(argmax_conf_rows(logits, R, pd.n_cls, NC, ids, pmax_dev, s, mask_dev, L));
   else
-    RUN(argmax_rows(logits, R, pd.n_cls, NC, ids, 1, nullptr, 0, nullptr, 0, s));
+    RUN(argmax_rows(logits, R, pd.n_cls, NC, ids, 1, nullptr, 0, nullptr, 0, s, mask_dev, L));
   // decoder: 2 x 0.153 GMAC per crop over L + 1 passes; its floor is one read of the crop's memory K|V (128 x 768 bf16) per
   // pass the crop takes part in: L AR steps (fewer with the early exit) + the refinement
   {

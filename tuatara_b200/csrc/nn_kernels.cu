@@ -969,18 +969,24 @@ __global__ void __launch_bounds__(128) k_dec_attn_refine(const void* __restrict_
     }
 }
 
+// MASK: only the classes whose bit is set in the row's class mask compete (mask [rows / rows_per_mask][4], bit c & 31 of
+// word c >> 5).  Lane `lane` visits classes lane + 32 k, so its bit of word k is bit `lane`.
+template <bool MASK>
 __global__ void k_argmax(const float* __restrict__ logits, int rows, int n_cls, int ld, int* __restrict__ ids,
                          int ids_stride, int* __restrict__ next, int next_stride, const int* __restrict__ forced,
-                         int forced_stride) {
+                         int forced_stride, const uint32_t* __restrict__ mask, int rows_per_mask) {
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (row >= rows) return;
   const float* l = logits + static_cast<long long>(row) * ld;
+  uint4 mw = make_uint4(~0u, ~0u, ~0u, ~0u);
+  if constexpr (MASK) mw = *reinterpret_cast<const uint4*>(mask + static_cast<long long>(row / rows_per_mask) * 4);
+  const uint32_t mws[4] = {mw.x, mw.y, mw.z, mw.w};
   float best = -INFINITY;
   int bi = 0x7fffffff;
-  for (int c = lane; c < n_cls; c += 32) {
+  for (int c = lane, k = 0; c < n_cls; c += 32, ++k) {
     const float v = l[c];
-    if (v > best) { best = v; bi = c; }  // strictly greater: first max per lane
+    if ((!MASK || ((mws[k & 3] >> lane) & 1u)) && v > best) { best = v; bi = c; }  // strictly greater: first max per lane
   }
   for (int o = 16; o > 0; o >>= 1) {
     const float ov = __shfl_xor_sync(0xffffffffu, best, o);
@@ -997,18 +1003,23 @@ __global__ void k_argmax(const float* __restrict__ logits, int rows, int n_cls, 
 // Refinement head with scores: the argmax of k_argmax (same per-lane and cross-lane rules, so the ids are bit-identical)
 // and the row's largest softmax probability p = 1 / sum_c exp(l[c] - max), summed per lane in class order and then over
 // a fixed xor butterfly (every lane ends with the same bits), accurate expf: p is deterministic.  A row with a NaN
-// gets p = NaN.  The second pass re-reads the row from L1.
+// gets p = NaN.  The second pass re-reads the row from L1.  MASK: the argmax and the sum both skip the classes whose bit
+// is clear (p renormalised over the allowed classes); a mask that allows every class gives the bits of MASK = false.
+template <bool MASK>
 __global__ void k_argmax_conf(const float* __restrict__ logits, int rows, int n_cls, int ld, int* __restrict__ ids,
-                              float* __restrict__ pmax) {
+                              float* __restrict__ pmax, const uint32_t* __restrict__ mask, int rows_per_mask) {
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (row >= rows) return;
   const float* l = logits + static_cast<long long>(row) * ld;
+  uint4 mw = make_uint4(~0u, ~0u, ~0u, ~0u);
+  if constexpr (MASK) mw = *reinterpret_cast<const uint4*>(mask + static_cast<long long>(row / rows_per_mask) * 4);
+  const uint32_t mws[4] = {mw.x, mw.y, mw.z, mw.w};
   float best = -INFINITY;
   int bi = 0x7fffffff;
-  for (int c = lane; c < n_cls; c += 32) {
+  for (int c = lane, k = 0; c < n_cls; c += 32, ++k) {
     const float v = l[c];
-    if (v > best) { best = v; bi = c; }  // strictly greater: first max per lane
+    if ((!MASK || ((mws[k & 3] >> lane) & 1u)) && v > best) { best = v; bi = c; }  // strictly greater: first max per lane
   }
   for (int o = 16; o > 0; o >>= 1) {
     const float ov = __shfl_xor_sync(0xffffffffu, best, o);
@@ -1017,7 +1028,8 @@ __global__ void k_argmax_conf(const float* __restrict__ logits, int rows, int n_
   }
   if (bi >= n_cls) bi = 0;  // all-NaN row
   float sum = 0.f;
-  for (int c = lane; c < n_cls; c += 32) sum += expf(l[c] - best);
+  for (int c = lane, k = 0; c < n_cls; c += 32, ++k)
+    if (!MASK || ((mws[k & 3] >> lane) & 1u)) sum += expf(l[c] - best);
   for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
   if (lane == 0) {
     ids[row] = bi;
@@ -1240,17 +1252,26 @@ cudaError_t tokens_init(int* tokens, int n, int L, int bos, int pad, cudaStream_
 }
 
 cudaError_t argmax_rows(const float* logits, int rows, int n_cls, int ld, int* ids, int ids_stride, int* next,
-                        int next_stride, const int* forced, int forced_stride, cudaStream_t s) {
+                        int next_stride, const int* forced, int forced_stride, cudaStream_t s, const uint32_t* mask,
+                        int rows_per_mask) {
   if (rows <= 0) return cudaSuccess;
-  k_argmax<<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, ids_stride, next, next_stride, forced,
-                                          forced_stride);
+  if (mask)
+    k_argmax<true><<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, ids_stride, next, next_stride, forced,
+                                                  forced_stride, mask, rows_per_mask);
+  else
+    k_argmax<false><<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, ids_stride, next, next_stride, forced,
+                                                   forced_stride, nullptr, 1);
   TT_LAUNCH_CHECK();
   return cudaSuccess;
 }
 
-cudaError_t argmax_conf_rows(const float* logits, int rows, int n_cls, int ld, int* ids, float* pmax, cudaStream_t s) {
+cudaError_t argmax_conf_rows(const float* logits, int rows, int n_cls, int ld, int* ids, float* pmax, cudaStream_t s,
+                             const uint32_t* mask, int rows_per_mask) {
   if (rows <= 0) return cudaSuccess;
-  k_argmax_conf<<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, pmax);
+  if (mask)
+    k_argmax_conf<true><<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, pmax, mask, rows_per_mask);
+  else
+    k_argmax_conf<false><<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, pmax, nullptr, 1);
   TT_LAUNCH_CHECK();
   return cudaSuccess;
 }

@@ -60,11 +60,16 @@ cudaError_t dec_cross_attn(const DecoderStep& st, const __nv_bfloat16* q, const 
                            __nv_bfloat16* out, cudaStream_t s);
 // argmax over the first n_cls of ld logits per row (first max wins) -> ids[row*ids_stride]; when
 // `forced` != null the value written to next_tokens comes from forced instead of the argmax.
+// mask (nullable, device [rows / rows_per_mask][4] uint32, 16-byte aligned): the class mask of each group of
+// rows_per_mask consecutive rows (1: row = crop; L: row = crop * L + t); only classes whose bit is set compete.
 cudaError_t argmax_rows(const float* logits, int rows, int n_cls, int ld, int* ids, int ids_stride,
-                        int* next_tokens, int next_stride, const int* forced, int forced_stride, cudaStream_t s);
+                        int* next_tokens, int next_stride, const int* forced, int forced_stride, cudaStream_t s,
+                        const uint32_t* mask = nullptr, int rows_per_mask = 1);
 // argmax_rows' ids (same tie and NaN rules, bit-identical) fused with the largest softmax probability of the row,
 // pmax[row] = 1 / sum_c exp(logits[row][c] - max) in fp32 (deterministic; NaN for a row holding a NaN).  ids, pmax [rows].
-cudaError_t argmax_conf_rows(const float* logits, int rows, int n_cls, int ld, int* ids, float* pmax, cudaStream_t s);
+// mask as in argmax_rows: the max and the sum run over the allowed classes only.
+cudaError_t argmax_conf_rows(const float* logits, int rows, int n_cls, int ld, int* ids, float* pmax, cudaStream_t s,
+                             const uint32_t* mask = nullptr, int rows_per_mask = 1);
 // u8 crops [n][32][128][3] -> bf16 patch rows [n*128][96] (raw 0..255), k = c*32 + (y%4)*8 + x%8
 cudaError_t tokens_init(int* tokens, int n, int L, int bos, int pad, cudaStream_t s);
 // AR early exit: the crops of (active_in, *n_in) -- null: all n crops -- whose token at position `pos` is not EOS, in the

@@ -4,6 +4,10 @@
 
 namespace tt {
 
+namespace {
+constexpr int kNumClasses = 95;   // PARSeq head outputs (TT_NUM_CLASSES)
+}
+
 const TokenizerTable& tokenizer_table() {
   static const TokenizerTable table = [] {
     TokenizerTable t;
@@ -55,6 +59,21 @@ void decode_ids_scored(const int32_t* ids, const float* p, int len, std::string*
   double prod = 1.0;
   for (int i = 0; i <= end; ++i) prod *= static_cast<double>(p[i]);
   *conf = static_cast<float>(prod);
+}
+
+void char_filter_mask(const char* allow, const char* block, uint32_t mask[4]) {
+  const TokenizerTable& t = tokenizer_table();
+  auto holds = [](const char* s, char ch) {
+    for (; *s; ++s)
+      if (*s == ch) return true;
+    return false;
+  };
+  for (int w = 0; w < 4; ++w) mask[w] = 0;
+  for (int c = 0; c < kNumClasses; ++c) {
+    const char ch = t.itos[c];
+    const bool ok = c == 0 || c == t.eos_id || ((!allow || holds(allow, ch)) && (!block || !holds(block, ch)));
+    if (ok) mask[c >> 5] |= 1u << (c & 31);
+  }
 }
 
 }  // namespace tt

@@ -27,4 +27,9 @@ std::string decode_ids(const int32_t* ids, int len);
 void decode_ids_scored(const int32_t* ids, const float* p, int len, std::string* text, std::vector<float>* char_conf,
                        float* conf);
 
+// Class mask of a character filter (tt_char_filter_mask): bit c & 31 of mask[c >> 5] is set when class c (0..94) is
+// allowed.  Classes 0 and eos_id print nothing and are always allowed; any other class c is allowed iff (allow is null
+// or holds itos[c]) and (block is null or does not hold itos[c]).  Characters no class prints are ignored; mask[3] = 0.
+void char_filter_mask(const char* allow, const char* block, uint32_t mask[4]);
+
 }  // namespace tt
