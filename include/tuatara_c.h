@@ -250,6 +250,27 @@ TT_API int tt_enc_mlp_dev(void* x_hi, void* x_lo, float* stats, long long M, con
 TT_API int tt_conv_dev(const void* src0, int C0, const void* src1, int C1, int batch, int H, int W, int taps, int dil,
                 const void* weight, const float* bias, int Cout, int relu, void* out, int BN, int resident,
                 void* stream);
+/* Kernel tests of the PARSeq attention family: each calls the launcher the engine calls.  All pointers are device
+ * pointers; bf16 buffers are passed as void*.
+ * tt_attn_enc_dev: encoder self attention, T = 128 tokens, head dim 64 (D = 64 * heads): qkv bf16 [crops*128][3D]
+ *   (q | k | v, head-major inside each) -> out bf16 [crops*128][D]; onepass != 0 reads the S row from TMEM once. */
+TT_API int tt_attn_enc_dev(const void* qkv, void* out, int crops, int D, int heads, int onepass, void* stream);
+/* out fp32 [L][L][n_tok][heads] = q_table fp32 [L][D] . K of kv_table bf16 [L][n_tok][2D] (K | V), per head / sqrt(32) */
+TT_API int tt_dec_score_table_dev(const float* q_table, const void* kv_table, int L, int n_tok, int D, int heads, float* out,
+                                  void* stream);
+/* Decoder self attention of query positions [p0, p0+np): key j of crop c is row (j, tokens[c][j]) of kv_table
+ * bf16 [L][n_tok][2D]; q_table fp32 [L][D]; tokens int32 [n_crops][L].  refine == 0: keys j <= p (np == 1 with a
+ * score table sc_table fp32 [L][L][n_tok][heads] takes the AR-step kernel, which alone honours active / n_act: output row
+ * = slot, crop = active[slot], slots < *n_act); refine != 0: j != p+1 and j before the first eos_id among tokens[c][1..].
+ * out bf16 [n_crops*np][D] (crop-major, then position).  active / n_act may be NULL. */
+TT_API int tt_dec_self_attn_dev(int n_crops, int D, int heads, int L, int p0, int np, int refine, const int32_t* active,
+                                const int32_t* n_act, const float* q_table, const float* sc_table, const void* kv_table,
+                                const int32_t* tokens, int eos_id, int n_tok, void* out, void* stream);
+/* Decoder cross attention over the 128 memory rows of each crop, no mask: q bf16 [n_crops*np][D], mem_kv bf16
+ * [n_crops][128][2D] (K | V) -> out bf16 [n_crops*np][D].  active / n_act (may be NULL) as above, honoured when the
+ * per-position kernel runs (np == 1, or D == 192): q / out rows by slot, memory by crop. */
+TT_API int tt_dec_cross_attn_dev(int n_crops, int D, int heads, int L, int p0, int np, const int32_t* active,
+                                 const int32_t* n_act, const void* q, const void* mem_kv, void* out, void* stream);
 /* Batched device-side post-processing (bench): maps_dev [batch][H][W][2] fp32. Returns total rects. */
 TT_API int tt_postprocess_dev(tt_engine* e, const float* maps_dev, int batch, int H, int W, int* n_rects_total,
                        void* stream);

@@ -13,6 +13,7 @@
 #include "engine.h"
 #include "gemm_tc.cuh"
 #include "geometry.h"
+#include "nn_kernels.cuh"
 #include "postprocess.cuh"
 #include "resize.cuh"
 #include "tokenizer.h"
@@ -401,6 +402,42 @@ int tt_conv_dev(const void* src0, int C0, const void* src1, int C1, int batch, i
     Epilogue e;
     e.bias = bias; e.act = relu ? ACT_RELU : ACT_NONE; e.out = out; e.out_type = OUT_BF16; e.ldc = Cout;
     return conv_forward(c, e, static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : 1;
+  });
+}
+
+int tt_attn_enc_dev(const void* qkv, void* out, int crops, int D, int heads, int onepass, void* stream) {
+  return guarded([&]() -> int {
+    return attention_enc(static_cast<const __nv_bfloat16*>(qkv), static_cast<__nv_bfloat16*>(out), crops, D, heads,
+                         onepass != 0, static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : 1;
+  });
+}
+
+int tt_dec_score_table_dev(const float* q_table, const void* kv_table, int L, int n_tok, int D, int heads, float* out,
+                           void* stream) {
+  return guarded([&]() -> int {
+    return dec_score_table(q_table, static_cast<const __nv_bfloat16*>(kv_table), L, n_tok, D, heads, out,
+                           static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : 1;
+  });
+}
+
+int tt_dec_self_attn_dev(int n_crops, int D, int heads, int L, int p0, int np, int refine, const int32_t* active,
+                         const int32_t* n_act, const float* q_table, const float* sc_table, const void* kv_table,
+                         const int32_t* tokens, int eos_id, int n_tok, void* out, void* stream) {
+  return guarded([&]() -> int {
+    DecoderStep st{n_crops, D, heads, L, p0, np, refine};
+    st.active = active; st.n_act = n_act;
+    return dec_self_attn(st, q_table, sc_table, static_cast<const __nv_bfloat16*>(kv_table), tokens, eos_id, n_tok,
+                         static_cast<__nv_bfloat16*>(out), static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : 1;
+  });
+}
+
+int tt_dec_cross_attn_dev(int n_crops, int D, int heads, int L, int p0, int np, const int32_t* active, const int32_t* n_act,
+                          const void* q, const void* mem_kv, void* out, void* stream) {
+  return guarded([&]() -> int {
+    DecoderStep st{n_crops, D, heads, L, p0, np, 0};
+    st.active = active; st.n_act = n_act;
+    return dec_cross_attn(st, static_cast<const __nv_bfloat16*>(q), static_cast<const __nv_bfloat16*>(mem_kv),
+                          static_cast<__nv_bfloat16*>(out), static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : 1;
   });
 }
 

@@ -295,6 +295,7 @@ cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const
   const bool mlp_fuse = lnf && !(mf_env && std::atoi(mf_env) == 0) && enc_mlp_supported(D, pd.mlp);
   const char* pf_env = std::getenv("TT_ENC_PROJFUSE");   // 0: the attention output projection stays a GEMM launch (A/B runs)
   const bool proj_fuse = !(pf_env && std::atoi(pf_env) == 0);
+  static const bool attn_onepass = !(std::getenv("TT_ATTN_ONEPASS") && std::atoi(std::getenv("TT_ATTN_ONEPASS")) == 0);  // 0: A/B runs
   ARENA_GET(x, float, Mc * D);       // fp32 residual stream (unfused) / the lo half of the split stream (fused; first half of the buffer)
   ARENA_GET(h, bf, Mc * D);          // LayerNorm output (unfused) / the hi half of the split stream = bf16(x) (fused)
   bf* const x_lo = reinterpret_cast<bf*>(x);
@@ -347,7 +348,7 @@ cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const
       const std::string p = "b" + std::to_string(i) + ".";
       if (!lnf) RUN(layernorm(x, Mi, D, wf.f32(p + "ln1.g"), wf.f32(p + "ln1.b"), 1e-6f, h, nullptr, 0, s));
       RUN(ln_gemm(p + "qkv", Mi, 3 * D, ACT_NONE, qkv));
-      RUN(attention_enc(qkv, att, nc, D, pd.enc_heads, s));
+      RUN(attention_enc(qkv, att, nc, D, pd.enc_heads, attn_onepass, s));
       if (mlp_fuse && proj_fuse) {
         // proj + residual + fc1 -> GELU -> fc2 + residual in one kernel: x1 never leaves the SM either (enc_mlp.cu)
         EncMlpWeights mw;

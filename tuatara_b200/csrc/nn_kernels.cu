@@ -1110,7 +1110,8 @@ cudaError_t layernorm(const float* x, int rows, int D, const float* gamma, const
   return cudaSuccess;
 }
 
-cudaError_t attention_enc(const __nv_bfloat16* qkv, __nv_bfloat16* out, int crops, int D, int heads, cudaStream_t s) {
+cudaError_t attention_enc(const __nv_bfloat16* qkv, __nv_bfloat16* out, int crops, int D, int heads, bool onepass,
+                          cudaStream_t s) {
   if (crops <= 0) return cudaSuccess;
   if (D != heads * 64) { set_error("attention_enc: head dim must be 64"); return cudaErrorInvalidValue; }
   CUtensorMap tm;
@@ -1118,7 +1119,6 @@ cudaError_t attention_enc(const __nv_bfloat16* qkv, __nv_bfloat16* out, int crop
   const cuuint64_t strides[1] = {static_cast<cuuint64_t>(3 * D) * 2};
   const cuuint32_t box[2] = {64, 128};
   if (!make_tmap_bf16(&tm, qkv, 2, dims, strides, box, 128)) return cudaErrorInvalidValue;
-  static const bool onepass = !(std::getenv("TT_ATTN_ONEPASS") && std::atoi(std::getenv("TT_ATTN_ONEPASS")) == 0);  // 0: A/B runs
   const void* fn = onepass ? reinterpret_cast<const void*>(k_attn_enc<true>) : reinterpret_cast<const void*>(k_attn_enc<false>);
   TT_CUDA_TRY(ensure_dynamic_smem(fn, kAttnSmem));
   const float scale_log2e = 0.125f * 1.4426950408889634f;  // head_dim^-0.5 * log2(e)

@@ -27,8 +27,10 @@ cudaError_t layernorm(const float* x, int rows, int D, const float* gamma, const
 
 // Encoder self-attention for T = 128 tokens, head dim 64: qkv bf16 [crops*128][3*D] (timm layout
 // q|k|v, head-major inside each) -> out bf16 [crops*128][D].  One CTA per (head, crop); QK^T and PV
-// on tcgen05 with S/O in TMEM, softmax in registers.
-cudaError_t attention_enc(const __nv_bfloat16* qkv, __nv_bfloat16* out, int crops, int D, int heads, cudaStream_t s);
+// on tcgen05 with S/O in TMEM, softmax in registers.  onepass: the S row is read from TMEM once (k_attn_enc<true>, the
+// default); false selects the two-pass kernel.
+cudaError_t attention_enc(const __nv_bfloat16* qkv, __nv_bfloat16* out, int crops, int D, int heads, bool onepass,
+                          cudaStream_t s);
 
 struct DecoderStep {
   int n_crops;
