@@ -54,6 +54,7 @@ struct ScoredItem {
   float confidence = -1.f;               // word confidence; -1 when the word was not recognised
   float detection_score = 0.f;           // the box's maximum normalised text score (>= text_threshold)
   std::vector<float> char_confidence;    // one probability per character of text
+  int angle = 0;                         // image_to_data_oriented: the candidate read (0, 90, 180, 270 ccw)
 };
 
 // Character filter (tt_char_filter, INTEGRATION.md section 7): recognition only produces characters that are in `allow`
@@ -88,7 +89,8 @@ namespace detail {
 // opt == nullptr: plain tt_ocr_pages.  filters != nullptr: tt_ocr_pages_filtered (one filter, or one per page).
 inline tt_result* ocr_pages(const std::vector<ImageView>& images, const std::string& weights_dir,
                             const std::string& outputs_dir, const tt_ocr_options* opt,
-                            const std::vector<CharFilter>* filters = nullptr) {
+                            const std::vector<CharFilter>* filters = nullptr,
+                            const std::vector<int>* rotation_info = nullptr) {
   if (weights_dir.empty()) { std::cerr << "Please provide a value for weights_dir" << std::endl; return nullptr; }
   if (outputs_dir.empty()) { std::cerr << "Please provide a value for outputs_dir" << std::endl; return nullptr; }
   std::vector<tt_image> pages(images.size());
@@ -101,12 +103,17 @@ inline tt_result* ocr_pages(const std::vector<ImageView>& images, const std::str
   if (!e) { std::cerr << "error loading the models: " << tt_last_error() << std::endl; return nullptr; }
   tt_result* r = nullptr;
   int rc = 0;
-  if (filters) {
+  if (filters || rotation_info) {
     std::vector<tt_char_filter> f;
-    for (const CharFilter& cf : *filters) f.push_back(tt_char_filter{cf.allow, cf.block});
+    if (filters)
+      for (const CharFilter& cf : *filters) f.push_back(tt_char_filter{cf.allow, cf.block});
     const tt_ocr_options none = {};
-    rc = tt_ocr_pages_filtered(e, pages.data(), static_cast<int>(pages.size()), opt ? opt : &none, f.data(),
-                               static_cast<int>(f.size()), &r);
+    rc = rotation_info
+             ? tt_ocr_pages_oriented(e, pages.data(), static_cast<int>(pages.size()), opt ? opt : &none, f.data(),
+                                     static_cast<int>(f.size()), rotation_info->data(),
+                                     static_cast<int>(rotation_info->size()), &r)
+             : tt_ocr_pages_filtered(e, pages.data(), static_cast<int>(pages.size()), opt ? opt : &none, f.data(),
+                                     static_cast<int>(f.size()), &r);
   } else {
     rc = opt ? tt_ocr_pages_ex(e, pages.data(), static_cast<int>(pages.size()), opt, &r)
              : tt_ocr_pages(e, pages.data(), static_cast<int>(pages.size()), &r);
@@ -134,11 +141,12 @@ inline std::vector<std::vector<OutputItem>> batch_items(const std::vector<ImageV
 }
 
 inline std::vector<std::vector<ScoredItem>> scored_items(const std::vector<ImageView>& images, const std::string& weights_dir,
-                                                         const std::string& outputs_dir, const std::vector<CharFilter>* filters) {
+                                                         const std::string& outputs_dir, const std::vector<CharFilter>* filters,
+                                                         const std::vector<int>* rotation_info = nullptr) {
   std::vector<std::vector<ScoredItem>> out;
   tt_ocr_options opt = {};
   opt.with_scores = 1;
-  tt_result* r = ocr_pages(images, weights_dir, outputs_dir, &opt, filters);
+  tt_result* r = ocr_pages(images, weights_dir, outputs_dir, &opt, filters, rotation_info);
   if (!r) return out;
   out.resize(r->n_pages);
   for (int p = 0; p < r->n_pages; ++p)
@@ -149,7 +157,8 @@ inline std::vector<std::vector<ScoredItem>> scored_items(const std::vector<Image
       s.bbox.assign(it.bbox, it.bbox + 4);
       const float* cc = nullptr;
       int n = 0;
-      if (tt_item_scores(r, p, k, &s.confidence, &s.detection_score, &cc, &n) != 0) {
+      if (tt_item_scores(r, p, k, &s.confidence, &s.detection_score, &cc, &n) != 0 ||
+          (rotation_info && !rotation_info->empty() && tt_item_angle(r, p, k, &s.angle) != 0)) {
         std::cerr << "tuatara: " << tt_last_error() << std::endl;
         tt_result_free(r);
         return std::vector<std::vector<ScoredItem>>{};
@@ -203,6 +212,27 @@ inline std::vector<ScoredItem> image_to_data_scored(const ImageView& image, cons
                                                     const std::string& outputs_dir, const CharFilter& filter) {
   std::vector<std::vector<ScoredItem>> pages =
       image_to_data_scored_batch({image}, weights_dir, outputs_dir, std::vector<CharFilter>{filter});
+  return pages.empty() ? std::vector<ScoredItem>{} : pages[0];
+}
+
+// Rotation candidates (tt_ocr_pages_oriented, INTEGRATION.md section 8): every word is also read turned by each angle of
+// rotation_info (90, 180, 270 degrees counter-clockwise) and the reading with the highest confidence is kept;
+// ScoredItem::angle says which.  filters: none (empty), one for every page, or one per page.  Same soft failures as
+// image_to_data; an invalid angle prints the error and returns {}.
+inline std::vector<std::vector<ScoredItem>> image_to_data_oriented_batch(const std::vector<ImageView>& images,
+                                                                         const std::string& weights_dir,
+                                                                         const std::string& outputs_dir,
+                                                                         const std::vector<int>& rotation_info,
+                                                                         const std::vector<CharFilter>& filters = {}) {
+  return detail::scored_items(images, weights_dir, outputs_dir, filters.empty() ? nullptr : &filters, &rotation_info);
+}
+
+inline std::vector<ScoredItem> image_to_data_oriented(const ImageView& image, const std::string& weights_dir,
+                                                      const std::string& outputs_dir, const std::vector<int>& rotation_info,
+                                                      const CharFilter& filter = CharFilter()) {
+  const bool filtered = filter.allow != nullptr || filter.block != nullptr;
+  std::vector<std::vector<ScoredItem>> pages = image_to_data_oriented_batch(
+      {image}, weights_dir, outputs_dir, rotation_info, filtered ? std::vector<CharFilter>{filter} : std::vector<CharFilter>{});
   return pages.empty() ? std::vector<ScoredItem>{} : pages[0];
 }
 

@@ -132,6 +132,21 @@ TT_API int tt_ocr_pages_filtered(tt_engine* e, const tt_image* pages, int n_page
  * Every output pointer may be NULL. */
 TT_API int tt_item_scores(const tt_result* r, int page, int item, float* conf, float* det_score, const float** char_conf,
                           int* n_chars);
+/* Rotation candidates (INTEGRATION.md section 8): tt_ocr_pages_filtered where every word is also read turned 90, 180 or
+ * 270 degrees counter-clockwise, as listed in rotation_info (n_rotations distinct values from {90, 180, 270}, any order).
+ * Candidate 0, the crop tt_ocr_pages_filtered reads, is always included; candidates are ordered 0, 90, 180, 270.  With
+ * rectify == 0 candidate a is cv::resize(cv::rotate(roi, a), 128 x 32); with rectify == 1 it is the warp of the box's
+ * quad with its corners shifted cyclically by a / 90.  Each candidate gets the conf of tt_item_scores (under its page's
+ * filter); a later candidate replaces the best so far only when its conf is strictly greater.  The item's text (and,
+ * with with_scores, conf and char_conf) are the winner's; bbox, det_score and item order do not change.  Read the angle
+ * with tt_item_angle.  n_rotations == 0 (rotation_info may be NULL) is tt_ocr_pages_filtered; any other value outside
+ * {90, 180, 270}, or one given twice, is an error that names it, reported before any device work. */
+TT_API int tt_ocr_pages_oriented(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
+                                 const tt_char_filter* filters, int n_filters, const int* rotation_info, int n_rotations,
+                                 tt_result** out);
+/* The angle (0, 90, 180 or 270) of the candidate that was read for item `item` of page `page`, -1 when the item was not
+ * recognised (detect_only).  An error on a result not made by tt_ocr_pages_oriented with n_rotations > 0. */
+TT_API int tt_item_angle(const tt_result* r, int page, int item, int* angle);
 /* Kernel launches issued by this library so far (bench.py's gpu_launches). */
 TT_API unsigned long long tt_launch_count(void);
 
@@ -178,6 +193,9 @@ TT_API int tt_postprocess(const float* maps, int H, int W, const tt_config* cfg,
 /* Crop + resize to 128x32 (tuatara.cpp:416, :440-441). rects_xywh already clamped to the image.
  * out: [n][32][128][3] u8 in the caller's channel order. */
 TT_API int tt_crop_resize(const tt_image* image, const int32_t* rects_xywh, int n, uint8_t* out);
+/* tt_crop_resize with each crop turned angles[i] degrees counter-clockwise (0, 90, 180 or 270) before the resize:
+ * cv::resize(cv::rotate(roi, code), (128, 32)).  Angle 0 gives tt_crop_resize's bytes. */
+TT_API int tt_crop_resize_rotated(const tt_image* image, const int32_t* rects_xywh, const int32_t* angles, int n, uint8_t* out);
 /* Per-slice parity of the CRAFT forward (SURVEY 8d): a named activation of the LAST tt_craft_forward call on this
  * engine as fp32 [H][W][C] (names: relu2_2, relu3_2, relu4_3, relu5_3, fc7, up1, up2, up3, up4 -- upstream CRAFT's
  * skip / U-net tensors).  out == NULL only reports dims_out = {H, W, C}.  Test entry point: not thread safe against
@@ -271,6 +289,11 @@ TT_API int tt_dec_self_attn_dev(int n_crops, int D, int heads, int L, int p0, in
  * per-position kernel runs (np == 1, or D == 192): q / out rows by slot, memory by crop. */
 TT_API int tt_dec_cross_attn_dev(int n_crops, int D, int heads, int L, int p0, int np, const int32_t* active,
                                  const int32_t* n_act, const void* q, const void* mem_kv, void* out, void* stream);
+/* Kernel test of the rotation choice (tt_ocr_pages_oriented): ids int32 / pmax fp32 [n_words * n_candidates][26], crop
+ * w * n_candidates + r being candidate r (angle angles[r], host array) of word w.  Writes the winner's ids_out [n_words][26],
+ * pmax_out [n_words][26] (nullable) and angle_out [n_words].  Device pointers except angles. */
+TT_API int tt_orient_select_dev(const int32_t* ids, const float* pmax, int n_words, const int32_t* angles, int n_candidates,
+                                int32_t* ids_out, float* pmax_out, int32_t* angle_out, void* stream);
 /* Batched device-side post-processing (bench): maps_dev [batch][H][W][2] fp32. Returns total rects. */
 TT_API int tt_postprocess_dev(tt_engine* e, const float* maps_dev, int batch, int H, int W, int* n_rects_total,
                        void* stream);

@@ -196,12 +196,20 @@ def postprocess(maps: np.ndarray, cfg: _native.tt_config | None = None, want_lab
                 rect_labels=rlabels[: n_rects.value].copy())
 
 
-def crop_resize(image: np.ndarray, rects_xywh) -> np.ndarray:
-    """Batched crop + 128x32 bilinear resize on the GPU -> uint8 [n, 32, 128, 3]."""
+def crop_resize(image: np.ndarray, rects_xywh, angles=None) -> np.ndarray:
+    """Batched crop + 128x32 bilinear resize on the GPU -> uint8 [n, 32, 128, 3].  angles: None, or one angle per rect
+    from {0, 90, 180, 270}: the crop is turned that many degrees counter-clockwise before the resize
+    (tt_crop_resize_rotated, cv2.resize(cv2.rotate(roi, code), (128, 32)))."""
     r = np.ascontiguousarray(np.asarray(rects_xywh, np.int32).reshape(-1, 4))
     out = np.empty((len(r), 32, 128, 3), np.uint8)
     im = _native.image_struct(image)
-    check(lib().tt_crop_resize(C.byref(im), ptr(r), len(r), ptr(out)), "tt_crop_resize")
+    if angles is None:
+        check(lib().tt_crop_resize(C.byref(im), ptr(r), len(r), ptr(out)), "tt_crop_resize")
+    else:
+        a = np.ascontiguousarray(np.asarray(angles, np.int32).reshape(-1))
+        if len(a) != len(r):
+            raise ValueError(f"crop_resize: {len(r)} rects but {len(a)} angles")
+        check(lib().tt_crop_resize_rotated(C.byref(im), ptr(r), ptr(a), len(r), ptr(out)), "tt_crop_resize_rotated")
     return out
 
 
@@ -246,14 +254,17 @@ class Engine:
     __del__ = close
 
     def ocr_pages(self, images: list, score_override: list | None = None, detect_only: bool = False,
-                  scores: bool = False, *, allowlist=None, blocklist=None) -> list[list[dict]]:
+                  scores: bool = False, *, allowlist=None, blocklist=None, rotation_info=None) -> list[list[dict]]:
         """images: uint8 [H,W,3] numpy arrays (host) or torch CUDA tensors (already on the device).
         score_override: optional per-page float32 [h32/2, w32/2, 2] maps (numpy or CUDA tensors, or
         None entries) that replace CRAFT's output after CRAFT has run (benchmark / parity tests).
         scores: every item also carries conf (word confidence 0..1, None when not recognised), det_score (the
         detection score of its box) and char_conf (one probability per character of text); see tt_item_scores.
         allowlist / blocklist: character filters (tt_ocr_pages_filtered): recognition only produces characters in
-        allowlist and not in blocklist.  Each is None, a str for every page, or a list with one str or None per page."""
+        allowlist and not in blocklist.  Each is None, a str for every page, or a list with one str or None per page.
+        rotation_info: an iterable of angles from {90, 180, 270} (tt_ocr_pages_oriented): each word is also read turned
+        that many degrees counter-clockwise and the candidate with the highest word confidence wins; every item then
+        carries "angle" (0, 90, 180 or 270; -1 when not recognised).  An empty iterable reads every word upright."""
         n = len(images)
         on_dev = n > 0 and not isinstance(images[0], np.ndarray)
         if on_dev:
@@ -280,7 +291,11 @@ class Engine:
             opt.score_override = ptrs
         res = C.POINTER(_native.tt_result)()
         filters = _filters(allowlist, blocklist, n)
-        if filters is None:
+        rot = None if rotation_info is None else _rotations(rotation_info)
+        if rot is not None:
+            check(lib().tt_ocr_pages_oriented(self._h, arr, n, C.byref(opt), filters, len(filters) if filters else 0,
+                                              rot, len(rot), C.byref(res)), "tt_ocr_pages_oriented")
+        elif filters is None:
             check(lib().tt_ocr_pages_ex(self._h, arr, n, C.byref(opt), C.byref(res)), "tt_ocr_pages_ex")
         else:
             check(lib().tt_ocr_pages_filtered(self._h, arr, n, C.byref(opt), filters, len(filters), C.byref(res)),
@@ -294,6 +309,9 @@ class Engine:
                 if scores:
                     for i, item in enumerate(out[-1]):
                         item.update(_item_scores(res, p, i))
+                if rot is not None:
+                    for i, item in enumerate(out[-1]):
+                        item["angle"] = _item_angle(res, p, i) if len(rot) else (-1 if detect_only else 0)
             return out
         finally:
             lib().tt_result_free(res)
@@ -356,6 +374,22 @@ def _class_masks(class_masks, n: int) -> np.ndarray:
     return m
 
 
+def _rotations(rotation_info):
+    """rotation_info keyword -> an int32 ctypes array (the values are checked by tt_ocr_pages_oriented)."""
+    if isinstance(rotation_info, (str, bytes)) or not hasattr(rotation_info, "__iter__"):
+        raise TypeError("rotation_info: expected an iterable of ints from {90, 180, 270}")
+    vals = list(rotation_info)
+    if not all(isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in vals):
+        raise TypeError(f"rotation_info: expected ints, got {vals!r}")
+    return (C.c_int * len(vals))(*[int(v) for v in vals])
+
+
+def _item_angle(res, page: int, item: int) -> int:
+    a = C.c_int()
+    check(lib().tt_item_angle(res, page, item, C.byref(a)), "tt_item_angle")
+    return a.value
+
+
 def _item_scores(res, page: int, item: int) -> dict:
     conf, det = C.c_float(), C.c_float()
     cc, n = C.POINTER(C.c_float)(), C.c_int()
@@ -377,11 +411,12 @@ def _engine_for(weights_dir: str) -> Engine:
 
 
 def image_to_data(image: np.ndarray, weights_dir: str, outputs_dir: str, *, allowlist: str | None = None,
-                  blocklist: str | None = None) -> list[dict]:
+                  blocklist: str | None = None, rotation_info=None) -> list[dict]:
     """Same call as the reference's ``pytuatara.image_to_data`` (bindings/python.cpp:43-57):
     uint8 [H, W, 3] in, list of ``dict(text=str, bbox=[4 floats])`` out.  Empty directory
     strings print to stderr and return [] like tuatara.cpp:315-323.  allowlist / blocklist: recognition only produces
-    characters in allowlist and not in blocklist (INTEGRATION.md section 7)."""
+    characters in allowlist and not in blocklist (INTEGRATION.md section 7).  rotation_info: angles from {90, 180, 270}
+    at which each word is also read; items then carry "angle" (INTEGRATION.md section 8)."""
     import sys
 
     if not weights_dir:
@@ -392,18 +427,20 @@ def image_to_data(image: np.ndarray, weights_dir: str, outputs_dir: str, *, allo
         return []
     if image.ndim != 3:
         raise RuntimeError("Input array should have 3 dimensions")
-    return _engine_for(weights_dir).ocr_pages([image], allowlist=allowlist, blocklist=blocklist)[0]
+    return _engine_for(weights_dir).ocr_pages([image], allowlist=allowlist, blocklist=blocklist,
+                                              rotation_info=rotation_info)[0]
 
 
 def images_to_data(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".", *, allowlist=None,
-                   blocklist=None) -> list[list[dict]]:
+                   blocklist=None, rotation_info=None) -> list[list[dict]]:
     """Additive batch API: one call, many pages (sharded over the engine's GPUs).  allowlist / blocklist: None, a str
     for every page, or a list with one str or None per page."""
-    return _engine_for(weights_dir).ocr_pages(list(images), allowlist=allowlist, blocklist=blocklist)
+    return _engine_for(weights_dir).ocr_pages(list(images), allowlist=allowlist, blocklist=blocklist,
+                                              rotation_info=rotation_info)
 
 
 def image_to_data_scored(image: np.ndarray, weights_dir: str, outputs_dir: str, *, allowlist: str | None = None,
-                         blocklist: str | None = None) -> list[dict]:
+                         blocklist: str | None = None, rotation_info=None) -> list[dict]:
     """image_to_data whose items also carry ``conf`` (word confidence 0..1), ``det_score`` (the detection score of the
     box) and ``char_conf`` (one probability per character of ``text``).  Same inputs, errors and soft failures;
     ``text`` and ``bbox`` are what image_to_data returns."""
@@ -417,10 +454,12 @@ def image_to_data_scored(image: np.ndarray, weights_dir: str, outputs_dir: str, 
         return []
     if image.ndim != 3:
         raise RuntimeError("Input array should have 3 dimensions")
-    return _engine_for(weights_dir).ocr_pages([image], scores=True, allowlist=allowlist, blocklist=blocklist)[0]
+    return _engine_for(weights_dir).ocr_pages([image], scores=True, allowlist=allowlist, blocklist=blocklist,
+                                              rotation_info=rotation_info)[0]
 
 
 def images_to_data_scored(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".", *, allowlist=None,
-                          blocklist=None) -> list[list[dict]]:
+                          blocklist=None, rotation_info=None) -> list[list[dict]]:
     """Batch variant of image_to_data_scored."""
-    return _engine_for(weights_dir).ocr_pages(list(images), scores=True, allowlist=allowlist, blocklist=blocklist)
+    return _engine_for(weights_dir).ocr_pages(list(images), scores=True, allowlist=allowlist, blocklist=blocklist,
+                                              rotation_info=rotation_info)

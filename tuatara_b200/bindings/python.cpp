@@ -44,6 +44,33 @@ static py::dict scored_item_to_dict(const tuatara::ScoredItem& item) {
   return d;
 }
 
+// rotation_info keyword -> angles (None: no rotation candidates)
+struct RotationArgs {
+  bool given = false;
+  std::vector<int> angles;
+};
+
+static RotationArgs rotation_args(const py::object& rotation_info) {
+  RotationArgs ra;
+  if (rotation_info.is_none()) return ra;
+  if (py::isinstance<py::str>(rotation_info) || !py::isinstance<py::iterable>(rotation_info))
+    throw py::type_error("rotation_info: expected an iterable of ints from {90, 180, 270}");
+  ra.given = true;
+  for (const py::handle& v : rotation_info) {
+    if (!py::isinstance<py::int_>(v) || py::isinstance<py::bool_>(v)) throw py::type_error("rotation_info: expected ints");
+    ra.angles.push_back(v.cast<int>());
+  }
+  return ra;
+}
+
+// the items of an oriented call; as_scored: with conf / det_score / char_conf, else text / bbox only.  An empty
+// rotation_info reads every word upright: angle 0.
+static py::dict oriented_item_to_dict(const tuatara::ScoredItem& item, bool as_scored) {
+  py::dict d = as_scored ? scored_item_to_dict(item) : output_item_to_dict(OutputItem{item.text, item.bbox});
+  d["angle"] = item.angle;
+  return d;
+}
+
 // allowlist / blocklist keywords -> character filters (tuatara::CharFilter).  Each is None, a str (every page) or, for
 // the batch functions, a list with one str or None per page.  No filter at all when both are None.
 struct FilterArgs {
@@ -78,11 +105,32 @@ static FilterArgs filter_args(const py::object& allow, const py::object& block, 
   return fa;
 }
 
+static py::list oriented_pages(const std::vector<tuatara::ImageView>& views, const std::string& weights_dir,
+                               const std::string& output_dir, const FilterArgs& fa, const RotationArgs& ra, bool as_scored) {
+  std::vector<std::vector<tuatara::ScoredItem>> pages;
+  {
+    py::gil_scoped_release release;
+    pages = tuatara::image_to_data_oriented_batch(views, weights_dir, output_dir, ra.angles, fa.filters);
+  }
+  py::list result;
+  for (const auto& page : pages) {
+    py::list items;
+    for (const auto& item : page) items.append(oriented_item_to_dict(item, as_scored));
+    result.append(items);
+  }
+  return result;
+}
+
 static py::list image_to_data_wrapper(py::array_t<unsigned char, py::array::c_style | py::array::forcecast> image_data,
                                       std::string weights_dir, std::string output_dir, py::object allowlist,
-                                      py::object blocklist) {
+                                      py::object blocklist, py::object rotation_info) {
   const tuatara::ImageView img = buffer_to_view(image_data);
   const FilterArgs fa = filter_args(allowlist, blocklist, 1, false);
+  const RotationArgs ra = rotation_args(rotation_info);
+  if (ra.given) {
+    py::list pages = oriented_pages({img}, weights_dir, output_dir, fa, ra, false);
+    return pages.empty() ? py::list() : py::list(pages[0]);
+  }
   std::vector<OutputItem> items;
   {
     py::gil_scoped_release release;
@@ -96,10 +144,12 @@ static py::list image_to_data_wrapper(py::array_t<unsigned char, py::array::c_st
 
 static py::list images_to_data_wrapper(std::vector<py::array_t<unsigned char, py::array::c_style | py::array::forcecast>> images,
                                        std::string weights_dir, std::string output_dir, py::object allowlist,
-                                       py::object blocklist) {
+                                       py::object blocklist, py::object rotation_info) {
   std::vector<tuatara::ImageView> views;
   for (auto& a : images) views.push_back(buffer_to_view(a));
   const FilterArgs fa = filter_args(allowlist, blocklist, views.size(), true);
+  const RotationArgs ra = rotation_args(rotation_info);
+  if (ra.given) return oriented_pages(views, weights_dir, output_dir, fa, ra, false);
   std::vector<std::vector<OutputItem>> pages;
   {
     py::gil_scoped_release release;
@@ -117,9 +167,14 @@ static py::list images_to_data_wrapper(std::vector<py::array_t<unsigned char, py
 
 static py::list image_to_data_scored_wrapper(py::array_t<unsigned char, py::array::c_style | py::array::forcecast> image_data,
                                              std::string weights_dir, std::string output_dir, py::object allowlist,
-                                             py::object blocklist) {
+                                             py::object blocklist, py::object rotation_info) {
   const tuatara::ImageView img = buffer_to_view(image_data);
   const FilterArgs fa = filter_args(allowlist, blocklist, 1, false);
+  const RotationArgs ra = rotation_args(rotation_info);
+  if (ra.given) {
+    py::list pages = oriented_pages({img}, weights_dir, output_dir, fa, ra, true);
+    return pages.empty() ? py::list() : py::list(pages[0]);
+  }
   std::vector<tuatara::ScoredItem> items;
   {
     py::gil_scoped_release release;
@@ -133,10 +188,12 @@ static py::list image_to_data_scored_wrapper(py::array_t<unsigned char, py::arra
 
 static py::list images_to_data_scored_wrapper(std::vector<py::array_t<unsigned char, py::array::c_style | py::array::forcecast>> images,
                                               std::string weights_dir, std::string output_dir, py::object allowlist,
-                                              py::object blocklist) {
+                                              py::object blocklist, py::object rotation_info) {
   std::vector<tuatara::ImageView> views;
   for (auto& a : images) views.push_back(buffer_to_view(a));
   const FilterArgs fa = filter_args(allowlist, blocklist, views.size(), true);
+  const RotationArgs ra = rotation_args(rotation_info);
+  if (ra.given) return oriented_pages(views, weights_dir, output_dir, fa, ra, true);
   std::vector<std::vector<tuatara::ScoredItem>> pages;
   {
     py::gil_scoped_release release;
@@ -154,17 +211,18 @@ static py::list images_to_data_scored_wrapper(std::vector<py::array_t<unsigned c
 
 PYBIND11_MODULE(pytuatara, m) {
   m.doc() = "Tuatara ocr";
-  // allowlist / blocklist (keyword only): recognition only produces characters in allowlist and not in blocklist
+  // allowlist / blocklist (keyword only): recognition only produces characters in allowlist and not in blocklist.
+  // rotation_info (keyword only): angles from {90, 180, 270} at which each word is also read; items then carry "angle".
   m.def("image_to_data", &image_to_data_wrapper, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"), py::kw_only(),
-        py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(),
+        py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
         "Extract text and bounding boxes from an image");
   m.def("images_to_data", &images_to_data_wrapper, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"), py::kw_only(),
-        py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(),
+        py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
         "Batch variant: list of images -> list of per-page results");
   m.def("image_to_data_scored", &image_to_data_scored_wrapper, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"),
-        py::kw_only(), py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(),
+        py::kw_only(), py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
         "image_to_data whose items also carry conf (word confidence 0..1, None when not recognised), det_score and char_conf");
   m.def("images_to_data_scored", &images_to_data_scored_wrapper, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"),
-        py::kw_only(), py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(),
+        py::kw_only(), py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
         "Batch variant of image_to_data_scored");
 }

@@ -14,6 +14,7 @@
 #include "gemm_tc.cuh"
 #include "geometry.h"
 #include "nn_kernels.cuh"
+#include "orient.cuh"
 #include "postprocess.cuh"
 #include "resize.cuh"
 #include "tokenizer.h"
@@ -199,6 +200,47 @@ int tt_crop_resize(const tt_image* image, const int32_t* rects_xywh, int n, uint
     const size_t out_bytes = static_cast<size_t>(n) * 32 * 128 * 3;
     TT_CUDA_INT(dout.alloc(out_bytes));
     TT_TRY_INT(crop_resize(dpages.as<PageRef>(), dboxes.as<CropBox>(), n, dout.as<uint8_t>(), nullptr, 0));
+    TT_CUDA_INT(cudaMemcpy(out, dout.p, out_bytes, cudaMemcpyDeviceToHost));
+    return 0;
+  });
+}
+
+int tt_crop_resize_rotated(const tt_image* image, const int32_t* rects_xywh, const int32_t* angles, int n, uint8_t* out) {
+  return guarded([&]() -> int {
+    if (!image || !image->data || image->channels != 3) { set_error("tt_crop_resize_rotated: need a 3-channel image"); return 1; }
+    if (n <= 0) return 0;
+    if (!rects_xywh || !angles || !out) { set_error("tt_crop_resize_rotated: null rects, angles or output"); return 1; }
+    std::vector<CropBox> boxes(n);
+    std::vector<uint8_t> rot(n);
+    for (int i = 0; i < n; ++i) {
+      const int32_t* r = rects_xywh + 4 * i;
+      if (r[0] < 0 || r[1] < 0 || r[2] < 0 || r[3] < 0 || r[0] + r[2] > image->cols || r[1] + r[3] > image->rows) {
+        set_error("tt_crop_resize_rotated: rect " + std::to_string(i) + " leaves the image (clamp it first)");
+        return 1;
+      }
+      const int a = angles[i];
+      if (a != 0 && a != 90 && a != 180 && a != 270) {
+        set_error("tt_crop_resize_rotated: angle " + std::to_string(a) + " of crop " + std::to_string(i) +
+                  "; the angles are 0, 90, 180 and 270");
+        return 1;
+      }
+      boxes[i] = CropBox{0, r[0], r[1], r[2], r[3]};
+      rot[i] = static_cast<uint8_t>(a / 90);
+    }
+    DevBuf src, dpages, dboxes, drot, dout;
+    const size_t src_bytes = image->step * image->rows;
+    TT_CUDA_INT(src.alloc(src_bytes));
+    TT_CUDA_INT(cudaMemcpy(src.p, image->data, src_bytes, cudaMemcpyHostToDevice));
+    PageRef pr{src.as<uint8_t>(), image->rows, image->cols, image->step};
+    TT_CUDA_INT(dpages.alloc(sizeof(PageRef)));
+    TT_CUDA_INT(cudaMemcpy(dpages.p, &pr, sizeof(pr), cudaMemcpyHostToDevice));
+    TT_CUDA_INT(dboxes.alloc(sizeof(CropBox) * n));
+    TT_CUDA_INT(cudaMemcpy(dboxes.p, boxes.data(), sizeof(CropBox) * n, cudaMemcpyHostToDevice));
+    TT_CUDA_INT(drot.alloc(n));
+    TT_CUDA_INT(cudaMemcpy(drot.p, rot.data(), n, cudaMemcpyHostToDevice));
+    const size_t out_bytes = static_cast<size_t>(n) * 32 * 128 * 3;
+    TT_CUDA_INT(dout.alloc(out_bytes));
+    TT_TRY_INT(crop_resize_rot(dpages.as<PageRef>(), dboxes.as<CropBox>(), drot.as<uint8_t>(), 1, n, dout.as<uint8_t>(), nullptr, 0));
     TT_CUDA_INT(cudaMemcpy(out, dout.p, out_bytes, cudaMemcpyDeviceToHost));
     return 0;
   });
@@ -428,6 +470,20 @@ int tt_dec_self_attn_dev(int n_crops, int D, int heads, int L, int p0, int np, i
     st.active = active; st.n_act = n_act;
     return dec_self_attn(st, q_table, sc_table, static_cast<const __nv_bfloat16*>(kv_table), tokens, eos_id, n_tok,
                          static_cast<__nv_bfloat16*>(out), static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : 1;
+  });
+}
+
+int tt_orient_select_dev(const int32_t* ids, const float* pmax, int n_words, const int32_t* angles, int n_candidates,
+                         int32_t* ids_out, float* pmax_out, int32_t* angle_out, void* stream) {
+  return guarded([&]() -> int {
+    if (n_candidates < 1 || n_candidates > 4 || !angles) {
+      set_error("tt_orient_select_dev: n_candidates must be 1..4 with its angles, got " + std::to_string(n_candidates));
+      return 1;
+    }
+    OrientSet set{n_candidates, {0, 0, 0, 0}};
+    for (int r = 0; r < n_candidates; ++r) set.angle[r] = angles[r];
+    return orient_select(ids, pmax, n_words, TT_MAX_LABEL_LEN, set, ids_out, pmax_out, angle_out,
+                         static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : 1;
   });
 }
 

@@ -129,6 +129,78 @@ __global__ void __launch_bounds__(128) k_crop(const PageRef* __restrict__ pages,
   }
 }
 
+// Rotation candidates (INTEGRATION.md section 8): crop b is box b / R turned rot[b] quarter turns counter-clockwise
+// before the resize, cv::resize(cv::rotate(roi, code), (128, 32)).  The turned ROI T is rw x rh = w x h (0, 180) or
+// h x w (90, 270) and gets k_crop's coefficients for that size.  T's pixel (ty, tx) is the source pixel
+//   0: (ty, tx)   90: (tx, w-1-ty)   180: (h-1-ty, w-1-tx)   270: (h-1-tx, ty)
+// so each output row blends two "lines" of the source (rows for 0 / 180, columns for 90 / 270), and pixel k of a line
+// sits at line + k * stride (stride 3, -3, step or -step bytes).  Both lines are staged in shared memory in T's order:
+// coalesced for rows, one source row per three threads for columns.  grid (32, n_crops), 128 threads, as k_crop.
+__global__ void __launch_bounds__(128) k_crop_rot(const PageRef* __restrict__ pages, const CropBox* __restrict__ boxes,
+                                                  const uint8_t* __restrict__ rot, int R, uint8_t* __restrict__ out_u8,
+                                                  __nv_bfloat16* __restrict__ out_patch) {
+  __shared__ uint8_t rows[2][kCropStage];
+  const int dy = blockIdx.x, b = blockIdx.y, dx = threadIdx.x;
+  const CropBox box = boxes[b / R];
+  const int q = rot[b] & 3;
+  int val[3] = {0, 0, 0};
+  if (box.w > 0 && box.h > 0) {
+    const PageRef pg = pages[box.page];
+    const bool turned = q & 1;
+    const int rw = turned ? box.h : box.w, rh = turned ? box.w : box.h;
+    const double scale_x = 1.0 / (128.0 / static_cast<double>(rw));
+    const double scale_y = 1.0 / (32.0 / static_cast<double>(rh));
+    const AxisCoef ay = axis_coef(dy, scale_y, rh, false);
+    const int ty[2] = {min(max(ay.s, 0), rh - 1), min(max(ay.s + 1, 0), rh - 1)};
+    const long long step = static_cast<long long>(pg.step);
+    const uint8_t* org = pg.data + static_cast<long long>(box.y) * step + static_cast<long long>(box.x) * 3;
+    const long long stride = q == 0 ? 3 : q == 1 ? step : q == 2 ? -3 : -step;
+    const uint8_t* line[2];
+#pragma unroll
+    for (int j = 0; j < 2; ++j) {
+      const int t = ty[j];
+      line[j] = org + (q == 0 ? t * step
+                     : q == 1 ? static_cast<long long>(box.w - 1 - t) * 3
+                     : q == 2 ? (box.h - 1 - t) * step + static_cast<long long>(box.w - 1) * 3
+                              : static_cast<long long>(t) * 3 + (box.h - 1) * step);
+    }
+    const int nbytes = rw * 3;
+    const bool staged = nbytes <= kCropStage;
+    if (staged) {
+      for (int i = threadIdx.x; i < nbytes; i += blockDim.x) {
+        const long long off = (i / 3) * stride + i % 3;
+        rows[0][i] = line[0][off];
+        rows[1][i] = line[1][off];
+      }
+      __syncthreads();
+    }
+    const AxisCoef ax = axis_coef(dx, scale_x, rw, true);
+    const int x1 = min(ax.s + 1, rw - 1);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      int v[2][2];
+#pragma unroll
+      for (int j = 0; j < 2; ++j) {
+        v[j][0] = staged ? rows[j][ax.s * 3 + c] : line[j][ax.s * stride + c];
+        v[j][1] = staged ? rows[j][x1 * 3 + c] : line[j][x1 * stride + c];
+      }
+      const int S0 = v[0][0] * ax.c0 + v[0][1] * ax.c1;
+      const int S1 = v[1][0] * ax.c0 + v[1][1] * ax.c1;
+      val[c] = vblend(S0, S1, ay.c0, ay.c1);
+    }
+  }
+  if (out_u8 != nullptr) {
+    uint8_t* o = out_u8 + ((static_cast<size_t>(b) * 32 + dy) * 128 + dx) * 3;
+    o[0] = static_cast<uint8_t>(val[0]); o[1] = static_cast<uint8_t>(val[1]); o[2] = static_cast<uint8_t>(val[2]);
+  }
+  if (out_patch != nullptr) {
+    const size_t row = static_cast<size_t>(b) * 128 + (dy >> 2) * 16 + (dx >> 3);
+    __nv_bfloat16* o = out_patch + row * 96 + (dy & 3) * 8 + (dx & 7);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) o[c * 32] = __float2bfloat16(static_cast<float>(val[c]));
+  }
+}
+
 // grid (32, n), 128 threads: one output row of one crop per block, as k_crop.  Arithmetic follows
 // cv::warpPerspective's block loop (64 x 16 blocks for a 128 x 32 destination): X0 = M0*x + M1*y + M2 at the block
 // origin, then (X0 + M0*x1) * (32 / W) per pixel, no fused multiply-add (the CPU code has none either).
@@ -196,6 +268,14 @@ cudaError_t crop_resize(const PageRef* pages_dev, const CropBox* boxes_dev, int 
                         __nv_bfloat16* out_patches, cudaStream_t s) {
   if (n_boxes <= 0) return cudaSuccess;
   k_crop<<<dim3(32, n_boxes), 128, 0, s>>>(pages_dev, boxes_dev, out_u8, out_patches);
+  TT_LAUNCH_CHECK();
+  return cudaSuccess;
+}
+
+cudaError_t crop_resize_rot(const PageRef* pages_dev, const CropBox* boxes_dev, const uint8_t* rot_dev, int R, int n_crops,
+                            uint8_t* out_u8, __nv_bfloat16* out_patches, cudaStream_t s) {
+  if (n_crops <= 0) return cudaSuccess;
+  k_crop_rot<<<dim3(32, n_crops), 128, 0, s>>>(pages_dev, boxes_dev, rot_dev, R, out_u8, out_patches);
   TT_LAUNCH_CHECK();
   return cudaSuccess;
 }

@@ -34,6 +34,12 @@ struct PageRef {
 cudaError_t crop_resize(const PageRef* pages_dev, const CropBox* boxes_dev, int n_boxes, uint8_t* out_u8,
                         __nv_bfloat16* out_patches, cudaStream_t s);
 
+// Rotation candidates (tt_ocr_pages_oriented): crop b is box b / R (boxes_dev holds n_crops / R boxes) turned rot_dev[b]
+// quarter turns counter-clockwise (0..3) before the resize, cv::resize(cv::rotate(roi, code), (128, 32)) bit for bit.
+// Outputs as crop_resize; rot_dev[b] == 0 gives crop_resize's bytes.
+cudaError_t crop_resize_rot(const PageRef* pages_dev, const CropBox* boxes_dev, const uint8_t* rot_dev, int R, int n_crops,
+                            uint8_t* out_u8, __nv_bfloat16* out_patches, cudaStream_t s);
+
 // Opt-in rectified crops (tt_config.rectify; the TODO at tuatara.cpp:411-415): every crop is the 128 x 32 perspective
 // warp of its box's quadrilateral, sampled the way cv::warpPerspective(INTER_LINEAR, BORDER_REPLICATE) samples it
 // (source coordinates in double, rounded to 1/32 pixel, 15-bit fixed-point bilinear weights).
