@@ -85,69 +85,34 @@ inline tt_engine* engine_for(const std::string& weights_dir) {
 }  // namespace detail
 
 namespace detail {
-// The checks, soft failures and engine call shared by the batch entry points: nullptr after printing the reason.
-// opt == nullptr: plain tt_ocr_pages.  filters != nullptr: tt_ocr_pages_filtered (one filter, or one per page).
-inline tt_result* ocr_pages(const std::vector<ImageView>& images, const std::string& weights_dir,
-                            const std::string& outputs_dir, const tt_ocr_options* opt,
-                            const std::vector<CharFilter>* filters = nullptr,
-                            const std::vector<int>* rotation_info = nullptr) {
-  if (weights_dir.empty()) { std::cerr << "Please provide a value for weights_dir" << std::endl; return nullptr; }
-  if (outputs_dir.empty()) { std::cerr << "Please provide a value for outputs_dir" << std::endl; return nullptr; }
+// The one path of every entry point: the checks, the soft failures ({} after printing the reason), one
+// tt_ocr_pages_oriented call and the walk over its result.  Each item's scores are fetched when `scores`, its angle when
+// rotation_info is not empty.  filters: none (empty), one for every page, or one per page.
+inline std::vector<std::vector<ScoredItem>> ocr_pages(const std::vector<ImageView>& images, const std::string& weights_dir,
+                                                      const std::string& outputs_dir, bool scores,
+                                                      const std::vector<CharFilter>& filters,
+                                                      const std::vector<int>& rotation_info = {}) {
+  std::vector<std::vector<ScoredItem>> out;
+  if (weights_dir.empty()) { std::cerr << "Please provide a value for weights_dir" << std::endl; return out; }
+  if (outputs_dir.empty()) { std::cerr << "Please provide a value for outputs_dir" << std::endl; return out; }
   std::vector<tt_image> pages(images.size());
   for (size_t i = 0; i < images.size(); ++i) {
     const ImageView& v = images[i];
-    if (!v.data || v.rows <= 0 || v.cols <= 0) { std::cerr << "Error reading image from file"; return nullptr; }
+    if (!v.data || v.rows <= 0 || v.cols <= 0) { std::cerr << "Error reading image from file"; return out; }
     pages[i] = tt_image{v.data, v.rows, v.cols, v.channels, v.step ? v.step : static_cast<size_t>(v.cols) * v.channels};
   }
   tt_engine* e = engine_for(weights_dir);
-  if (!e) { std::cerr << "error loading the models: " << tt_last_error() << std::endl; return nullptr; }
-  tt_result* r = nullptr;
-  int rc = 0;
-  if (filters || rotation_info) {
-    std::vector<tt_char_filter> f;
-    if (filters)
-      for (const CharFilter& cf : *filters) f.push_back(tt_char_filter{cf.allow, cf.block});
-    const tt_ocr_options none = {};
-    rc = rotation_info
-             ? tt_ocr_pages_oriented(e, pages.data(), static_cast<int>(pages.size()), opt ? opt : &none, f.data(),
-                                     static_cast<int>(f.size()), rotation_info->data(),
-                                     static_cast<int>(rotation_info->size()), &r)
-             : tt_ocr_pages_filtered(e, pages.data(), static_cast<int>(pages.size()), opt ? opt : &none, f.data(),
-                                     static_cast<int>(f.size()), &r);
-  } else {
-    rc = opt ? tt_ocr_pages_ex(e, pages.data(), static_cast<int>(pages.size()), opt, &r)
-             : tt_ocr_pages(e, pages.data(), static_cast<int>(pages.size()), &r);
-  }
-  if (rc != 0) {
-    std::cerr << "tuatara: " << tt_last_error() << std::endl;
-    return nullptr;
-  }
-  return r;
-}
-
-inline std::vector<std::vector<OutputItem>> batch_items(const std::vector<ImageView>& images, const std::string& weights_dir,
-                                                        const std::string& outputs_dir, const std::vector<CharFilter>* filters) {
-  std::vector<std::vector<OutputItem>> out;
-  tt_result* r = ocr_pages(images, weights_dir, outputs_dir, nullptr, filters);
-  if (!r) return out;
-  out.resize(r->n_pages);
-  for (int p = 0; p < r->n_pages; ++p)
-    for (int k = 0; k < r->pages[p].n_items; ++k) {
-      const tt_item& it = r->pages[p].items[k];
-      out[p].push_back(OutputItem{it.text, std::vector<float>(it.bbox, it.bbox + 4)});
-    }
-  tt_result_free(r);
-  return out;
-}
-
-inline std::vector<std::vector<ScoredItem>> scored_items(const std::vector<ImageView>& images, const std::string& weights_dir,
-                                                         const std::string& outputs_dir, const std::vector<CharFilter>* filters,
-                                                         const std::vector<int>* rotation_info = nullptr) {
-  std::vector<std::vector<ScoredItem>> out;
+  if (!e) { std::cerr << "error loading the models: " << tt_last_error() << std::endl; return out; }
+  std::vector<tt_char_filter> f;
+  for (const CharFilter& cf : filters) f.push_back(tt_char_filter{cf.allow, cf.block});
   tt_ocr_options opt = {};
-  opt.with_scores = 1;
-  tt_result* r = ocr_pages(images, weights_dir, outputs_dir, &opt, filters, rotation_info);
-  if (!r) return out;
+  opt.with_scores = scores ? 1 : 0;
+  tt_result* r = nullptr;
+  if (tt_ocr_pages_oriented(e, pages.data(), static_cast<int>(pages.size()), &opt, f.data(), static_cast<int>(f.size()),
+                            rotation_info.data(), static_cast<int>(rotation_info.size()), &r) != 0) {
+    std::cerr << "tuatara: " << tt_last_error() << std::endl;
+    return out;
+  }
   out.resize(r->n_pages);
   for (int p = 0; p < r->n_pages; ++p)
     for (int k = 0; k < r->pages[p].n_items; ++k) {
@@ -157,16 +122,23 @@ inline std::vector<std::vector<ScoredItem>> scored_items(const std::vector<Image
       s.bbox.assign(it.bbox, it.bbox + 4);
       const float* cc = nullptr;
       int n = 0;
-      if (tt_item_scores(r, p, k, &s.confidence, &s.detection_score, &cc, &n) != 0 ||
-          (rotation_info && !rotation_info->empty() && tt_item_angle(r, p, k, &s.angle) != 0)) {
+      if ((scores && tt_item_scores(r, p, k, &s.confidence, &s.detection_score, &cc, &n) != 0) ||
+          (!rotation_info.empty() && tt_item_angle(r, p, k, &s.angle) != 0)) {
         std::cerr << "tuatara: " << tt_last_error() << std::endl;
         tt_result_free(r);
         return std::vector<std::vector<ScoredItem>>{};
       }
       if (n > 0) s.char_confidence.assign(cc, cc + n);
-      out[p].push_back(s);
+      out[p].push_back(std::move(s));
     }
   tt_result_free(r);
+  return out;
+}
+
+inline std::vector<std::vector<OutputItem>> unscored(std::vector<std::vector<ScoredItem>> pages) {
+  std::vector<std::vector<OutputItem>> out(pages.size());
+  for (size_t p = 0; p < pages.size(); ++p)
+    for (ScoredItem& s : pages[p]) out[p].push_back(OutputItem{std::move(s.text), std::move(s.bbox)});
   return out;
 }
 }  // namespace detail
@@ -175,7 +147,7 @@ inline std::vector<std::vector<ScoredItem>> scored_items(const std::vector<Image
 inline std::vector<std::vector<OutputItem>> image_to_data_batch(const std::vector<ImageView>& images,
                                                                 const std::string& weights_dir,
                                                                 const std::string& outputs_dir) {
-  return detail::batch_items(images, weights_dir, outputs_dir, nullptr);
+  return detail::unscored(detail::ocr_pages(images, weights_dir, outputs_dir, false, {}));
 }
 
 // image_to_data_batch with character filters: `filters` holds one filter for every page, or one per page.
@@ -183,14 +155,14 @@ inline std::vector<std::vector<OutputItem>> image_to_data_batch(const std::vecto
                                                                 const std::string& weights_dir,
                                                                 const std::string& outputs_dir,
                                                                 const std::vector<CharFilter>& filters) {
-  return detail::batch_items(images, weights_dir, outputs_dir, &filters);
+  return detail::unscored(detail::ocr_pages(images, weights_dir, outputs_dir, false, filters));
 }
 
 // image_to_data_batch with scores: same items (text, bbox) and the same soft failures, plus each item's scores.
 inline std::vector<std::vector<ScoredItem>> image_to_data_scored_batch(const std::vector<ImageView>& images,
                                                                        const std::string& weights_dir,
                                                                        const std::string& outputs_dir) {
-  return detail::scored_items(images, weights_dir, outputs_dir, nullptr);
+  return detail::ocr_pages(images, weights_dir, outputs_dir, true, {});
 }
 
 // image_to_data_scored_batch with character filters (one for every page, or one per page); the scores are renormalised
@@ -199,7 +171,7 @@ inline std::vector<std::vector<ScoredItem>> image_to_data_scored_batch(const std
                                                                        const std::string& weights_dir,
                                                                        const std::string& outputs_dir,
                                                                        const std::vector<CharFilter>& filters) {
-  return detail::scored_items(images, weights_dir, outputs_dir, &filters);
+  return detail::ocr_pages(images, weights_dir, outputs_dir, true, filters);
 }
 
 inline std::vector<ScoredItem> image_to_data_scored(const ImageView& image, const std::string& weights_dir,
@@ -224,7 +196,7 @@ inline std::vector<std::vector<ScoredItem>> image_to_data_oriented_batch(const s
                                                                          const std::string& outputs_dir,
                                                                          const std::vector<int>& rotation_info,
                                                                          const std::vector<CharFilter>& filters = {}) {
-  return detail::scored_items(images, weights_dir, outputs_dir, filters.empty() ? nullptr : &filters, &rotation_info);
+  return detail::ocr_pages(images, weights_dir, outputs_dir, true, filters, rotation_info);
 }
 
 inline std::vector<ScoredItem> image_to_data_oriented(const ImageView& image, const std::string& weights_dir,

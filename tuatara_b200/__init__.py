@@ -260,9 +260,9 @@ class Engine:
         None entries) that replace CRAFT's output after CRAFT has run (benchmark / parity tests).
         scores: every item also carries conf (word confidence 0..1, None when not recognised), det_score (the
         detection score of its box) and char_conf (one probability per character of text); see tt_item_scores.
-        allowlist / blocklist: character filters (tt_ocr_pages_filtered): recognition only produces characters in
+        allowlist / blocklist: character filters (tt_char_filter): recognition only produces characters in
         allowlist and not in blocklist.  Each is None, a str for every page, or a list with one str or None per page.
-        rotation_info: an iterable of angles from {90, 180, 270} (tt_ocr_pages_oriented): each word is also read turned
+        rotation_info: an iterable of angles from {90, 180, 270}: each word is also read turned
         that many degrees counter-clockwise and the candidate with the highest word confidence wins; every item then
         carries "angle" (0, 90, 180 or 270; -1 when not recognised).  An empty iterable reads every word upright."""
         n = len(images)
@@ -292,14 +292,8 @@ class Engine:
         res = C.POINTER(_native.tt_result)()
         filters = _filters(allowlist, blocklist, n)
         rot = None if rotation_info is None else _rotations(rotation_info)
-        if rot is not None:
-            check(lib().tt_ocr_pages_oriented(self._h, arr, n, C.byref(opt), filters, len(filters) if filters else 0,
-                                              rot, len(rot), C.byref(res)), "tt_ocr_pages_oriented")
-        elif filters is None:
-            check(lib().tt_ocr_pages_ex(self._h, arr, n, C.byref(opt), C.byref(res)), "tt_ocr_pages_ex")
-        else:
-            check(lib().tt_ocr_pages_filtered(self._h, arr, n, C.byref(opt), filters, len(filters), C.byref(res)),
-                  "tt_ocr_pages_filtered")
+        check(lib().tt_ocr_pages_oriented(self._h, arr, n, C.byref(opt), filters or None, len(filters) if filters else 0,
+                                          rot, len(rot) if rot is not None else 0, C.byref(res)), "tt_ocr_pages_oriented")
         try:
             out = []
             for p in range(res.contents.n_pages):
@@ -417,18 +411,8 @@ def image_to_data(image: np.ndarray, weights_dir: str, outputs_dir: str, *, allo
     strings print to stderr and return [] like tuatara.cpp:315-323.  allowlist / blocklist: recognition only produces
     characters in allowlist and not in blocklist (INTEGRATION.md section 7).  rotation_info: angles from {90, 180, 270}
     at which each word is also read; items then carry "angle" (INTEGRATION.md section 8)."""
-    import sys
-
-    if not weights_dir:
-        print("Please provide a value for weights_dir", file=sys.stderr)
-        return []
-    if not outputs_dir:
-        print("Please provide a value for outputs_dir", file=sys.stderr)
-        return []
-    if image.ndim != 3:
-        raise RuntimeError("Input array should have 3 dimensions")
-    return _engine_for(weights_dir).ocr_pages([image], allowlist=allowlist, blocklist=blocklist,
-                                              rotation_info=rotation_info)[0]
+    return _one_page(image, weights_dir, outputs_dir, allowlist=allowlist, blocklist=blocklist,
+                     rotation_info=rotation_info)
 
 
 def images_to_data(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".", *, allowlist=None,
@@ -444,6 +428,20 @@ def image_to_data_scored(image: np.ndarray, weights_dir: str, outputs_dir: str, 
     """image_to_data whose items also carry ``conf`` (word confidence 0..1), ``det_score`` (the detection score of the
     box) and ``char_conf`` (one probability per character of ``text``).  Same inputs, errors and soft failures;
     ``text`` and ``bbox`` are what image_to_data returns."""
+    return _one_page(image, weights_dir, outputs_dir, scores=True, allowlist=allowlist, blocklist=blocklist,
+                     rotation_info=rotation_info)
+
+
+def images_to_data_scored(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".", *, allowlist=None,
+                          blocklist=None, rotation_info=None) -> list[list[dict]]:
+    """Batch variant of image_to_data_scored."""
+    return _engine_for(weights_dir).ocr_pages(list(images), scores=True, allowlist=allowlist, blocklist=blocklist,
+                                              rotation_info=rotation_info)
+
+
+def _one_page(image: np.ndarray, weights_dir: str, outputs_dir: str, **kw) -> list[dict]:
+    """image_to_data and image_to_data_scored: empty directory strings print to stderr and return [] like
+    tuatara.cpp:315-323; else the page's items from Engine.ocr_pages(**kw)."""
     import sys
 
     if not weights_dir:
@@ -454,12 +452,4 @@ def image_to_data_scored(image: np.ndarray, weights_dir: str, outputs_dir: str, 
         return []
     if image.ndim != 3:
         raise RuntimeError("Input array should have 3 dimensions")
-    return _engine_for(weights_dir).ocr_pages([image], scores=True, allowlist=allowlist, blocklist=blocklist,
-                                              rotation_info=rotation_info)[0]
-
-
-def images_to_data_scored(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".", *, allowlist=None,
-                          blocklist=None, rotation_info=None) -> list[list[dict]]:
-    """Batch variant of image_to_data_scored."""
-    return _engine_for(weights_dir).ocr_pages(list(images), scores=True, allowlist=allowlist, blocklist=blocklist,
-                                              rotation_info=rotation_info)
+    return _engine_for(weights_dir).ocr_pages([image], **kw)[0]

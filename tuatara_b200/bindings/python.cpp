@@ -13,7 +13,9 @@
 
 namespace py = pybind11;
 
-static tuatara::ImageView buffer_to_view(const py::array_t<unsigned char, py::array::c_style | py::array::forcecast>& input) {
+using Image = py::array_t<unsigned char, py::array::c_style | py::array::forcecast>;
+
+static tuatara::ImageView buffer_to_view(const Image& input) {
   py::buffer_info buf = input.request();
   if (buf.ndim != 3) throw std::runtime_error("Input array should have 3 dimensions");  // python.cpp:15-17
   tuatara::ImageView v;
@@ -24,24 +26,6 @@ static tuatara::ImageView buffer_to_view(const py::array_t<unsigned char, py::ar
   v.step = static_cast<size_t>(buf.strides[0]);
   if (v.channels != 3) throw std::runtime_error("Input array should have 3 channels");
   return v;
-}
-
-static py::dict output_item_to_dict(const OutputItem& item) {  // python.cpp:36-41
-  py::dict d;
-  d["text"] = item.text;
-  d["bbox"] = item.bbox;
-  return d;
-}
-
-// conf is None for a word that was not recognised (ScoredItem::confidence == -1)
-static py::dict scored_item_to_dict(const tuatara::ScoredItem& item) {
-  py::dict d;
-  d["text"] = item.text;
-  d["bbox"] = item.bbox;
-  d["conf"] = item.confidence < 0.f ? py::object(py::none()) : py::object(py::float_(item.confidence));
-  d["det_score"] = item.detection_score;
-  d["char_conf"] = item.char_confidence;
-  return d;
 }
 
 // rotation_info keyword -> angles (None: no rotation candidates)
@@ -61,14 +45,6 @@ static RotationArgs rotation_args(const py::object& rotation_info) {
     ra.angles.push_back(v.cast<int>());
   }
   return ra;
-}
-
-// the items of an oriented call; as_scored: with conf / det_score / char_conf, else text / bbox only.  An empty
-// rotation_info reads every word upright: angle 0.
-static py::dict oriented_item_to_dict(const tuatara::ScoredItem& item, bool as_scored) {
-  py::dict d = as_scored ? scored_item_to_dict(item) : output_item_to_dict(OutputItem{item.text, item.bbox});
-  d["angle"] = item.angle;
-  return d;
 }
 
 // allowlist / blocklist keywords -> character filters (tuatara::CharFilter).  Each is None, a str (every page) or, for
@@ -105,124 +81,73 @@ static FilterArgs filter_args(const py::object& allow, const py::object& block, 
   return fa;
 }
 
-static py::list oriented_pages(const std::vector<tuatara::ImageView>& views, const std::string& weights_dir,
-                               const std::string& output_dir, const FilterArgs& fa, const RotationArgs& ra, bool as_scored) {
+// One item as a dict: text and bbox; conf (None for a word that was not recognised, ScoredItem::confidence == -1),
+// det_score and char_conf when scored; angle when rotation_info was given (0 for every word when it is empty).
+static py::dict item_to_dict(const tuatara::ScoredItem& item, bool scored, bool angle) {  // python.cpp:36-41
+  py::dict d;
+  d["text"] = item.text;
+  d["bbox"] = item.bbox;
+  if (scored) {
+    d["conf"] = item.confidence < 0.f ? py::object(py::none()) : py::object(py::float_(item.confidence));
+    d["det_score"] = item.detection_score;
+    d["char_conf"] = item.char_confidence;
+  }
+  if (angle) d["angle"] = item.angle;
+  return d;
+}
+
+// The four functions' one path -> a list of pages of item dicts.  batch: allowlist / blocklist may hold one entry per page.
+static py::list ocr_pages(const std::vector<tuatara::ImageView>& views, bool batch, const std::string& weights_dir,
+                          const std::string& output_dir, const py::object& allowlist, const py::object& blocklist,
+                          const py::object& rotation_info, bool scored) {
+  const FilterArgs fa = filter_args(allowlist, blocklist, views.size(), batch);
+  const RotationArgs ra = rotation_args(rotation_info);
   std::vector<std::vector<tuatara::ScoredItem>> pages;
   {
     py::gil_scoped_release release;
-    pages = tuatara::image_to_data_oriented_batch(views, weights_dir, output_dir, ra.angles, fa.filters);
+    pages = tuatara::detail::ocr_pages(views, weights_dir, output_dir, scored, fa.filters, ra.angles);
   }
   py::list result;
   for (const auto& page : pages) {
     py::list items;
-    for (const auto& item : page) items.append(oriented_item_to_dict(item, as_scored));
+    for (const auto& item : page) items.append(item_to_dict(item, scored, ra.given));
     result.append(items);
   }
   return result;
 }
 
-static py::list image_to_data_wrapper(py::array_t<unsigned char, py::array::c_style | py::array::forcecast> image_data,
-                                      std::string weights_dir, std::string output_dir, py::object allowlist,
-                                      py::object blocklist, py::object rotation_info) {
-  const tuatara::ImageView img = buffer_to_view(image_data);
-  const FilterArgs fa = filter_args(allowlist, blocklist, 1, false);
-  const RotationArgs ra = rotation_args(rotation_info);
-  if (ra.given) {
-    py::list pages = oriented_pages({img}, weights_dir, output_dir, fa, ra, false);
-    return pages.empty() ? py::list() : py::list(pages[0]);
-  }
-  std::vector<OutputItem> items;
-  {
-    py::gil_scoped_release release;
-    items = fa.filters.empty() ? image_to_data(img, weights_dir, output_dir)
-                               : image_to_data(img, weights_dir, output_dir, fa.filters[0]);
-  }
-  py::list result;
-  for (const auto& item : items) result.append(output_item_to_dict(item));
-  return result;
+// image_to_data / image_to_data_scored: page 0, or [] after a soft failure
+template <bool kScored>
+static py::list image_wrapper(Image image_data, std::string weights_dir, std::string output_dir, py::object allowlist,
+                              py::object blocklist, py::object rotation_info) {
+  py::list pages = ocr_pages({buffer_to_view(image_data)}, false, weights_dir, output_dir, allowlist, blocklist,
+                             rotation_info, kScored);
+  return pages.empty() ? py::list() : py::list(pages[0]);
 }
 
-static py::list images_to_data_wrapper(std::vector<py::array_t<unsigned char, py::array::c_style | py::array::forcecast>> images,
-                                       std::string weights_dir, std::string output_dir, py::object allowlist,
-                                       py::object blocklist, py::object rotation_info) {
+// images_to_data / images_to_data_scored
+template <bool kScored>
+static py::list images_wrapper(std::vector<Image> images, std::string weights_dir, std::string output_dir,
+                               py::object allowlist, py::object blocklist, py::object rotation_info) {
   std::vector<tuatara::ImageView> views;
   for (auto& a : images) views.push_back(buffer_to_view(a));
-  const FilterArgs fa = filter_args(allowlist, blocklist, views.size(), true);
-  const RotationArgs ra = rotation_args(rotation_info);
-  if (ra.given) return oriented_pages(views, weights_dir, output_dir, fa, ra, false);
-  std::vector<std::vector<OutputItem>> pages;
-  {
-    py::gil_scoped_release release;
-    pages = fa.filters.empty() ? tuatara::image_to_data_batch(views, weights_dir, output_dir)
-                               : tuatara::image_to_data_batch(views, weights_dir, output_dir, fa.filters);
-  }
-  py::list result;
-  for (const auto& page : pages) {
-    py::list items;
-    for (const auto& item : page) items.append(output_item_to_dict(item));
-    result.append(items);
-  }
-  return result;
-}
-
-static py::list image_to_data_scored_wrapper(py::array_t<unsigned char, py::array::c_style | py::array::forcecast> image_data,
-                                             std::string weights_dir, std::string output_dir, py::object allowlist,
-                                             py::object blocklist, py::object rotation_info) {
-  const tuatara::ImageView img = buffer_to_view(image_data);
-  const FilterArgs fa = filter_args(allowlist, blocklist, 1, false);
-  const RotationArgs ra = rotation_args(rotation_info);
-  if (ra.given) {
-    py::list pages = oriented_pages({img}, weights_dir, output_dir, fa, ra, true);
-    return pages.empty() ? py::list() : py::list(pages[0]);
-  }
-  std::vector<tuatara::ScoredItem> items;
-  {
-    py::gil_scoped_release release;
-    items = fa.filters.empty() ? tuatara::image_to_data_scored(img, weights_dir, output_dir)
-                               : tuatara::image_to_data_scored(img, weights_dir, output_dir, fa.filters[0]);
-  }
-  py::list result;
-  for (const auto& item : items) result.append(scored_item_to_dict(item));
-  return result;
-}
-
-static py::list images_to_data_scored_wrapper(std::vector<py::array_t<unsigned char, py::array::c_style | py::array::forcecast>> images,
-                                              std::string weights_dir, std::string output_dir, py::object allowlist,
-                                              py::object blocklist, py::object rotation_info) {
-  std::vector<tuatara::ImageView> views;
-  for (auto& a : images) views.push_back(buffer_to_view(a));
-  const FilterArgs fa = filter_args(allowlist, blocklist, views.size(), true);
-  const RotationArgs ra = rotation_args(rotation_info);
-  if (ra.given) return oriented_pages(views, weights_dir, output_dir, fa, ra, true);
-  std::vector<std::vector<tuatara::ScoredItem>> pages;
-  {
-    py::gil_scoped_release release;
-    pages = fa.filters.empty() ? tuatara::image_to_data_scored_batch(views, weights_dir, output_dir)
-                               : tuatara::image_to_data_scored_batch(views, weights_dir, output_dir, fa.filters);
-  }
-  py::list result;
-  for (const auto& page : pages) {
-    py::list items;
-    for (const auto& item : page) items.append(scored_item_to_dict(item));
-    result.append(items);
-  }
-  return result;
+  return ocr_pages(views, true, weights_dir, output_dir, allowlist, blocklist, rotation_info, kScored);
 }
 
 PYBIND11_MODULE(pytuatara, m) {
   m.doc() = "Tuatara ocr";
   // allowlist / blocklist (keyword only): recognition only produces characters in allowlist and not in blocklist.
   // rotation_info (keyword only): angles from {90, 180, 270} at which each word is also read; items then carry "angle".
-  m.def("image_to_data", &image_to_data_wrapper, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"), py::kw_only(),
+  m.def("image_to_data", &image_wrapper<false>, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"), py::kw_only(),
         py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
         "Extract text and bounding boxes from an image");
-  m.def("images_to_data", &images_to_data_wrapper, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"), py::kw_only(),
+  m.def("images_to_data", &images_wrapper<false>, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"), py::kw_only(),
         py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
         "Batch variant: list of images -> list of per-page results");
-  m.def("image_to_data_scored", &image_to_data_scored_wrapper, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"),
+  m.def("image_to_data_scored", &image_wrapper<true>, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"),
         py::kw_only(), py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
         "image_to_data whose items also carry conf (word confidence 0..1, None when not recognised), det_score and char_conf");
-  m.def("images_to_data_scored", &images_to_data_scored_wrapper, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"),
+  m.def("images_to_data_scored", &images_wrapper<true>, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"),
         py::kw_only(), py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
         "Batch variant of image_to_data_scored");
 }

@@ -49,7 +49,7 @@ struct PageOut {
   std::vector<float> det;                        // per item: the component's maximum normalised text score
   std::vector<float> conf;                       // per item: word confidence, -1 until recognised
   std::vector<std::vector<float>> char_conf;     // per item: one probability per character of text
-  // tt_ocr_pages_oriented only (empty otherwise): per item the winning candidate's angle, -1 until recognised
+  // with rotation candidates only (empty otherwise): per item the winning candidate's angle, -1 until recognised
   std::vector<int> angle;
 };
 
@@ -118,6 +118,13 @@ struct CropOwner { int page, box; };
 
 using ClassMask = std::array<uint32_t, 4>;   // tt_char_filter_mask
 
+// What a request asks for besides its pages, checked by make_request; every tt_ocr_pages* entry point builds one.
+struct Request {
+  tt_ocr_options opt{0, 0, nullptr, 0, 0};   // zeroed when the caller passes none
+  std::vector<ClassMask> masks;              // one class mask per page; empty when no page has a filter
+  OrientSet orient{1, {0, 0, 0, 0}};         // the rotation candidates; n == 1 (angle 0 alone) without
+};
+
 // crops waiting for recognition in one slot (device patch rows live in DeviceCtx::patch_buf)
 struct Pending {
   std::vector<CropOwner> owner;
@@ -141,10 +148,11 @@ cudaError_t ensure_patch_buf(DeviceCtx& d, size_t crops, size_t keep_crops) {
 }
 
 // Detection + cropping of one unit (tuatara.cpp:349-418, :437-441).  Fills bbox of every page of the unit, sizes its
-// text vector, appends the crops to the slot's recognition batch.  orient (null: none): every word gets orient->n crops,
-// candidate r turned orient->angle[r] degrees counter-clockwise, stored word-major (crop = word * n + r).
-int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const Unit& u, const tt_ocr_options& opt,
-                const OrientSet* orient, std::vector<PageOut>* results, Pending* pend) {
+// text vector, appends the crops to the slot's recognition batch.  Every word gets R = req.orient.n crops, candidate r
+// turned req.orient.angle[r] degrees counter-clockwise, stored word-major (crop = word * R + r).
+int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const Unit& u, const Request& req,
+                std::vector<PageOut>* results, Pending* pend) {
+  const tt_ocr_options& opt = req.opt;
   const cudaMemcpyKind page_kind = opt.pages_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
   const int nb = static_cast<int>(u.pages.size());
   const tt_image& first = pages[u.pages[0]];
@@ -199,7 +207,7 @@ int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const
   std::vector<CropBox> crops;
   std::vector<WarpBox> warps;   // cfg.rectify: one perspective warp per box instead of the axis-aligned crop
   const bool rectify = cfg.rectify != 0;
-  const int R = orient ? orient->n : 1;
+  const int R = req.orient.n;
   for (int b = 0; b < nb; ++b) {
     PageOut& po = (*results)[u.pages[b]];
     const tt_image& im = pages[u.pages[b]];
@@ -218,7 +226,7 @@ int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const
         Pt2f quad[4];
         rect_to_quad(adj, quad);
         for (int r = 0; r < R; ++r) {   // candidate angle a: the corners shifted cyclically by a / 90
-          const int sh = orient ? orient->angle[r] / 90 : 0;
+          const int sh = req.orient.angle[r] / 90;
           const Pt2f q[4] = {quad[sh & 3], quad[(sh + 1) & 3], quad[(sh + 2) & 3], quad[(sh + 3) & 3]};
           WarpBox wb{};
           wb.page = quad_to_warp(q, wb.m) ? b : -1;
@@ -232,7 +240,7 @@ int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const
       po.conf.assign(po.bbox.size(), -1.f);
       po.char_conf.resize(po.bbox.size());
     }
-    if (orient) po.angle.assign(po.bbox.size(), -1);
+    if (R > 1) po.angle.assign(po.bbox.size(), -1);
   }
   const int n = static_cast<int>(crops.size());
   if (opt.detect_only) {   // boxes only: nothing joins the recognition batch
@@ -257,9 +265,9 @@ int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const
     E_CUDA(cudaMemcpyAsync(warps_dev, warps.data(), sizeof(WarpBox) * nc, cudaMemcpyHostToDevice, d.stream));
     g_h2d_bytes += sizeof(WarpBox) * nc;
     E_TRY(crop_warp(refs_dev, warps_dev, nc, nullptr, d.patch_buf + have * 128 * 96, d.stream));
-  } else if (orient) {
+  } else if (R > 1) {
     std::vector<uint8_t> rot(nc);
-    for (int c = 0; c < nc; ++c) rot[c] = static_cast<uint8_t>(orient->angle[c % R] / 90);
+    for (int c = 0; c < nc; ++c) rot[c] = static_cast<uint8_t>(req.orient.angle[c % R] / 90);
     uint8_t* rot_dev = d.arena.get<uint8_t>(nc);
     if (!rot_dev) { set_error("arena exhausted (rotations)"); return 1; }
     E_CUDA(cudaMemcpyAsync(rot_dev, rot.data(), nc, cudaMemcpyHostToDevice, d.stream));
@@ -274,116 +282,72 @@ int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const
   return 0;
 }
 
-// PARSeq + tokenizer over the slot's recognition batch (tuatara.cpp:450-505).  scores: the refinement head also
-// writes each position's largest softmax probability, copied back next to the ids and decoded into conf / char_conf.
-// page_masks (null: no page of the request has a character filter): the class mask of every page of the request; each
-// crop decodes under its page's mask, uploaded per pass as [nc][4] words.
-int recognise_oriented(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, bool scores,
-                       const std::vector<ClassMask>* page_masks, const OrientSet& orient);
-int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, bool scores,
-              const std::vector<ClassMask>* page_masks, const OrientSet* orient) {
-  if (orient) return recognise_oriented(d, results, pend, scores, page_masks, *orient);
+// PARSeq + tokenizer over the slot's recognition batch (tuatara.cpp:450-505), which holds R = req.orient.n crops per
+// word.  A pass takes whole words (at most kMaxCropsPerPass crops).  With scores the refinement head also writes each
+// position's largest softmax probability, copied back next to the ids and decoded into conf / char_conf.  With
+// rotation candidates (R > 1) it always writes them, and orient_select leaves one candidate per word on the device, so
+// the copy back is the same ids (and pmax with scores) per word plus its 4-byte angle.  With filters (req.masks) each
+// crop decodes under its page's class mask, uploaded per pass as [nc][4] words.
+int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, const Request& req) {
   const int n = static_cast<int>(pend->owner.size());
-  const int L = d.w->pd.L;
-  for (int c0 = 0; c0 < n; c0 += kMaxCropsPerPass) {
-    const int nc = std::min(kMaxCropsPerPass, n - c0);
-    const size_t bytes = sizeof(int) * static_cast<size_t>(nc) * L;   // ids; with scores as many bytes of pmax follow
-    const size_t mask_bytes = page_masks ? sizeof(ClassMask) * nc : 0;
-    const size_t need = d.parseq_bytes(nc) + (4u << 20) + (scores ? bytes : 0) + mask_bytes;
-    if (need > d.arena.capacity()) E_TRY(stream_sync(d.stream));
-    E_TRY(d.arena.reserve(need));
-    d.arena.reset();
-    float* pmax = scores ? d.arena.get<float>(static_cast<size_t>(nc) * L) : nullptr;
-    if (scores && !pmax) { set_error("arena exhausted (pmax)"); return 1; }
-    uint32_t* mask = nullptr;
-    E_TRY(d.ensure_pinned(std::max(scores ? 2 * bytes : bytes, mask_bytes)));
-    if (page_masks) {
-      mask = d.arena.get<uint32_t>(4 * static_cast<size_t>(nc));
-      if (!mask) { set_error("arena exhausted (class masks)"); return 1; }
-      ClassMask* host_mask = reinterpret_cast<ClassMask*>(d.pinned);   // the ids' D2H below is ordered after this copy
-      for (int c = 0; c < nc; ++c) host_mask[c] = (*page_masks)[pend->owner[c0 + c].page];
-      E_CUDA(cudaMemcpyAsync(mask, host_mask, mask_bytes, cudaMemcpyHostToDevice, d.stream));
-      g_h2d_bytes += mask_bytes;
-    }
-    float* logits = nullptr;
-    int* ids = nullptr;
-    E_TRY(d.parseq_forward(d.patch_buf + static_cast<size_t>(c0) * 128 * 96, nc, nullptr, &logits, &ids, pmax, mask));
-    E_CUDA(cudaMemcpyAsync(d.pinned, ids, bytes, cudaMemcpyDeviceToHost, d.stream));
-    g_d2h_bytes += bytes;
-    if (scores) {
-      E_CUDA(cudaMemcpyAsync(d.pinned + bytes, pmax, bytes, cudaMemcpyDeviceToHost, d.stream));
-      g_d2h_bytes += bytes;
-    }
-    E_TRY(stream_sync(d.stream));
-    const int* host_ids = reinterpret_cast<const int*>(d.pinned);
-    const float* host_p = reinterpret_cast<const float*>(d.pinned + bytes);
-    for (int c = 0; c < nc; ++c) {   // tokenizer (tuatara.cpp:492-505)
-      const CropOwner& o = pend->owner[c0 + c];
-      PageOut& po = (*results)[o.page];
-      if (scores)
-        decode_ids_scored(host_ids + static_cast<size_t>(c) * L, host_p + static_cast<size_t>(c) * L, L, &po.text[o.box],
-                          &po.char_conf[o.box], &po.conf[o.box]);
-      else
-        po.text[o.box] = decode_ids(host_ids + static_cast<size_t>(c) * L, L);
-    }
-  }
-  pend->owner.clear();
-  pend->pages = 0;
-  return 0;
-}
-
-// recognise with rotation candidates: the batch holds orient.n crops per word.  A pass takes whole words (at most
-// kMaxCropsPerPass crops), the refinement head always writes pmax, and orient_select leaves one candidate per word on
-// the device, so the copy back is recognise's (ids, pmax with scores) plus the 4-byte angle per word.
-int recognise_oriented(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, bool scores,
-                       const std::vector<ClassMask>* page_masks, const OrientSet& orient) {
-  const int n = static_cast<int>(pend->owner.size());
-  const int L = d.w->pd.L, R = orient.n;
+  const int L = d.w->pd.L, R = req.orient.n;
+  const bool scores = req.opt.with_scores != 0;
   const int words_per_pass = kMaxCropsPerPass / R;
   for (int w0 = 0; w0 < n; w0 += words_per_pass) {
     const int nw = std::min(words_per_pass, n - w0);
     const int nc = nw * R;
-    const size_t bytes = sizeof(int) * static_cast<size_t>(nw) * L;   // winner ids; with scores as many bytes of pmax follow
-    const size_t angle_bytes = sizeof(int) * static_cast<size_t>(nw);
-    const size_t mask_bytes = page_masks ? sizeof(ClassMask) * nc : 0;
-    const size_t need = d.parseq_bytes(nc) + (4u << 20) + sizeof(float) * static_cast<size_t>(nc) * L + 2 * bytes +
-                        angle_bytes + mask_bytes;
+    const size_t bytes = sizeof(int) * static_cast<size_t>(nw) * L;   // ids per word; with scores as many bytes of pmax
+    const size_t angle_bytes = R > 1 ? sizeof(int) * static_cast<size_t>(nw) : 0;
+    const size_t pmax_bytes = scores || R > 1 ? sizeof(float) * static_cast<size_t>(nc) * L : 0;
+    const size_t mask_bytes = req.masks.empty() ? 0 : sizeof(ClassMask) * nc;
+    const size_t need = d.parseq_bytes(nc) + (4u << 20) + pmax_bytes + (R > 1 ? 2 * bytes + angle_bytes : 0) + mask_bytes;
     if (need > d.arena.capacity()) E_TRY(stream_sync(d.stream));
     E_TRY(d.arena.reserve(need));
     d.arena.reset();
-    float* pmax = d.arena.get<float>(static_cast<size_t>(nc) * L);
-    int* win_ids = d.arena.get<int>(static_cast<size_t>(nw) * L);
-    float* win_p = d.arena.get<float>(static_cast<size_t>(nw) * L);
-    int* win_angle = d.arena.get<int>(nw);
-    if (!pmax || !win_ids || !win_p || !win_angle) { set_error("arena exhausted (orientation)"); return 1; }
-    uint32_t* mask = nullptr;
+    float* pmax = pmax_bytes ? d.arena.get<float>(static_cast<size_t>(nc) * L) : nullptr;
+    if (pmax_bytes && !pmax) { set_error("arena exhausted (pmax)"); return 1; }
+    int* win_ids = nullptr;   // R > 1: the winning candidate of every word
+    float* win_p = nullptr;
+    int* win_angle = nullptr;
+    if (R > 1) {
+      win_ids = d.arena.get<int>(static_cast<size_t>(nw) * L);
+      win_p = d.arena.get<float>(static_cast<size_t>(nw) * L);
+      win_angle = d.arena.get<int>(nw);
+      if (!win_ids || !win_p || !win_angle) { set_error("arena exhausted (orientation)"); return 1; }
+    }
+    // pinned staging: ids | angle | pmax on the way back, the class masks on the way in
     E_TRY(d.ensure_pinned(std::max((scores ? 2 * bytes : bytes) + angle_bytes, mask_bytes)));
-    if (page_masks) {
+    uint32_t* mask = nullptr;
+    if (!req.masks.empty()) {
       mask = d.arena.get<uint32_t>(4 * static_cast<size_t>(nc));
       if (!mask) { set_error("arena exhausted (class masks)"); return 1; }
       ClassMask* host_mask = reinterpret_cast<ClassMask*>(d.pinned);   // the ids' D2H below is ordered after this copy
-      for (int c = 0; c < nc; ++c) host_mask[c] = (*page_masks)[pend->owner[w0 + c / R].page];
+      for (int c = 0; c < nc; ++c) host_mask[c] = req.masks[pend->owner[w0 + c / R].page];
       E_CUDA(cudaMemcpyAsync(mask, host_mask, mask_bytes, cudaMemcpyHostToDevice, d.stream));
       g_h2d_bytes += mask_bytes;
     }
     float* logits = nullptr;
     int* ids = nullptr;
     E_TRY(d.parseq_forward(d.patch_buf + static_cast<size_t>(w0) * R * 128 * 96, nc, nullptr, &logits, &ids, pmax, mask));
-    stage_begin(d.stream);
-    E_TRY(orient_select(ids, pmax, nw, L, orient, win_ids, scores ? win_p : nullptr, win_angle, d.stream));
-    stage_end(d.stream, "orient_select", 0.0, static_cast<double>(nc) * L * 8 + static_cast<double>(nw) * (L * 8 + 4));
-    E_CUDA(cudaMemcpyAsync(d.pinned, win_ids, bytes, cudaMemcpyDeviceToHost, d.stream));
-    E_CUDA(cudaMemcpyAsync(d.pinned + bytes, win_angle, angle_bytes, cudaMemcpyDeviceToHost, d.stream));
+    if (R > 1) {
+      stage_begin(d.stream);
+      E_TRY(orient_select(ids, pmax, nw, L, req.orient, win_ids, scores ? win_p : nullptr, win_angle, d.stream));
+      stage_end(d.stream, "orient_select", 0.0, static_cast<double>(nc) * L * 8 + static_cast<double>(nw) * (L * 8 + 4));
+      ids = win_ids;
+      pmax = win_p;
+    }
+    E_CUDA(cudaMemcpyAsync(d.pinned, ids, bytes, cudaMemcpyDeviceToHost, d.stream));
+    if (R > 1) E_CUDA(cudaMemcpyAsync(d.pinned + bytes, win_angle, angle_bytes, cudaMemcpyDeviceToHost, d.stream));
     g_d2h_bytes += bytes + angle_bytes;
     if (scores) {
-      E_CUDA(cudaMemcpyAsync(d.pinned + bytes + angle_bytes, win_p, bytes, cudaMemcpyDeviceToHost, d.stream));
+      E_CUDA(cudaMemcpyAsync(d.pinned + bytes + angle_bytes, pmax, bytes, cudaMemcpyDeviceToHost, d.stream));
       g_d2h_bytes += bytes;
     }
     E_TRY(stream_sync(d.stream));
     const int* host_ids = reinterpret_cast<const int*>(d.pinned);
     const int* host_angle = reinterpret_cast<const int*>(d.pinned + bytes);
     const float* host_p = reinterpret_cast<const float*>(d.pinned + bytes + angle_bytes);
-    for (int w = 0; w < nw; ++w) {
+    for (int w = 0; w < nw; ++w) {   // tokenizer (tuatara.cpp:492-505)
       const CropOwner& o = pend->owner[w0 + w];
       PageOut& po = (*results)[o.page];
       if (scores)
@@ -391,7 +355,7 @@ int recognise_oriented(DeviceCtx& d, std::vector<PageOut>* results, Pending* pen
                           &po.char_conf[o.box], &po.conf[o.box]);
       else
         po.text[o.box] = decode_ids(host_ids + static_cast<size_t>(w) * L, L);
-      po.angle[o.box] = host_angle[w];
+      if (R > 1) po.angle[o.box] = host_angle[w];
     }
   }
   pend->owner.clear();
@@ -417,8 +381,7 @@ struct WorkQueues {
 };
 
 // One execution slot draining the queues.
-void slot_worker(tt_engine& e, int g, int sidx, int want, const tt_image* pages, const tt_ocr_options& opt,
-                 const std::vector<ClassMask>* page_masks, const OrientSet* orient, WorkQueues* q,
+void slot_worker(tt_engine& e, int g, int sidx, int want, const tt_image* pages, const Request& req, WorkQueues* q,
                  std::vector<PageOut>* results, int* rc, std::string* err) {
   // take an idle slot of this GPU if there is one (concurrent callers spread over the slots), else queue on our own
   DeviceCtx* dp = nullptr;
@@ -437,20 +400,56 @@ void slot_worker(tt_engine& e, int g, int sidx, int want, const tt_image* pages,
   const int max_b = cfg.max_batch_pages > 0 ? cfg.max_batch_pages : 32;
   Pending pend;
   for (int ui = q->pop(g); ui >= 0; ui = q->pop(g)) {
-    if (detect_unit(d, cfg, pages, q->units[ui], opt, orient, results, &pend)) { *err = last_error(); *rc = 1; return; }
-    if (pend.pages >= max_b && recognise(d, results, &pend, opt.with_scores != 0, page_masks, orient)) {
-      *err = last_error();
-      *rc = 1;
-      return;
-    }
+    if (detect_unit(d, cfg, pages, q->units[ui], req, results, &pend)) { *err = last_error(); *rc = 1; return; }
+    if (pend.pages >= max_b && recognise(d, results, &pend, req)) { *err = last_error(); *rc = 1; return; }
   }
-  if (recognise(d, results, &pend, opt.with_scores != 0, page_masks, orient)) { *err = last_error(); *rc = 1; return; }
+  if (recognise(d, results, &pend, req)) { *err = last_error(); *rc = 1; return; }
 }
 
-int ocr_pages(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt_in,
-              const std::vector<ClassMask>* page_masks, const OrientSet* orient, tt_result** out);
-int ocr_pages_filtered(const char* fn, tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
-                       const tt_char_filter* filters, int n_filters, const OrientSet* orient, tt_result** out);
+// The argument checks of the tt_ocr_pages* entry points (fn: the one called, named in the messages), made before any
+// device work: the rotation candidates, then the filters, turned into one class mask per page.  ocr_pages checks the
+// engine and the pages.
+int make_request(const char* fn, const tt_ocr_options* opt, const tt_char_filter* filters, int n_filters,
+                 const int* rotation_info, int n_rotations, int n_pages, Request* req) {
+  try {
+    if (opt) req->opt = *opt;
+    if (n_rotations < 0 || (n_rotations > 0 && !rotation_info)) {
+      set_error(std::string(fn) + ": rotation_info is NULL or n_rotations (" + std::to_string(n_rotations) + ") is negative");
+      return 1;
+    }
+    bool seen[4] = {true, false, false, false};
+    for (int i = 0; i < n_rotations; ++i) {
+      const int a = rotation_info[i];
+      if (a != 90 && a != 180 && a != 270) {
+        set_error(std::string(fn) + ": rotation_info holds " + std::to_string(a) + "; the angles are 90, 180 and 270");
+        return 1;
+      }
+      if (seen[a / 90]) { set_error(std::string(fn) + ": rotation_info holds " + std::to_string(a) + " twice"); return 1; }
+      seen[a / 90] = true;
+    }
+    req->orient.n = 0;
+    for (int q = 0; q < 4; ++q)
+      if (seen[q]) req->orient.angle[req->orient.n++] = 90 * q;
+    if (n_filters == 0) return 0;
+    if (!filters) { set_error(std::string(fn) + ": filters is NULL but n_filters is " + std::to_string(n_filters)); return 1; }
+    if (n_filters != 1 && n_filters != n_pages) {
+      set_error(std::string(fn) + ": n_filters must be 0, 1 or n_pages (" + std::to_string(n_pages) + "), got " +
+                std::to_string(n_filters));
+      return 1;
+    }
+    req->masks.resize(std::max(n_pages, 0));
+    for (int i = 0; i < n_pages; ++i) {
+      const tt_char_filter& f = filters[n_filters == 1 ? 0 : i];
+      char_filter_mask(f.allow, f.block, req->masks[i].data());
+    }
+    return 0;
+  } catch (const std::exception& ex) {
+    set_error(std::string(fn) + ": " + ex.what());
+    return 1;
+  }
+}
+
+int ocr_pages(tt_engine* e, const tt_image* pages, int n_pages, const Request& req, tt_result** out);
 
 }  // namespace
 
@@ -546,72 +545,32 @@ int tt_ocr_pages(tt_engine* e, const tt_image* pages, int n_pages, tt_result** o
 }
 
 int tt_ocr_pages_ex(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt, tt_result** out) {
-  return ocr_pages(e, pages, n_pages, opt, nullptr, nullptr, out);
+  Request req;
+  return make_request("tt_ocr_pages_ex", opt, nullptr, 0, nullptr, 0, n_pages, &req) ? 1 : ocr_pages(e, pages, n_pages, req, out);
 }
 
 int tt_ocr_pages_filtered(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
                           const tt_char_filter* filters, int n_filters, tt_result** out) {
-  return ocr_pages_filtered("tt_ocr_pages_filtered", e, pages, n_pages, opt, filters, n_filters, nullptr, out);
+  Request req;
+  return make_request("tt_ocr_pages_filtered", opt, filters, n_filters, nullptr, 0, n_pages, &req)
+             ? 1 : ocr_pages(e, pages, n_pages, req, out);
 }
 
 int tt_ocr_pages_oriented(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
                           const tt_char_filter* filters, int n_filters, const int* rotation_info, int n_rotations,
                           tt_result** out) {
-  if (n_rotations == 0)
-    return ocr_pages_filtered("tt_ocr_pages_oriented", e, pages, n_pages, opt, filters, n_filters, nullptr, out);
-  if (n_rotations < 0 || !rotation_info) {
-    set_error("tt_ocr_pages_oriented: rotation_info is NULL or n_rotations (" + std::to_string(n_rotations) + ") is negative");
-    return 1;
-  }
-  bool seen[4] = {true, false, false, false};
-  for (int i = 0; i < n_rotations; ++i) {
-    const int a = rotation_info[i];
-    if (a != 90 && a != 180 && a != 270) {
-      set_error("tt_ocr_pages_oriented: rotation_info holds " + std::to_string(a) + "; the angles are 90, 180 and 270");
-      return 1;
-    }
-    if (seen[a / 90]) { set_error("tt_ocr_pages_oriented: rotation_info holds " + std::to_string(a) + " twice"); return 1; }
-    seen[a / 90] = true;
-  }
-  OrientSet set{0, {0, 0, 0, 0}};
-  for (int q = 0; q < 4; ++q)
-    if (seen[q]) set.angle[set.n++] = 90 * q;
-  return ocr_pages_filtered("tt_ocr_pages_oriented", e, pages, n_pages, opt, filters, n_filters, &set, out);
+  Request req;
+  return make_request("tt_ocr_pages_oriented", opt, filters, n_filters, rotation_info, n_rotations, n_pages, &req)
+             ? 1 : ocr_pages(e, pages, n_pages, req, out);
 }
 
 }  // extern "C"
 
 namespace {
-// tt_ocr_pages_filtered and tt_ocr_pages_oriented: the filters checked and turned into one class mask per page
-int ocr_pages_filtered(const char* fn, tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
-                       const tt_char_filter* filters, int n_filters, const OrientSet* orient, tt_result** out) {
+// every tt_ocr_pages* entry point, after make_request
+int ocr_pages(tt_engine* e, const tt_image* pages, int n_pages, const Request& req, tt_result** out) {
   try {
-    if (n_filters == 0) return ocr_pages(e, pages, n_pages, opt, nullptr, orient, out);
-    if (!filters) { set_error(std::string(fn) + ": filters is NULL but n_filters is " + std::to_string(n_filters)); return 1; }
-    if (n_filters != 1 && n_filters != n_pages) {
-      set_error(std::string(fn) + ": n_filters must be 0, 1 or n_pages (" + std::to_string(n_pages) + "), got " +
-                std::to_string(n_filters));
-      return 1;
-    }
-    std::vector<ClassMask> masks(std::max(n_pages, 0));
-    for (int i = 0; i < n_pages; ++i) {
-      const tt_char_filter& f = filters[n_filters == 1 ? 0 : i];
-      char_filter_mask(f.allow, f.block, masks[i].data());
-    }
-    return ocr_pages(e, pages, n_pages, opt, &masks, orient, out);
-  } catch (const std::exception& ex) {
-    set_error(std::string(fn) + ": " + ex.what());
-    return 1;
-  }
-}
-
-// tt_ocr_pages_ex, tt_ocr_pages_filtered and tt_ocr_pages_oriented (page_masks: one class mask per page, null without
-// filters; orient: the rotation candidates, null without)
-int ocr_pages(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt_in,
-              const std::vector<ClassMask>* page_masks, const OrientSet* orient, tt_result** out) {
-  try {
-    tt_ocr_options opt{0, 0, nullptr, 0, 0};
-    if (opt_in) opt = *opt_in;
+    const tt_ocr_options& opt = req.opt;
     if (!e || !out) { set_error("tt_ocr_pages: null argument"); return 1; }
     if (n_pages < 0 || (n_pages > 0 && !pages)) { set_error("tt_ocr_pages: bad page array"); return 1; }
     for (int i = 0; i < n_pages; ++i) {
@@ -658,11 +617,9 @@ int ocr_pages(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_opt
     std::vector<int> rcs(ws.size(), 0);
     std::vector<std::thread> workers;
     for (size_t w = 1; w < ws.size(); ++w)
-      workers.emplace_back([&, w] {
-        slot_worker(*e, ws[w].g, ws[w].sidx, want, pages, opt, page_masks, orient, &q, &results, &rcs[w], &errs[w]);
-      });
+      workers.emplace_back([&, w] { slot_worker(*e, ws[w].g, ws[w].sidx, want, pages, req, &q, &results, &rcs[w], &errs[w]); });
     if (!ws.empty())
-      slot_worker(*e, ws[0].g, ws[0].sidx, want, pages, opt, page_masks, orient, &q, &results, &rcs[0], &errs[0]);
+      slot_worker(*e, ws[0].g, ws[0].sidx, want, pages, req, &q, &results, &rcs[0], &errs[0]);
     for (auto& w : workers) w.join();
     for (size_t w = 0; w < ws.size(); ++w)
       if (rcs[w]) { set_error("device " + std::to_string(e->devs[ws[w].g * kSlotsPerDevice]->device) + ": " + errs[w]); return 1; }
@@ -682,7 +639,7 @@ int ocr_pages(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_opt
         std::memcpy(pr.items[k].bbox, po.bbox[k].data(), sizeof(float) * 4);
       }
     }
-    if (orient) {
+    if (req.orient.n > 1) {
       rb->angles = new std::vector<std::vector<int>>(n_pages);
       for (int i = 0; i < n_pages; ++i) (*rb->angles)[i] = std::move(results[i].angle);
     }
