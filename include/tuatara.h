@@ -64,6 +64,42 @@ struct CharFilter {
   const char* block = nullptr;
 };
 
+// A caller's word list (tt_lexicon, INTEGRATION.md section 9): every word recognised under it is one of its words.
+// Build it once and pass it to as many calls as needed; it is immutable.  Move-only.  A list that tt_lexicon_create
+// rejects gives !ok() and error() says why; the entry points print that and return {} when given it.
+class Lexicon {
+ public:
+  Lexicon() = default;
+  explicit Lexicon(const std::vector<std::string>& words) {
+    std::vector<const char*> p;
+    for (const std::string& w : words) p.push_back(w.c_str());
+    if (tt_lexicon_create(p.data(), static_cast<int>(p.size()), &h_) != 0) {
+      h_ = nullptr;
+      err_ = tt_last_error();
+    }
+  }
+  ~Lexicon() { if (h_) tt_lexicon_destroy(h_); }
+  Lexicon(Lexicon&& o) noexcept : h_(o.h_), err_(std::move(o.err_)) { o.h_ = nullptr; }
+  Lexicon& operator=(Lexicon&& o) noexcept {
+    if (this != &o) {
+      if (h_) tt_lexicon_destroy(h_);
+      h_ = o.h_;
+      err_ = std::move(o.err_);
+      o.h_ = nullptr;
+    }
+    return *this;
+  }
+  Lexicon(const Lexicon&) = delete;
+  Lexicon& operator=(const Lexicon&) = delete;
+  bool ok() const { return h_ != nullptr; }
+  const std::string& error() const { return err_; }
+  const tt_lexicon* get() const { return h_; }
+
+ private:
+  tt_lexicon* h_ = nullptr;
+  std::string err_ = "empty lexicon";
+};
+
 namespace detail {
 inline tt_engine* engine_for(const std::string& weights_dir) {
   static std::mutex mu;
@@ -86,12 +122,14 @@ inline tt_engine* engine_for(const std::string& weights_dir) {
 
 namespace detail {
 // The one path of every entry point: the checks, the soft failures ({} after printing the reason), one
-// tt_ocr_pages_oriented call and the walk over its result.  Each item's scores are fetched when `scores`, its angle when
-// rotation_info is not empty.  filters: none (empty), one for every page, or one per page.
+// tt_ocr_pages_lexicon call and the walk over its result.  Each item's scores are fetched when `scores`, its angle when
+// rotation_info is not empty.  filters: none (empty), one for every page, or one per page.  lexicons (tt_lexicon
+// handles): likewise; a null entry is a page without lexicon.
 inline std::vector<std::vector<ScoredItem>> ocr_pages(const std::vector<ImageView>& images, const std::string& weights_dir,
                                                       const std::string& outputs_dir, bool scores,
                                                       const std::vector<CharFilter>& filters,
-                                                      const std::vector<int>& rotation_info = {}) {
+                                                      const std::vector<int>& rotation_info = {},
+                                                      const std::vector<const tt_lexicon*>& lexicons = {}) {
   std::vector<std::vector<ScoredItem>> out;
   if (weights_dir.empty()) { std::cerr << "Please provide a value for weights_dir" << std::endl; return out; }
   if (outputs_dir.empty()) { std::cerr << "Please provide a value for outputs_dir" << std::endl; return out; }
@@ -108,8 +146,9 @@ inline std::vector<std::vector<ScoredItem>> ocr_pages(const std::vector<ImageVie
   tt_ocr_options opt = {};
   opt.with_scores = scores ? 1 : 0;
   tt_result* r = nullptr;
-  if (tt_ocr_pages_oriented(e, pages.data(), static_cast<int>(pages.size()), &opt, f.data(), static_cast<int>(f.size()),
-                            rotation_info.data(), static_cast<int>(rotation_info.size()), &r) != 0) {
+  if (tt_ocr_pages_lexicon(e, pages.data(), static_cast<int>(pages.size()), &opt, f.data(), static_cast<int>(f.size()),
+                           rotation_info.data(), static_cast<int>(rotation_info.size()), lexicons.data(),
+                           static_cast<int>(lexicons.size()), &r) != 0) {
     std::cerr << "tuatara: " << tt_last_error() << std::endl;
     return out;
   }
@@ -133,6 +172,19 @@ inline std::vector<std::vector<ScoredItem>> ocr_pages(const std::vector<ImageVie
     }
   tt_result_free(r);
   return out;
+}
+
+// ocr_pages with Lexicon objects (null: a page without lexicon); one that is not ok() prints its error and gives {}.
+inline std::vector<std::vector<ScoredItem>> ocr_pages_lex(const std::vector<ImageView>& images, const std::string& weights_dir,
+                                                          const std::string& outputs_dir, bool scores,
+                                                          const std::vector<int>& rotation_info,
+                                                          const std::vector<const Lexicon*>& lexicons) {
+  std::vector<const tt_lexicon*> h;
+  for (const Lexicon* l : lexicons) {
+    if (l && !l->ok()) { std::cerr << "tuatara: " << l->error() << std::endl; return {}; }
+    h.push_back(l ? l->get() : nullptr);
+  }
+  return ocr_pages(images, weights_dir, outputs_dir, scores, {}, rotation_info, h);
 }
 
 inline std::vector<std::vector<OutputItem>> unscored(std::vector<std::vector<ScoredItem>> pages) {
@@ -208,6 +260,65 @@ inline std::vector<ScoredItem> image_to_data_oriented(const ImageView& image, co
   return pages.empty() ? std::vector<ScoredItem>{} : pages[0];
 }
 
+// Lexicons (tt_ocr_pages_lexicon, INTEGRATION.md section 9): every recognised word is one of the lexicon's words.  One
+// lexicon for every page, or one pointer per page (nullptr: the page reads as without lexicon).  Same soft failures.
+inline std::vector<std::vector<OutputItem>> image_to_data_batch(const std::vector<ImageView>& images,
+                                                                const std::string& weights_dir,
+                                                                const std::string& outputs_dir, const Lexicon& lexicon) {
+  return detail::unscored(detail::ocr_pages_lex(images, weights_dir, outputs_dir, false, {}, {&lexicon}));
+}
+
+inline std::vector<std::vector<OutputItem>> image_to_data_batch(const std::vector<ImageView>& images,
+                                                                const std::string& weights_dir,
+                                                                const std::string& outputs_dir,
+                                                                const std::vector<const Lexicon*>& lexicons) {
+  return detail::unscored(detail::ocr_pages_lex(images, weights_dir, outputs_dir, false, {}, lexicons));
+}
+
+inline std::vector<std::vector<ScoredItem>> image_to_data_scored_batch(const std::vector<ImageView>& images,
+                                                                       const std::string& weights_dir,
+                                                                       const std::string& outputs_dir,
+                                                                       const Lexicon& lexicon) {
+  return detail::ocr_pages_lex(images, weights_dir, outputs_dir, true, {}, {&lexicon});
+}
+
+inline std::vector<std::vector<ScoredItem>> image_to_data_scored_batch(const std::vector<ImageView>& images,
+                                                                       const std::string& weights_dir,
+                                                                       const std::string& outputs_dir,
+                                                                       const std::vector<const Lexicon*>& lexicons) {
+  return detail::ocr_pages_lex(images, weights_dir, outputs_dir, true, {}, lexicons);
+}
+
+inline std::vector<ScoredItem> image_to_data_scored(const ImageView& image, const std::string& weights_dir,
+                                                    const std::string& outputs_dir, const Lexicon& lexicon) {
+  std::vector<std::vector<ScoredItem>> pages = image_to_data_scored_batch({image}, weights_dir, outputs_dir, lexicon);
+  return pages.empty() ? std::vector<ScoredItem>{} : pages[0];
+}
+
+inline std::vector<std::vector<ScoredItem>> image_to_data_oriented_batch(const std::vector<ImageView>& images,
+                                                                         const std::string& weights_dir,
+                                                                         const std::string& outputs_dir,
+                                                                         const std::vector<int>& rotation_info,
+                                                                         const Lexicon& lexicon) {
+  return detail::ocr_pages_lex(images, weights_dir, outputs_dir, true, rotation_info, {&lexicon});
+}
+
+inline std::vector<std::vector<ScoredItem>> image_to_data_oriented_batch(const std::vector<ImageView>& images,
+                                                                         const std::string& weights_dir,
+                                                                         const std::string& outputs_dir,
+                                                                         const std::vector<int>& rotation_info,
+                                                                         const std::vector<const Lexicon*>& lexicons) {
+  return detail::ocr_pages_lex(images, weights_dir, outputs_dir, true, rotation_info, lexicons);
+}
+
+inline std::vector<ScoredItem> image_to_data_oriented(const ImageView& image, const std::string& weights_dir,
+                                                      const std::string& outputs_dir, const std::vector<int>& rotation_info,
+                                                      const Lexicon& lexicon) {
+  std::vector<std::vector<ScoredItem>> pages =
+      image_to_data_oriented_batch({image}, weights_dir, outputs_dir, rotation_info, lexicon);
+  return pages.empty() ? std::vector<ScoredItem>{} : pages[0];
+}
+
 }  // namespace tuatara
 
 inline std::vector<OutputItem> image_to_data(const tuatara::ImageView& image, std::string weights_dir,
@@ -220,6 +331,13 @@ inline std::vector<OutputItem> image_to_data(const tuatara::ImageView& image, st
 inline std::vector<OutputItem> image_to_data(const tuatara::ImageView& image, std::string weights_dir,
                                              std::string outputs_dir, const tuatara::CharFilter& filter) {
   auto pages = tuatara::image_to_data_batch({image}, weights_dir, outputs_dir, std::vector<tuatara::CharFilter>{filter});
+  return pages.empty() ? std::vector<OutputItem>{} : pages[0];
+}
+
+// image_to_data with a lexicon: every item's text is one of its words.
+inline std::vector<OutputItem> image_to_data(const tuatara::ImageView& image, std::string weights_dir,
+                                             std::string outputs_dir, const tuatara::Lexicon& lexicon) {
+  auto pages = tuatara::image_to_data_batch({image}, weights_dir, outputs_dir, lexicon);
   return pages.empty() ? std::vector<OutputItem>{} : pages[0];
 }
 

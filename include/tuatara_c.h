@@ -144,6 +144,34 @@ TT_API int tt_item_scores(const tt_result* r, int page, int item, float* conf, f
 TT_API int tt_ocr_pages_oriented(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
                                  const tt_char_filter* filters, int n_filters, const int* rotation_info, int n_rotations,
                                  tt_result** out);
+/* Lexicons (INTEGRATION.md section 9): every recognised word is read from a caller's word list.  Class c of the 95 prints
+ * itos[c] (tt_tokenizer_table); class 0 ends the word, class 88 prints nothing and backslash is printed by classes 69 and 87.
+ *  Words: 1..25 bytes each, every byte printed by a class of 1..94 other than 88 (so not ']', '~', a control byte or a
+ *    non-ASCII byte).  Anything else is an error naming the word's index and the byte (or the length); so are
+ *    words == NULL and n_words < 1.  Duplicates count once.
+ *  Automaton: a trie over the words.  A state allows class 0 iff a word ends there, and class c (1..94, not 88) iff a
+ *    word continues with itos[c] (both backslash classes lead to the same child).  After class 0 the crop is in a done
+ *    state that allows every class and loops to itself; nothing decoded there reaches the text.
+ *  Greedy choice: at every AR step the token fed back is the first maximum over the classes the crop's state allows (the
+ *    lowest allowed class when no allowed logit compares, i.e. all are NaN); the state then advances by it.  The ids are a
+ *    second walk over the refinement logits from the root with the same rule, and with scores p[t] of tt_item_scores is
+ *    renormalised over the classes the state at position t allows.  Rotation candidates are chosen by that conf.
+ * A tt_lexicon is immutable: concurrent requests may share it; destroy it once they have returned. */
+typedef struct tt_lexicon tt_lexicon;
+TT_API int tt_lexicon_create(const char* const* words, int n_words, tt_lexicon** out);
+TT_API void tt_lexicon_destroy(tt_lexicon* lex);
+/* n_words: the distinct words; n_states: the states of the trie (the root included, the done state not).  Both nullable. */
+TT_API int tt_lexicon_info(const tt_lexicon* lex, int* n_words, int* n_states);
+/* tt_ocr_pages_oriented with lexicons.  n_lexicons == 1: lexicons[0] for every page; == n_pages: lexicons[i] for page i;
+ * == 0 (lexicons may be NULL): exactly tt_ocr_pages_oriented.  Any other count, or lexicons == NULL with n_lexicons > 0, is
+ * an error.  A NULL entry decodes its page under a one-state automaton allowing its filter's classes (every class without
+ * a filter): its results are bit-identical to tt_ocr_pages_oriented's.  A page with a filter and a lexicon reads from the
+ * lexicon's words whose every character the filter allows; none is an error naming the page.  Every check is made
+ * before any device work.  Each item's text is then one of its page's words (or empty for a detect_only request);
+ * bbox, det_score and item order do not change. */
+TT_API int tt_ocr_pages_lexicon(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
+                                const tt_char_filter* filters, int n_filters, const int* rotation_info, int n_rotations,
+                                const tt_lexicon* const* lexicons, int n_lexicons, tt_result** out);
 /* The angle (0, 90, 180 or 270) of the candidate that was read for item `item` of page `page`, -1 when the item was not
  * recognised (detect_only).  An error on a result not made by tt_ocr_pages_oriented with n_rotations > 0. */
 TT_API int tt_item_angle(const tt_result* r, int page, int item, int* angle);
@@ -220,6 +248,12 @@ TT_API int tt_parseq_forward_scores(tt_engine* e, const uint8_t* crops, int n, i
  * raw, unmasked head output.  Every output pointer may be NULL. */
 TT_API int tt_parseq_forward_masked(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens,
                                     const uint32_t* class_masks, float* logits_out, int32_t* ids_out, float* pmax_out);
+/* tt_parseq_forward_masked with one lexicon for every crop instead of class masks: every AR step feeds back the choice of
+ * the crop's trie walk (forced_tokens, when given, win and the AR steps do not consult the trie), and ids_out / pmax_out
+ * are the refinement walk's.  logits_out holds the raw head output (TT_PARSEQ_AR_LOGITS=1: the AR pass's, like the other
+ * forwards).  Every output pointer may be NULL. */
+TT_API int tt_parseq_forward_lexicon(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens,
+                                     const tt_lexicon* lex, float* logits_out, int32_t* ids_out, float* pmax_out);
 /* Tokenizer::decode + truncation (tuatara.cpp:61-116, :497-502). ids [n][len]; out [n][out_stride] chars. */
 TT_API int tt_decode(const int32_t* ids, int n, int len, char* out, int out_stride);
 /* tt_decode with the scores of tt_item_scores (host only).  pmax [n][len]; conf_out (nullable) [n];
@@ -294,6 +328,10 @@ TT_API int tt_dec_cross_attn_dev(int n_crops, int D, int heads, int L, int p0, i
  * pmax_out [n_words][26] (nullable) and angle_out [n_words].  Device pointers except angles. */
 TT_API int tt_orient_select_dev(const int32_t* ids, const float* pmax, int n_words, const int32_t* angles, int n_candidates,
                                 int32_t* ids_out, float* pmax_out, int32_t* angle_out, void* stream);
+/* Kernel test of the lexicon refinement head: the walk of lex's trie over device logits fp32 [n][26][95], every crop from
+ * the root.  Writes ids_out int32 [n][26] and pmax_out fp32 [n][26] (nullable), device pointers. */
+TT_API int tt_lexicon_walk_dev(const tt_lexicon* lex, const float* logits, int n, int32_t* ids_out, float* pmax_out,
+                               void* stream);
 /* Batched device-side post-processing (bench): maps_dev [batch][H][W][2] fp32. Returns total rects. */
 TT_API int tt_postprocess_dev(tt_engine* e, const float* maps_dev, int batch, int H, int W, int* n_rects_total,
                        void* stream);

@@ -18,7 +18,7 @@ from ._native import TuataraError, check, lib, ptr
 __all__ = [
     "TuataraError", "Engine", "image_to_data", "images_to_data", "image_to_data_scored", "images_to_data_scored",
     "default_config", "resize_plan", "preprocess", "postprocess", "crop_resize", "decode_ids", "decode_scores", "tokenizer_table",
-    "char_filter_mask", "min_area_rect", "convex_hull",
+    "char_filter_mask", "Lexicon", "min_area_rect", "convex_hull",
     "rect_points", "rect_bounding", "adjust_rect", "rect_to_bbox", "launch_count",
 ]
 
@@ -82,6 +82,71 @@ def _filters(allowlist, blocklist, n_pages: int):
         else:
             cols.append([_filter_bytes(v, name)] * n)
     return (_native.tt_char_filter * n)(*[_native.tt_char_filter(a, b) for a, b in zip(*cols)])
+
+
+class Lexicon:
+    """A reusable word list (tt_lexicon, INTEGRATION.md section 9): every word recognised under it is one of its words.
+    words: an iterable of str, each 1..25 characters that PARSeq can print (no ']', '~', control or non-ASCII
+    characters); duplicates count once.  Build it once and pass it as ``lexicon=`` to as many calls as needed."""
+
+    def __init__(self, words):
+        if isinstance(words, (str, bytes)) or not hasattr(words, "__iter__"):
+            raise TypeError("Lexicon: expected an iterable of str")
+        ws = list(words)
+        for i, w in enumerate(ws):
+            if not isinstance(w, str):
+                raise TypeError(f"Lexicon: word {i} is a {type(w).__name__}, expected str")
+            if "\0" in w:
+                raise TuataraError(f"tt_lexicon_create: word {i} holds byte 0x00, which no class prints")
+        arr = (C.c_char_p * max(len(ws), 1))(*[w.encode() for w in ws])
+        self._h = C.c_void_p()
+        check(lib().tt_lexicon_create(arr, len(ws), C.byref(self._h)), "tt_lexicon_create")
+
+    def info(self) -> tuple[int, int]:
+        """-> (distinct words, states of the trie)."""
+        nw, ns = C.c_int(), C.c_int()
+        check(lib().tt_lexicon_info(self._h, C.byref(nw), C.byref(ns)), "tt_lexicon_info")
+        return nw.value, ns.value
+
+    def close(self):
+        if getattr(self, "_h", None) and self._h.value:
+            lib().tt_lexicon_destroy(self._h)
+            self._h = C.c_void_p()
+
+    __del__ = close
+
+
+def _is_words(v) -> bool:
+    return not isinstance(v, (str, bytes, Lexicon)) and v is not None and hasattr(v, "__iter__")
+
+
+def _lexicon_arg(lexicon, n_pages: int, strict: bool):
+    """lexicon keyword -> (a list of Lexicon or None, one entry or one per page) or None.  It is a Lexicon or an iterable
+    of str (one lexicon for every page), or a list with one entry per page, each None or one of those (strict: each None
+    or a Lexicon, so that a list of str is always one word list)."""
+    if lexicon is None:
+        return None
+    if isinstance(lexicon, Lexicon):
+        return [lexicon]
+    if isinstance(lexicon, (str, bytes)) or not hasattr(lexicon, "__iter__"):
+        raise TypeError("lexicon: expected a Lexicon, an iterable of str or a list with one entry per page")
+    vals = list(lexicon)
+    if all(isinstance(v, str) for v in vals):
+        return [Lexicon(vals)]
+    ok = (lambda v: v is None or isinstance(v, Lexicon)) if strict else (lambda v: v is None or isinstance(v, Lexicon) or _is_words(v))
+    if not isinstance(lexicon, (list, tuple)) or not all(ok(v) for v in vals):
+        raise TypeError("lexicon: a list with one entry per page holds " +
+                        ("Lexicon objects or None" if strict else "None, Lexicon objects or iterables of str") +
+                        ", and a word list holds only str")
+    if len(vals) != n_pages:
+        raise ValueError(f"lexicon: expected one entry per page ({n_pages}), got {len(vals)}")
+    return [v if v is None or isinstance(v, Lexicon) else Lexicon(v) for v in vals]
+
+
+def _engine_lexicon(lexicon, n_pages: int):
+    """The module functions' lexicon keyword (word lists allowed per page) -> what Engine.ocr_pages takes."""
+    lex = _lexicon_arg(lexicon, n_pages, strict=False)
+    return lex[0] if lex is not None and len(lex) == 1 and lex[0] is not None else lex
 
 
 def decode_ids(ids: np.ndarray) -> list[str]:
@@ -254,7 +319,8 @@ class Engine:
     __del__ = close
 
     def ocr_pages(self, images: list, score_override: list | None = None, detect_only: bool = False,
-                  scores: bool = False, *, allowlist=None, blocklist=None, rotation_info=None) -> list[list[dict]]:
+                  scores: bool = False, *, allowlist=None, blocklist=None, rotation_info=None,
+                  lexicon=None) -> list[list[dict]]:
         """images: uint8 [H,W,3] numpy arrays (host) or torch CUDA tensors (already on the device).
         score_override: optional per-page float32 [h32/2, w32/2, 2] maps (numpy or CUDA tensors, or
         None entries) that replace CRAFT's output after CRAFT has run (benchmark / parity tests).
@@ -264,7 +330,9 @@ class Engine:
         allowlist and not in blocklist.  Each is None, a str for every page, or a list with one str or None per page.
         rotation_info: an iterable of angles from {90, 180, 270}: each word is also read turned
         that many degrees counter-clockwise and the candidate with the highest word confidence wins; every item then
-        carries "angle" (0, 90, 180 or 270; -1 when not recognised).  An empty iterable reads every word upright."""
+        carries "angle" (0, 90, 180 or 270; -1 when not recognised).  An empty iterable reads every word upright.
+        lexicon: every recognised word is one of a word list (INTEGRATION.md section 9): a Lexicon or an iterable of
+        str for every page, or a list with one Lexicon or None per page (None: the page decodes as without lexicon)."""
         n = len(images)
         on_dev = n > 0 and not isinstance(images[0], np.ndarray)
         if on_dev:
@@ -292,8 +360,15 @@ class Engine:
         res = C.POINTER(_native.tt_result)()
         filters = _filters(allowlist, blocklist, n)
         rot = None if rotation_info is None else _rotations(rotation_info)
-        check(lib().tt_ocr_pages_oriented(self._h, arr, n, C.byref(opt), filters or None, len(filters) if filters else 0,
-                                          rot, len(rot) if rot is not None else 0, C.byref(res)), "tt_ocr_pages_oriented")
+        lex = _lexicon_arg(lexicon, n, strict=True)
+        if lex is None:
+            check(lib().tt_ocr_pages_oriented(self._h, arr, n, C.byref(opt), filters or None, len(filters) if filters else 0,
+                                              rot, len(rot) if rot is not None else 0, C.byref(res)), "tt_ocr_pages_oriented")
+        else:
+            handles = (C.c_void_p * len(lex))(*[None if x is None else x._h.value for x in lex])
+            check(lib().tt_ocr_pages_lexicon(self._h, arr, n, C.byref(opt), filters or None, len(filters) if filters else 0,
+                                             rot, len(rot) if rot is not None else 0, handles, len(lex), C.byref(res)),
+                  "tt_ocr_pages_lexicon")
         try:
             out = []
             for p in range(res.contents.n_pages):
@@ -360,6 +435,19 @@ class Engine:
                   "tt_parseq_forward_masked")
         return logits, ids
 
+    def parseq_forward_lexicon(self, crops_u8: np.ndarray, lexicon: Lexicon, forced_tokens: np.ndarray | None = None):
+        """parseq_forward with every crop walking one lexicon's trie (tt_parseq_forward_lexicon)
+        -> (logits float32 [n, 26, 95], ids int32 [n, 26], pmax float32 [n, 26])."""
+        x = np.ascontiguousarray(crops_u8, np.uint8)
+        n = x.shape[0]
+        logits = np.empty((n, 26, 95), np.float32)
+        ids = np.empty((n, 26), np.int32)
+        pmax = np.empty((n, 26), np.float32)
+        ft = None if forced_tokens is None else np.ascontiguousarray(forced_tokens, np.int32)
+        check(lib().tt_parseq_forward_lexicon(self._h, ptr(x), n, ptr(ft), lexicon._h, ptr(logits), ptr(ids), ptr(pmax)),
+              "tt_parseq_forward_lexicon")
+        return logits, ids, pmax
+
 
 def _class_masks(class_masks, n: int) -> np.ndarray:
     m = np.ascontiguousarray(class_masks, np.uint32)
@@ -405,38 +493,44 @@ def _engine_for(weights_dir: str) -> Engine:
 
 
 def image_to_data(image: np.ndarray, weights_dir: str, outputs_dir: str, *, allowlist: str | None = None,
-                  blocklist: str | None = None, rotation_info=None) -> list[dict]:
+                  blocklist: str | None = None, rotation_info=None, lexicon=None) -> list[dict]:
     """Same call as the reference's ``pytuatara.image_to_data`` (bindings/python.cpp:43-57):
     uint8 [H, W, 3] in, list of ``dict(text=str, bbox=[4 floats])`` out.  Empty directory
     strings print to stderr and return [] like tuatara.cpp:315-323.  allowlist / blocklist: recognition only produces
     characters in allowlist and not in blocklist (INTEGRATION.md section 7).  rotation_info: angles from {90, 180, 270}
-    at which each word is also read; items then carry "angle" (INTEGRATION.md section 8)."""
+    at which each word is also read; items then carry "angle" (INTEGRATION.md section 8).  lexicon: a Lexicon or an
+    iterable of str; every recognised word is one of its words (INTEGRATION.md section 9)."""
     return _one_page(image, weights_dir, outputs_dir, allowlist=allowlist, blocklist=blocklist,
-                     rotation_info=rotation_info)
+                     rotation_info=rotation_info, lexicon=lexicon)
 
 
 def images_to_data(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".", *, allowlist=None,
-                   blocklist=None, rotation_info=None) -> list[list[dict]]:
+                   blocklist=None, rotation_info=None, lexicon=None) -> list[list[dict]]:
     """Additive batch API: one call, many pages (sharded over the engine's GPUs).  allowlist / blocklist: None, a str
-    for every page, or a list with one str or None per page."""
-    return _engine_for(weights_dir).ocr_pages(list(images), allowlist=allowlist, blocklist=blocklist,
-                                              rotation_info=rotation_info)
+    for every page, or a list with one str or None per page.  lexicon: a Lexicon or an iterable of str for every page,
+    or a list with one entry per page, each None, a Lexicon or an iterable of str."""
+    images = list(images)
+    return _engine_for(weights_dir).ocr_pages(images, allowlist=allowlist, blocklist=blocklist,
+                                              rotation_info=rotation_info,
+                                              lexicon=_engine_lexicon(lexicon, len(images)))
 
 
 def image_to_data_scored(image: np.ndarray, weights_dir: str, outputs_dir: str, *, allowlist: str | None = None,
-                         blocklist: str | None = None, rotation_info=None) -> list[dict]:
+                         blocklist: str | None = None, rotation_info=None, lexicon=None) -> list[dict]:
     """image_to_data whose items also carry ``conf`` (word confidence 0..1), ``det_score`` (the detection score of the
     box) and ``char_conf`` (one probability per character of ``text``).  Same inputs, errors and soft failures;
     ``text`` and ``bbox`` are what image_to_data returns."""
     return _one_page(image, weights_dir, outputs_dir, scores=True, allowlist=allowlist, blocklist=blocklist,
-                     rotation_info=rotation_info)
+                     rotation_info=rotation_info, lexicon=lexicon)
 
 
 def images_to_data_scored(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".", *, allowlist=None,
-                          blocklist=None, rotation_info=None) -> list[list[dict]]:
+                          blocklist=None, rotation_info=None, lexicon=None) -> list[list[dict]]:
     """Batch variant of image_to_data_scored."""
-    return _engine_for(weights_dir).ocr_pages(list(images), scores=True, allowlist=allowlist, blocklist=blocklist,
-                                              rotation_info=rotation_info)
+    images = list(images)
+    return _engine_for(weights_dir).ocr_pages(images, scores=True, allowlist=allowlist, blocklist=blocklist,
+                                              rotation_info=rotation_info,
+                                              lexicon=_engine_lexicon(lexicon, len(images)))
 
 
 def _one_page(image: np.ndarray, weights_dir: str, outputs_dir: str, **kw) -> list[dict]:
@@ -452,4 +546,5 @@ def _one_page(image: np.ndarray, weights_dir: str, outputs_dir: str, **kw) -> li
         return []
     if image.ndim != 3:
         raise RuntimeError("Input array should have 3 dimensions")
+    kw["lexicon"] = _engine_lexicon(kw.get("lexicon"), 1)
     return _engine_for(weights_dir).ocr_pages([image], **kw)[0]

@@ -70,6 +70,11 @@ SIGNATURES = {
                                    C.POINTER(C.POINTER(tt_result))]),
     "tt_ocr_pages_oriented": (_I, [_P, C.POINTER(tt_image), _I, C.POINTER(tt_ocr_options), C.POINTER(tt_char_filter), _I,
                                    _P, _I, C.POINTER(C.POINTER(tt_result))]),
+    "tt_lexicon_create": (_I, [C.POINTER(C.c_char_p), _I, C.POINTER(_P)]),
+    "tt_lexicon_destroy": (None, [_P]),
+    "tt_lexicon_info": (_I, [_P, _PI, _PI]),
+    "tt_ocr_pages_lexicon": (_I, [_P, C.POINTER(tt_image), _I, C.POINTER(tt_ocr_options), C.POINTER(tt_char_filter), _I,
+                                  _P, _I, C.POINTER(_P), _I, C.POINTER(C.POINTER(tt_result))]),
     "tt_item_angle": (_I, [C.POINTER(tt_result), _I, _I, _PI]),
     "tt_item_scores": (_I, [C.POINTER(tt_result), _I, _I, _PF, _PF, C.POINTER(_PF), _PI]),
     "tt_launch_count": (C.c_ulonglong, []),
@@ -93,6 +98,7 @@ SIGNATURES = {
     "tt_parseq_forward": (_I, [_P, _P, _I, _P, _P, _P]),
     "tt_parseq_forward_scores": (_I, [_P, _P, _I, _P, _P]),
     "tt_parseq_forward_masked": (_I, [_P, _P, _I, _P, _P, _P, _P, _P]),
+    "tt_parseq_forward_lexicon": (_I, [_P, _P, _I, _P, _P, _P, _P, _P]),
     "tt_decode": (_I, [_P, _I, _I, _P, _I]),
     "tt_decode_scores": (_I, [_P, _P, _I, _I, _P, _I, _P, _P]),
     "tt_tokenizer_table": (_I, [C.c_char_p, _PI, _PI, _PI]),
@@ -113,6 +119,7 @@ SIGNATURES = {
     "tt_dec_self_attn_dev": (_I, [_I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _I, _I, _P, _P]),
     "tt_dec_cross_attn_dev": (_I, [_I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P]),
     "tt_orient_select_dev": (_I, [_P, _P, _I, _P, _I, _P, _P, _P, _P]),
+    "tt_lexicon_walk_dev": (_I, [_P, _P, _I, _P, _P, _P]),
     "tt_postprocess_dev": (_I, [_P, _P, _I, _I, _I, _PI, _P]),
 }
 

@@ -81,6 +81,51 @@ static FilterArgs filter_args(const py::object& allow, const py::object& block, 
   return fa;
 }
 
+// lexicon keyword -> tt_lexicon handles (empty: no lexicon).  A tuatara_b200.Lexicon (its handle is borrowed) or an
+// iterable of str is one lexicon for every page; for the batch functions a list with one entry per page, each None or one
+// of those, is a lexicon per page (a list of str alone is always one word list).
+struct LexiconArgs {
+  std::vector<std::unique_ptr<tuatara::Lexicon>> keep;   // lexicons built here from word lists
+  std::vector<const tt_lexicon*> handles;
+};
+
+static bool is_word_list(const py::handle& v) {
+  if (py::isinstance<py::str>(v) || py::isinstance<py::bytes>(v) || !py::isinstance<py::iterable>(v)) return false;
+  for (const py::handle& w : v)
+    if (!py::isinstance<py::str>(w)) return false;
+  return true;
+}
+
+static const tt_lexicon* lexicon_handle(const py::handle& v, LexiconArgs* la) {
+  if (v.is_none()) return nullptr;
+  if (py::hasattr(v, "_h") && py::hasattr(v, "info")) {   // tuatara_b200.Lexicon
+    const py::object h = v.attr("_h").attr("value");
+    if (h.is_none()) throw py::value_error("lexicon: the Lexicon was closed");
+    return reinterpret_cast<const tt_lexicon*>(h.cast<uintptr_t>());
+  }
+  if (!is_word_list(v)) throw py::type_error("lexicon: expected a Lexicon, an iterable of str, or None");
+  std::vector<std::string> words;
+  for (const py::handle& w : v) words.push_back(w.cast<std::string>());
+  la->keep.emplace_back(new tuatara::Lexicon(words));
+  if (!la->keep.back()->ok()) throw py::value_error(la->keep.back()->error());
+  return la->keep.back()->get();
+}
+
+static LexiconArgs lexicon_args(const py::object& lexicon, size_t n_pages, bool batch) {
+  LexiconArgs la;
+  if (lexicon.is_none()) return la;
+  if (batch && py::isinstance<py::list>(lexicon) && !is_word_list(lexicon)) {
+    if (py::len(lexicon) != n_pages)
+      throw py::value_error("lexicon: expected one entry per page (" + std::to_string(n_pages) + "), got " +
+                            std::to_string(py::len(lexicon)));
+    for (const py::handle& v : lexicon) la.handles.push_back(lexicon_handle(v, &la));
+    return la;
+  }
+  if (py::isinstance<py::str>(lexicon)) throw py::type_error("lexicon: expected a Lexicon or an iterable of str, not a str");
+  la.handles.push_back(lexicon_handle(lexicon, &la));
+  return la;
+}
+
 // One item as a dict: text and bbox; conf (None for a word that was not recognised, ScoredItem::confidence == -1),
 // det_score and char_conf when scored; angle when rotation_info was given (0 for every word when it is empty).
 static py::dict item_to_dict(const tuatara::ScoredItem& item, bool scored, bool angle) {  // python.cpp:36-41
@@ -99,13 +144,14 @@ static py::dict item_to_dict(const tuatara::ScoredItem& item, bool scored, bool 
 // The four functions' one path -> a list of pages of item dicts.  batch: allowlist / blocklist may hold one entry per page.
 static py::list ocr_pages(const std::vector<tuatara::ImageView>& views, bool batch, const std::string& weights_dir,
                           const std::string& output_dir, const py::object& allowlist, const py::object& blocklist,
-                          const py::object& rotation_info, bool scored) {
+                          const py::object& rotation_info, const py::object& lexicon, bool scored) {
   const FilterArgs fa = filter_args(allowlist, blocklist, views.size(), batch);
   const RotationArgs ra = rotation_args(rotation_info);
+  const LexiconArgs la = lexicon_args(lexicon, views.size(), batch);
   std::vector<std::vector<tuatara::ScoredItem>> pages;
   {
     py::gil_scoped_release release;
-    pages = tuatara::detail::ocr_pages(views, weights_dir, output_dir, scored, fa.filters, ra.angles);
+    pages = tuatara::detail::ocr_pages(views, weights_dir, output_dir, scored, fa.filters, ra.angles, la.handles);
   }
   py::list result;
   for (const auto& page : pages) {
@@ -119,35 +165,40 @@ static py::list ocr_pages(const std::vector<tuatara::ImageView>& views, bool bat
 // image_to_data / image_to_data_scored: page 0, or [] after a soft failure
 template <bool kScored>
 static py::list image_wrapper(Image image_data, std::string weights_dir, std::string output_dir, py::object allowlist,
-                              py::object blocklist, py::object rotation_info) {
+                              py::object blocklist, py::object rotation_info, py::object lexicon) {
   py::list pages = ocr_pages({buffer_to_view(image_data)}, false, weights_dir, output_dir, allowlist, blocklist,
-                             rotation_info, kScored);
+                             rotation_info, lexicon, kScored);
   return pages.empty() ? py::list() : py::list(pages[0]);
 }
 
 // images_to_data / images_to_data_scored
 template <bool kScored>
 static py::list images_wrapper(std::vector<Image> images, std::string weights_dir, std::string output_dir,
-                               py::object allowlist, py::object blocklist, py::object rotation_info) {
+                               py::object allowlist, py::object blocklist, py::object rotation_info, py::object lexicon) {
   std::vector<tuatara::ImageView> views;
   for (auto& a : images) views.push_back(buffer_to_view(a));
-  return ocr_pages(views, true, weights_dir, output_dir, allowlist, blocklist, rotation_info, kScored);
+  return ocr_pages(views, true, weights_dir, output_dir, allowlist, blocklist, rotation_info, lexicon, kScored);
 }
 
 PYBIND11_MODULE(pytuatara, m) {
   m.doc() = "Tuatara ocr";
   // allowlist / blocklist (keyword only): recognition only produces characters in allowlist and not in blocklist.
   // rotation_info (keyword only): angles from {90, 180, 270} at which each word is also read; items then carry "angle".
+  // lexicon (keyword only): every recognised word is one of a word list (a tuatara_b200.Lexicon or an iterable of str).
   m.def("image_to_data", &image_wrapper<false>, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"), py::kw_only(),
         py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
+        py::arg("lexicon") = py::none(),
         "Extract text and bounding boxes from an image");
   m.def("images_to_data", &images_wrapper<false>, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"), py::kw_only(),
         py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
+        py::arg("lexicon") = py::none(),
         "Batch variant: list of images -> list of per-page results");
   m.def("image_to_data_scored", &image_wrapper<true>, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"),
         py::kw_only(), py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
+        py::arg("lexicon") = py::none(),
         "image_to_data whose items also carry conf (word confidence 0..1, None when not recognised), det_score and char_conf");
   m.def("images_to_data_scored", &images_wrapper<true>, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"),
         py::kw_only(), py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
+        py::arg("lexicon") = py::none(),
         "Batch variant of image_to_data_scored");
 }

@@ -11,6 +11,7 @@
 #include "detect.h"
 #include "enc_mlp.cuh"
 #include "engine.h"
+#include "lexicon.h"
 #include "gemm_tc.cuh"
 #include "geometry.h"
 #include "nn_kernels.cuh"
@@ -484,6 +485,32 @@ int tt_orient_select_dev(const int32_t* ids, const float* pmax, int n_words, con
     for (int r = 0; r < n_candidates; ++r) set.angle[r] = angles[r];
     return orient_select(ids, pmax, n_words, TT_MAX_LABEL_LEN, set, ids_out, pmax_out, angle_out,
                          static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : 1;
+  });
+}
+
+int tt_lexicon_walk_dev(const tt_lexicon* lex, const float* logits, int n, int32_t* ids_out, float* pmax_out, void* stream) {
+  return guarded([&]() -> int {
+    if (!lex || !ids_out || n < 0 || (n > 0 && !logits)) { set_error("tt_lexicon_walk_dev: null argument or n < 0"); return 1; }
+    if (n == 0) return 0;
+    LexTableBuilder table;
+    const std::vector<int> roots(n, table.append(lex->trie));
+    const std::vector<uint32_t> words = table.words();
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    DevBuf tab, root, state;
+    TT_CUDA_INT(tab.alloc(sizeof(uint32_t) * words.size()));
+    TT_CUDA_INT(root.alloc(sizeof(int) * n));
+    TT_CUDA_INT(state.alloc(sizeof(int) * n));
+    TT_CUDA_INT(cudaMemcpyAsync(tab.p, words.data(), sizeof(uint32_t) * words.size(), cudaMemcpyHostToDevice, s));
+    TT_CUDA_INT(cudaMemcpyAsync(root.p, roots.data(), sizeof(int) * n, cudaMemcpyHostToDevice, s));
+    LexDev lx;
+    lx.allow = tab.as<const uint4>();
+    lx.first = tab.as<const int>() + 4 * static_cast<size_t>(table.n_states());
+    lx.next = lx.first + table.n_states();
+    lx.root = root.as<int>();
+    lx.state = state.as<int>();
+    TT_TRY_INT(lexicon_walk(logits, n, TT_MAX_LABEL_LEN, TT_NUM_CLASSES, TT_NUM_CLASSES, lx, ids_out, pmax_out, s));
+    TT_CUDA_INT(cudaStreamSynchronize(s));   // the table and the roots are freed on return
+    return 0;
   });
 }
 

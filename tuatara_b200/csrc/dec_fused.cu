@@ -21,6 +21,7 @@
 #include "common.h"
 #include "epi_math.cuh"
 #include "gemm_tc.cuh"
+#include "lexicon.cuh"
 #include "ptx.cuh"
 
 namespace tt {
@@ -50,7 +51,13 @@ struct DenseParams {
   const int* active;
   const int* n_act;
   unsigned long long* dbg;               // TT_DEC_DEBUG=1 (development): role cycle counters of CTA 0
-  const uint32_t* mask;                  // B, MASK only: [n][4] class masks, indexed by crop like tokens
+  const uint32_t* mask;                  // B, MASK_CROP only: [n][4] class masks, indexed by crop like tokens
+  // B, MASK_STATE only (lexicon.h): the automaton table and the crops' states, indexed by crop like tokens
+  const int* st_in;                      // state of each crop before this step (the roots at step 0)
+  int* st_out;                           // its state after this step's token
+  const uint4* lx_allow;
+  const int* lx_first;
+  const int* lx_next;
 };
 
 struct alignas(16) Ctl {
@@ -81,8 +88,10 @@ struct Cfg {
   static_assert(kSmem <= 227 * 1024, "shared memory budget");
 };
 
-// MASK (MODE_B only): the greedy token is the argmax over the classes allowed by the crop's class mask.
-template <int D, int MLP, int MODE, bool MASK>
+// MM (MODE_B only, lexicon.cuh): the greedy token is the argmax over the classes allowed by the crop's class mask
+// (MASK_CROP) or by its automaton state (MASK_STATE: an all-NaN row takes the lowest allowed class, and the state
+// advances by the chosen class).
+template <int D, int MLP, int MODE, int MM>
 __global__ void __launch_bounds__(kThreads, 1) k_dec_dense(const __grid_constant__ DenseParams p) {
   using C = Cfg<D, MLP, MODE>;
   constexpr int KB = C::KB, kStages = C::kStages;
@@ -391,26 +400,40 @@ __global__ void __launch_bounds__(kThreads, 1) k_dec_dense(const __grid_constant
       }
       rows_done();
       // ---- head: logits row + greedy token (the halves' maxima meet in smem; the lower half holds the lower classes)
+      // MASK_STATE: the crop's state and its allow row are loaded before the accumulator wait, so that the two dependent
+      // loads overlap it; half 0 also fetches where the state's successors start.
+      int st = 0, st_first = 0;
+      uint4 st_mw = make_uint4(~0u, ~0u, ~0u, ~0u);
+      if constexpr (MM == MASK_STATE) {
+        if (valid) {
+          const long long crop = p.active ? p.active[m] : m;
+          st = p.st_in[crop];
+          st_mw = p.lx_allow[st];
+          if (half == 0) st_first = p.lx_first[st];
+        }
+      }
       wait_md();
       {
         const long long crop = (valid && p.active) ? p.active[m] : m;
         float* lrow = p.logits + (crop * p.L + p.step) * p.ncp;
-        // MASK: the crop's class mask, one 16-byte load (rows past the live count compete unmasked: never stored)
+        // MASK_CROP: the crop's class mask, one 16-byte load (rows past the live count compete unmasked: never stored)
         uint4 mw = make_uint4(~0u, ~0u, ~0u, ~0u);
-        if constexpr (MASK) {
+        if constexpr (MM == MASK_CROP) {
           if (valid) mw = *reinterpret_cast<const uint4*>(p.mask + crop * 4);
         }
+        if constexpr (MM == MASK_STATE) mw = st_mw;
+        const uint32_t mws[4] = {mw.x, mw.y, mw.z, mw.w};
         float best = -INFINITY;
-        int bi = 0;
+        int bi = MM == MASK_STATE ? lowest_class(mws) : 0;
         const int nb = p.ncp / 32, hb0 = half ? (nb + 1) / 2 : 0, hb1 = half ? nb : (nb + 1) / 2;
         for_blocks(tl + D, hb0, hb1, [&](int blk, uint32_t (&raw)[32]) {
           float l[32];
           lds_f32x32(vec_s + (6 * D + MLP + blk * 32) * 4, l);
-          const uint32_t bits = MASK ? (blk == 0 ? mw.x : blk == 1 ? mw.y : blk == 2 ? mw.z : mw.w) : ~0u;
+          const uint32_t bits = MM != MASK_NONE ? (blk == 0 ? mw.x : blk == 1 ? mw.y : blk == 2 ? mw.z : mw.w) : ~0u;
 #pragma unroll
           for (int j = 0; j < 32; ++j) {
             l[j] += __uint_as_float(raw[j]);
-            if (blk * 32 + j < p.n_cls && (!MASK || ((bits >> j) & 1u)) && l[j] > best) { best = l[j]; bi = blk * 32 + j; }   // first max wins (at::max on CPU)
+            if (blk * 32 + j < p.n_cls && (MM == MASK_NONE || ((bits >> j) & 1u)) && l[j] > best) { best = l[j]; bi = blk * 32 + j; }   // first max wins (at::max on CPU)
           }
           if (valid) {
 #pragma unroll
@@ -425,6 +448,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_dec_dense(const __grid_constant
           if (ob > best) { best = ob; bi = __float_as_int(xch[r * 2 + 1]); }
           if (valid && p.step + 1 < p.L)
             p.tokens[crop * p.L + p.step + 1] = p.forced ? p.forced[crop * (p.L - 1) + p.step] : bi;
+          if constexpr (MM == MASK_STATE) {
+            if (valid) p.st_out[crop] = p.lx_next[st_first + classes_below(mws, bi)];
+          }
         }
       }
     }
@@ -462,10 +488,10 @@ int dense_priority() {
   return prio;
 }
 
-template <int D, int MLP, int MODE, bool MASK = false>
+template <int D, int MLP, int MODE, int MM = MASK_NONE>
 cudaError_t launch_dense(const DenseParams& p, cudaStream_t s) {
   using C = Cfg<D, MLP, MODE>;
-  TT_CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(k_dec_dense<D, MLP, MODE, MASK>), C::kSmem));
+  TT_CUDA_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(k_dec_dense<D, MLP, MODE, MM>), C::kSmem));
   // Highest launch priority: a CTA needs a whole SM (216 KB smem, 512 TMEM columns).  Next to the other half-batch's
   // cross-attention grid (thousands of small blocks, launched earlier) it would otherwise wait for that grid to drain.
   cudaLaunchConfig_t cfg{};
@@ -486,7 +512,7 @@ cudaError_t launch_dense(const DenseParams& p, cudaStream_t s) {
     cudaMemsetAsync(dbg_buf, 0, 8 * sizeof(unsigned long long), s);
     pp.dbg = dbg_buf;
   }
-  TT_CUDA_TRY(cudaLaunchKernelEx(&cfg, k_dec_dense<D, MLP, MODE, MASK>, pp));
+  TT_CUDA_TRY(cudaLaunchKernelEx(&cfg, k_dec_dense<D, MLP, MODE, MM>, pp));
   TT_LAUNCH_CHECK();
   if (dbg_env && p.step == 13) {
     unsigned long long h[8];
@@ -571,7 +597,7 @@ cudaError_t dec_dense_a2(const DecDenseWeights& w, const __nv_bfloat16* ab, int 
 
 cudaError_t dec_dense_b(const DecDenseWeights& w, const __nv_bfloat16* ab2, int n, int step, const float* t_scratch,
                         float* logits, int* tokens, const int* forced, cudaStream_t s, const int* active, const int* n_act,
-                        const uint32_t* mask) {
+                        const uint32_t* mask, const LexDev* lex, bool first_step) {
   if (n <= 0) return cudaSuccess;
   if (!w.ready) { set_error("dec_dense_b: weights not initialised for this width"); return cudaErrorInvalidValue; }
   DenseParams p{};
@@ -582,9 +608,16 @@ cudaError_t dec_dense_b(const DecDenseWeights& w, const __nv_bfloat16* ab2, int 
   p.logits = logits; p.tokens = tokens; p.forced = forced; p.mask = mask;
   p.n = n; p.L = w.L; p.step = step; p.n_cls = w.n_cls; p.ncp = w.ncp;
   p.active = active; p.n_act = n_act;
+  if (lex) {
+    p.st_in = first_step ? lex->root : lex->state;
+    p.st_out = lex->state;
+    p.lx_allow = lex->allow; p.lx_first = lex->first; p.lx_next = lex->next;
+    if (w.D == 384) return launch_dense<384, 1536, MODE_B, MASK_STATE>(p, s);
+    return launch_dense<192, 768, MODE_B, MASK_STATE>(p, s);
+  }
   if (mask) {
-    if (w.D == 384) return launch_dense<384, 1536, MODE_B, true>(p, s);
-    return launch_dense<192, 768, MODE_B, true>(p, s);
+    if (w.D == 384) return launch_dense<384, 1536, MODE_B, MASK_CROP>(p, s);
+    return launch_dense<192, 768, MODE_B, MASK_CROP>(p, s);
   }
   if (w.D == 384) return launch_dense<384, 1536, MODE_B>(p, s);
   return launch_dense<192, 768, MODE_B>(p, s);

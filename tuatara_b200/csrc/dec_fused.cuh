@@ -18,6 +18,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "nn_kernels.cuh"
+
 namespace tt {
 
 struct DecDenseWeights {
@@ -56,8 +58,12 @@ cudaError_t dec_dense_a2(const DecDenseWeights& w, const __nv_bfloat16* ab, int 
 // token: tokens[crop][step + 1] = forced ? forced[crop][step] : argmax over the first n_cls logits (first max wins).
 // mask (nullable): class masks [n][4] uint32 (16-byte aligned, indexed by crop like tokens): the argmax runs over the
 // classes whose bit (c & 31 of word c >> 5) is set; the logits are written unmasked.
+// lex (nullable; mask is then unused): the mask of crop c is the allow row of its state (lex->root[c] at first_step,
+// else lex->state[c], indexed by crop like tokens); an all-NaN row takes the lowest allowed class and lex->state[c]
+// becomes the chosen class's successor.
 cudaError_t dec_dense_b(const DecDenseWeights& w, const __nv_bfloat16* ab2, int n, int step, const float* t_scratch,
                         float* logits, int* tokens, const int* forced, cudaStream_t s, const int* active = nullptr,
-                        const int* n_act = nullptr, const uint32_t* mask = nullptr);
+                        const int* n_act = nullptr, const uint32_t* mask = nullptr, const LexDev* lex = nullptr,
+                        bool first_step = false);
 
 }  // namespace tt

@@ -14,6 +14,7 @@
 
 #include "common.h"
 #include "gemm_tc.cuh"
+#include "lexicon.h"
 #include "nn_kernels.cuh"
 #include "orient.cuh"
 #include "resize.cuh"
@@ -116,14 +117,40 @@ struct Unit {
 
 struct CropOwner { int page, box; };
 
-using ClassMask = std::array<uint32_t, 4>;   // tt_char_filter_mask
-
 // What a request asks for besides its pages, checked by make_request; every tt_ocr_pages* entry point builds one.
 struct Request {
   tt_ocr_options opt{0, 0, nullptr, 0, 0};   // zeroed when the caller passes none
   std::vector<ClassMask> masks;              // one class mask per page; empty when no page has a filter
   OrientSet orient{1, {0, 0, 0, 0}};         // the rotation candidates; n == 1 (angle 0 alone) without
+  // lexicon requests only (both empty otherwise; masks is then empty too, the filters being folded into the automata):
+  std::vector<int> roots;                    // the root state of every page's automaton
+  std::vector<uint32_t> lex_table;           // the request's automata, LexTableBuilder::words()
+  int lex_states = 0;                        //   its number of states
 };
+
+// The request's automaton table in the slot's lex_buf, uploaded at most once per slot per request; -> its device view.
+int upload_lex_table(DeviceCtx& d, const std::vector<uint32_t>& table, int n_states, LexDev* lx) {
+  const size_t bytes = sizeof(uint32_t) * table.size();
+  if (bytes > d.lex_cap) {
+    if (d.lex_buf) {
+      E_TRY(stream_sync(d.stream));
+      cudaFree(d.lex_buf);
+      d.lex_buf = nullptr;
+      d.lex_cap = 0;
+    }
+    E_CUDA(cudaMalloc(&d.lex_buf, bytes));
+    d.lex_cap = bytes;
+  }
+  stage_begin(d.stream);
+  E_CUDA(cudaMemcpyAsync(d.lex_buf, table.data(), bytes, cudaMemcpyHostToDevice, d.stream));
+  stage_end(d.stream, "lexicon_table", 0.0, static_cast<double>(bytes));
+  g_h2d_bytes += bytes;
+  const uint32_t* base = static_cast<const uint32_t*>(d.lex_buf);   // allow [S][4] | first [S] | next [E]
+  lx->allow = reinterpret_cast<const uint4*>(base);
+  lx->first = reinterpret_cast<const int*>(base + 4 * static_cast<size_t>(n_states));
+  lx->next = lx->first + n_states;
+  return 0;
+}
 
 // crops waiting for recognition in one slot (device patch rows live in DeviceCtx::patch_buf)
 struct Pending {
@@ -287,9 +314,18 @@ int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const
 // position's largest softmax probability, copied back next to the ids and decoded into conf / char_conf.  With
 // rotation candidates (R > 1) it always writes them, and orient_select leaves one candidate per word on the device, so
 // the copy back is the same ids (and pmax with scores) per word plus its 4-byte angle.  With filters (req.masks) each
-// crop decodes under its page's class mask, uploaded per pass as [nc][4] words.
-int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, const Request& req) {
+// crop decodes under its page's class mask, uploaded per pass as [nc][4] words.  With lexicons (req.roots) each crop
+// walks its page's automaton instead: the table goes to the slot once per request (*lex_ready), the crops' roots with
+// each pass as [nc] words.
+int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, const Request& req, bool* lex_ready) {
   const int n = static_cast<int>(pend->owner.size());
+  const bool lexed = !req.roots.empty();
+  LexDev lx{};
+  if (lexed && n > 0 && !*lex_ready) {
+    if (upload_lex_table(d, req.lex_table, req.lex_states, &d.lex_view)) return 1;
+    *lex_ready = true;
+  }
+  if (lexed) lx = d.lex_view;
   const int L = d.w->pd.L, R = req.orient.n;
   const bool scores = req.opt.with_scores != 0;
   const int words_per_pass = kMaxCropsPerPass / R;
@@ -300,7 +336,9 @@ int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, const 
     const size_t angle_bytes = R > 1 ? sizeof(int) * static_cast<size_t>(nw) : 0;
     const size_t pmax_bytes = scores || R > 1 ? sizeof(float) * static_cast<size_t>(nc) * L : 0;
     const size_t mask_bytes = req.masks.empty() ? 0 : sizeof(ClassMask) * nc;
-    const size_t need = d.parseq_bytes(nc) + (4u << 20) + pmax_bytes + (R > 1 ? 2 * bytes + angle_bytes : 0) + mask_bytes;
+    const size_t root_bytes = lexed ? sizeof(int) * static_cast<size_t>(nc) : 0;   // and as many for the walk state
+    const size_t need = d.parseq_bytes(nc) + (4u << 20) + pmax_bytes + (R > 1 ? 2 * bytes + angle_bytes : 0) + mask_bytes +
+                        2 * root_bytes;
     if (need > d.arena.capacity()) E_TRY(stream_sync(d.stream));
     E_TRY(d.arena.reserve(need));
     d.arena.reset();
@@ -315,8 +353,8 @@ int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, const 
       win_angle = d.arena.get<int>(nw);
       if (!win_ids || !win_p || !win_angle) { set_error("arena exhausted (orientation)"); return 1; }
     }
-    // pinned staging: ids | angle | pmax on the way back, the class masks on the way in
-    E_TRY(d.ensure_pinned(std::max((scores ? 2 * bytes : bytes) + angle_bytes, mask_bytes)));
+    // pinned staging: ids | angle | pmax on the way back, the class masks or the roots on the way in
+    E_TRY(d.ensure_pinned(std::max((scores ? 2 * bytes : bytes) + angle_bytes, std::max(mask_bytes, root_bytes))));
     uint32_t* mask = nullptr;
     if (!req.masks.empty()) {
       mask = d.arena.get<uint32_t>(4 * static_cast<size_t>(nc));
@@ -326,9 +364,20 @@ int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, const 
       E_CUDA(cudaMemcpyAsync(mask, host_mask, mask_bytes, cudaMemcpyHostToDevice, d.stream));
       g_h2d_bytes += mask_bytes;
     }
+    if (lexed) {
+      int* roots = d.arena.get<int>(nc);
+      lx.state = d.arena.get<int>(nc);
+      if (!roots || !lx.state) { set_error("arena exhausted (lexicon roots)"); return 1; }
+      int* host_roots = reinterpret_cast<int*>(d.pinned);   // the ids' D2H below is ordered after this copy
+      for (int c = 0; c < nc; ++c) host_roots[c] = req.roots[pend->owner[w0 + c / R].page];
+      E_CUDA(cudaMemcpyAsync(roots, host_roots, root_bytes, cudaMemcpyHostToDevice, d.stream));
+      g_h2d_bytes += root_bytes;
+      lx.root = roots;
+    }
     float* logits = nullptr;
     int* ids = nullptr;
-    E_TRY(d.parseq_forward(d.patch_buf + static_cast<size_t>(w0) * R * 128 * 96, nc, nullptr, &logits, &ids, pmax, mask));
+    E_TRY(d.parseq_forward(d.patch_buf + static_cast<size_t>(w0) * R * 128 * 96, nc, nullptr, &logits, &ids, pmax, mask,
+                           lexed ? &lx : nullptr));
     if (R > 1) {
       stage_begin(d.stream);
       E_TRY(orient_select(ids, pmax, nw, L, req.orient, win_ids, scores ? win_p : nullptr, win_angle, d.stream));
@@ -395,22 +444,24 @@ void slot_worker(tt_engine& e, int g, int sidx, int want, const tt_image* pages,
   }
   DeviceCtx& d = *dp;
   std::lock_guard<std::mutex> lock(d.mu, std::adopt_lock);
+  bool lex_ready = false;   // this request's automaton table is in the slot's lex_buf
   if (cudaSetDevice(d.device) != cudaSuccess) { *err = "cudaSetDevice failed"; *rc = 1; return; }
   const tt_config& cfg = e.cfg;
   const int max_b = cfg.max_batch_pages > 0 ? cfg.max_batch_pages : 32;
   Pending pend;
   for (int ui = q->pop(g); ui >= 0; ui = q->pop(g)) {
     if (detect_unit(d, cfg, pages, q->units[ui], req, results, &pend)) { *err = last_error(); *rc = 1; return; }
-    if (pend.pages >= max_b && recognise(d, results, &pend, req)) { *err = last_error(); *rc = 1; return; }
+    if (pend.pages >= max_b && recognise(d, results, &pend, req, &lex_ready)) { *err = last_error(); *rc = 1; return; }
   }
-  if (recognise(d, results, &pend, req)) { *err = last_error(); *rc = 1; return; }
+  if (recognise(d, results, &pend, req, &lex_ready)) { *err = last_error(); *rc = 1; return; }
 }
 
 // The argument checks of the tt_ocr_pages* entry points (fn: the one called, named in the messages), made before any
-// device work: the rotation candidates, then the filters, turned into one class mask per page.  ocr_pages checks the
-// engine and the pages.
+// device work: the rotation candidates, then the filters, turned into one class mask per page, then the lexicons, turned
+// into one automaton per page with the page's filter folded in.  ocr_pages checks the engine and the pages.
 int make_request(const char* fn, const tt_ocr_options* opt, const tt_char_filter* filters, int n_filters,
-                 const int* rotation_info, int n_rotations, int n_pages, Request* req) {
+                 const int* rotation_info, int n_rotations, const tt_lexicon* const* lexicons, int n_lexicons, int n_pages,
+                 Request* req) {
   try {
     if (opt) req->opt = *opt;
     if (n_rotations < 0 || (n_rotations > 0 && !rotation_info)) {
@@ -430,18 +481,60 @@ int make_request(const char* fn, const tt_ocr_options* opt, const tt_char_filter
     req->orient.n = 0;
     for (int q = 0; q < 4; ++q)
       if (seen[q]) req->orient.angle[req->orient.n++] = 90 * q;
-    if (n_filters == 0) return 0;
-    if (!filters) { set_error(std::string(fn) + ": filters is NULL but n_filters is " + std::to_string(n_filters)); return 1; }
-    if (n_filters != 1 && n_filters != n_pages) {
-      set_error(std::string(fn) + ": n_filters must be 0, 1 or n_pages (" + std::to_string(n_pages) + "), got " +
-                std::to_string(n_filters));
+    if (n_filters != 0) {
+      if (!filters) { set_error(std::string(fn) + ": filters is NULL but n_filters is " + std::to_string(n_filters)); return 1; }
+      if (n_filters != 1 && n_filters != n_pages) {
+        set_error(std::string(fn) + ": n_filters must be 0, 1 or n_pages (" + std::to_string(n_pages) + "), got " +
+                  std::to_string(n_filters));
+        return 1;
+      }
+      req->masks.resize(std::max(n_pages, 0));
+      for (int i = 0; i < n_pages; ++i) {
+        const tt_char_filter& f = filters[n_filters == 1 ? 0 : i];
+        char_filter_mask(f.allow, f.block, req->masks[i].data());
+      }
+    }
+    if (n_lexicons == 0) return 0;
+    if (!lexicons) { set_error(std::string(fn) + ": lexicons is NULL but n_lexicons is " + std::to_string(n_lexicons)); return 1; }
+    if (n_lexicons != 1 && n_lexicons != n_pages) {
+      set_error(std::string(fn) + ": n_lexicons must be 0, 1 or n_pages (" + std::to_string(n_pages) + "), got " +
+                std::to_string(n_lexicons));
       return 1;
     }
-    req->masks.resize(std::max(n_pages, 0));
+    // one automaton per distinct (lexicon, class mask) of the request: the lexicon's own trie when the page's filter
+    // allows all its words, else a trie over the words it allows; a one-state automaton for a NULL entry
+    ClassMask all;
+    char_filter_mask(nullptr, nullptr, all.data());
+    LexTableBuilder table;
+    std::map<std::pair<const tt_lexicon*, ClassMask>, int> built;
+    req->roots.resize(std::max(n_pages, 0));
     for (int i = 0; i < n_pages; ++i) {
-      const tt_char_filter& f = filters[n_filters == 1 ? 0 : i];
-      char_filter_mask(f.allow, f.block, req->masks[i].data());
+      const tt_lexicon* lex = lexicons[n_lexicons == 1 ? 0 : i];
+      const ClassMask& m = req->masks.empty() ? all : req->masks[i];
+      const auto key = std::make_pair(lex, m);
+      auto it = built.find(key);
+      if (it == built.end()) {
+        int root;
+        if (!lex) {
+          root = table.append(one_state(m));
+        } else {
+          std::vector<std::string> kept;
+          for (const std::string& w : lex->words)
+            if (word_allowed(w, m)) kept.push_back(w);
+          if (kept.empty()) {
+            set_error(std::string(fn) + ": page " + std::to_string(i) + ": its filter allows none of its lexicon's " +
+                      std::to_string(lex->words.size()) + " words");
+            return 1;
+          }
+          root = table.append(kept.size() == lex->words.size() ? lex->trie : build_trie(kept));
+        }
+        it = built.emplace(key, root).first;
+      }
+      req->roots[i] = it->second;
     }
+    req->lex_table = table.words();
+    req->lex_states = table.n_states();
+    req->masks.clear();
     return 0;
   } catch (const std::exception& ex) {
     set_error(std::string(fn) + ": " + ex.what());
@@ -546,13 +639,14 @@ int tt_ocr_pages(tt_engine* e, const tt_image* pages, int n_pages, tt_result** o
 
 int tt_ocr_pages_ex(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt, tt_result** out) {
   Request req;
-  return make_request("tt_ocr_pages_ex", opt, nullptr, 0, nullptr, 0, n_pages, &req) ? 1 : ocr_pages(e, pages, n_pages, req, out);
+  return make_request("tt_ocr_pages_ex", opt, nullptr, 0, nullptr, 0, nullptr, 0, n_pages, &req)
+             ? 1 : ocr_pages(e, pages, n_pages, req, out);
 }
 
 int tt_ocr_pages_filtered(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
                           const tt_char_filter* filters, int n_filters, tt_result** out) {
   Request req;
-  return make_request("tt_ocr_pages_filtered", opt, filters, n_filters, nullptr, 0, n_pages, &req)
+  return make_request("tt_ocr_pages_filtered", opt, filters, n_filters, nullptr, 0, nullptr, 0, n_pages, &req)
              ? 1 : ocr_pages(e, pages, n_pages, req, out);
 }
 
@@ -560,7 +654,16 @@ int tt_ocr_pages_oriented(tt_engine* e, const tt_image* pages, int n_pages, cons
                           const tt_char_filter* filters, int n_filters, const int* rotation_info, int n_rotations,
                           tt_result** out) {
   Request req;
-  return make_request("tt_ocr_pages_oriented", opt, filters, n_filters, rotation_info, n_rotations, n_pages, &req)
+  return make_request("tt_ocr_pages_oriented", opt, filters, n_filters, rotation_info, n_rotations, nullptr, 0, n_pages, &req)
+             ? 1 : ocr_pages(e, pages, n_pages, req, out);
+}
+
+int tt_ocr_pages_lexicon(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
+                         const tt_char_filter* filters, int n_filters, const int* rotation_info, int n_rotations,
+                         const tt_lexicon* const* lexicons, int n_lexicons, tt_result** out) {
+  Request req;
+  return make_request("tt_ocr_pages_lexicon", opt, filters, n_filters, rotation_info, n_rotations, lexicons, n_lexicons,
+                      n_pages, &req)
              ? 1 : ocr_pages(e, pages, n_pages, req, out);
 }
 
@@ -754,10 +857,11 @@ int tt_craft_tap(tt_engine* e, const char* name, float* out, long long capacity,
 }  // extern "C"
 
 namespace {
-// tt_parseq_forward, tt_parseq_forward_scores and tt_parseq_forward_masked (pmax_out != null: the refinement head also
-// writes the probabilities; class_masks != null: [n][4] per-crop class masks)
+// tt_parseq_forward, tt_parseq_forward_scores, tt_parseq_forward_masked and tt_parseq_forward_lexicon (pmax_out != null:
+// the refinement head also writes the probabilities; class_masks != null: [n][4] per-crop class masks; lex != null: every
+// crop walks the lexicon's trie)
 int parseq_stage(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens, const uint32_t* class_masks,
-                 float* logits_out, int32_t* ids_out, float* pmax_out) {
+                 const tt_lexicon* lex, float* logits_out, int32_t* ids_out, float* pmax_out) {
   try {
     if (!e) { set_error("tt_parseq_forward: null engine"); return 1; }
     if (n <= 0) return 0;
@@ -765,12 +869,26 @@ int parseq_stage(tt_engine* e, const uint8_t* crops, int n, const int32_t* force
     std::lock_guard<std::mutex> lock(d.mu);
     E_CUDA(cudaSetDevice(d.device));
     const int L = d.w->pd.L, NC = d.w->pd.n_cls_pad;
+    LexDev lx{};
+    std::vector<int> roots;
+    if (lex) {
+      LexTableBuilder table;
+      roots.assign(std::min(n, kMaxCropsPerPass), table.append(lex->trie));
+      if (upload_lex_table(d, table.words(), table.n_states(), &lx)) return 1;
+    }
     for (int c0 = 0; c0 < n; c0 += kMaxCropsPerPass) {
       const int nc = std::min(kMaxCropsPerPass, n - c0);
       const size_t crop_bytes = static_cast<size_t>(nc) * 32 * 128 * 3;
       E_TRY(d.arena.reserve(d.parseq_bytes(nc) + crop_bytes + static_cast<size_t>(nc) * (128 * 96 * 2 + 4 * L) + (8u << 20) +
-                            (pmax_out ? sizeof(float) * nc * L : 0) + (class_masks ? 16 * static_cast<size_t>(nc) : 0)));
+                            (pmax_out ? sizeof(float) * nc * L : 0) + (class_masks ? 16 * static_cast<size_t>(nc) : 0) +
+                            (lex ? 8 * static_cast<size_t>(nc) : 0)));
       d.arena.reset();
+      if (lex) {
+        int* root_dev = d.arena.get<int>(nc);
+        lx.state = d.arena.get<int>(nc);
+        E_CUDA(cudaMemcpyAsync(root_dev, roots.data(), sizeof(int) * nc, cudaMemcpyHostToDevice, d.stream));
+        lx.root = root_dev;
+      }
       float* pmax = pmax_out ? d.arena.get<float>(static_cast<size_t>(nc) * L) : nullptr;
       uint32_t* mask = class_masks ? d.arena.get<uint32_t>(4 * static_cast<size_t>(nc)) : nullptr;
       if (mask)
@@ -786,7 +904,7 @@ int parseq_stage(tt_engine* e, const uint8_t* crops, int n, const int32_t* force
       E_TRY(patchify_u8(cu8, nc, patches, d.stream));
       float* logits = nullptr;
       int* ids = nullptr;
-      E_TRY(d.parseq_forward(patches, nc, forced, &logits, &ids, pmax, mask));
+      E_TRY(d.parseq_forward(patches, nc, forced, &logits, &ids, pmax, mask, lex ? &lx : nullptr));
       if (logits_out)
         E_CUDA(cudaMemcpy2DAsync(logits_out + static_cast<size_t>(c0) * L * d.w->pd.n_cls, sizeof(float) * d.w->pd.n_cls, logits,
                                  sizeof(float) * NC, sizeof(float) * d.w->pd.n_cls, static_cast<size_t>(nc) * L,
@@ -809,17 +927,23 @@ extern "C" {
 
 int tt_parseq_forward(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens, float* logits_out,
                       int32_t* ids_out) {
-  return parseq_stage(e, crops, n, forced_tokens, nullptr, logits_out, ids_out, nullptr);
+  return parseq_stage(e, crops, n, forced_tokens, nullptr, nullptr, logits_out, ids_out, nullptr);
 }
 
 int tt_parseq_forward_scores(tt_engine* e, const uint8_t* crops, int n, int32_t* ids_out, float* pmax_out) {
   if (!pmax_out) { set_error("tt_parseq_forward_scores: null pmax_out"); return 1; }
-  return parseq_stage(e, crops, n, nullptr, nullptr, nullptr, ids_out, pmax_out);
+  return parseq_stage(e, crops, n, nullptr, nullptr, nullptr, nullptr, ids_out, pmax_out);
 }
 
 int tt_parseq_forward_masked(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens, const uint32_t* class_masks,
                              float* logits_out, int32_t* ids_out, float* pmax_out) {
-  return parseq_stage(e, crops, n, forced_tokens, class_masks, logits_out, ids_out, pmax_out);
+  return parseq_stage(e, crops, n, forced_tokens, class_masks, nullptr, logits_out, ids_out, pmax_out);
+}
+
+int tt_parseq_forward_lexicon(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens, const tt_lexicon* lex,
+                              float* logits_out, int32_t* ids_out, float* pmax_out) {
+  if (!lex) { set_error("tt_parseq_forward_lexicon: null lexicon"); return 1; }
+  return parseq_stage(e, crops, n, forced_tokens, nullptr, lex, logits_out, ids_out, pmax_out);
 }
 
 int tt_postprocess_dev(tt_engine* e, const float* maps_dev, int batch, int H, int W, int* n_rects_total, void*) {

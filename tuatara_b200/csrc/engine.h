@@ -97,6 +97,9 @@ struct DeviceCtx {
   PostWorkspace post;           // sized lazily for (batch, H, W)
   __nv_bfloat16* patch_buf = nullptr;  // recognition batch: bf16 patch rows [crops * 128][96] of the crops awaiting PARSeq
   size_t patch_cap = 0;                //   capacity in crops
+  void* lex_buf = nullptr;             // the automaton table of the lexicon request this slot runs (lexicon.h layout)
+  size_t lex_cap = 0;                  //   capacity in bytes
+  LexDev lex_view;                     //   its table pointers (root / state unset)
   uint8_t* pinned = nullptr;    // host staging for D2H of post results / ids
   size_t pinned_bytes = 0;
   std::mutex mu;                // one request at a time per device
@@ -113,8 +116,12 @@ struct DeviceCtx {
   // mask_dev (nullable, device [n][4] uint32, 16-byte aligned): per-crop class masks (tt_char_filter_mask); every greedy
   // choice -- each AR step's fed-back token and the refinement's ids -- and pmax run over the allowed classes only.  The
   // logits are not masked.
+  // lex (nullable; mask_dev is then null): the state path of a lexicon request (INTEGRATION.md section 9).  Every AR
+  // step feeds back the argmax over the classes its crop's state allows (from lex->root, advancing lex->state [n]);
+  // without forced_dev only.  The refinement's ids and pmax are a second walk from lex->root (lexicon_walk).
   cudaError_t parseq_forward(const __nv_bfloat16* patches_dev, int n, const int* forced_dev, float** logits_out,
-                             int** ids_out, float* pmax_dev = nullptr, const uint32_t* mask_dev = nullptr);
+                             int** ids_out, float* pmax_dev = nullptr, const uint32_t* mask_dev = nullptr,
+                             const LexDev* lex = nullptr);
   size_t parseq_bytes(int n) const;
 };
 

@@ -267,7 +267,7 @@ static cudaError_t lin(cudaStream_t s, const __nv_bfloat16* A, int lda, int M, i
 }
 
 cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const int* forced, float** logits_out,
-                                      int** ids_out, float* pmax_dev, const uint32_t* mask_dev) {
+                                      int** ids_out, float* pmax_dev, const uint32_t* mask_dev, const LexDev* lex) {
   using bf = __nv_bfloat16;
   const ParseqDims& pd = w->pd;
   const WeightFile& wf = w->parseq;
@@ -450,6 +450,12 @@ cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const
       const int* forced_h = forced ? forced + static_cast<size_t>(c0) * (L - 1) : nullptr;
       const bf* mkv_h = mem_kv + static_cast<size_t>(c0) * 128 * 2 * D;
       const uint32_t* mask_h = mask_dev ? mask_dev + static_cast<size_t>(c0) * 4 : nullptr;
+      LexDev lex_h{};   // the half's crops' walk state; under teacher forcing the AR steps do not consult the automaton
+      if (lex && !forced) {
+        lex_h = *lex;
+        lex_h.root += c0;
+        lex_h.state += c0;
+      }
       // lists hold crop indices relative to the half; step 0 works on all of them (no list)
       int* const cnt = act_n + half * L;
       const int* cur = (early && i > 0) ? act + static_cast<size_t>(i & 1) * n + c0 : nullptr;
@@ -459,7 +465,8 @@ cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const
       RUN(dec_self_attn(st, w->q_sa_table, w->sc_table, kv_table, tok_h, pd.eos_id, pd.n_tok, ab_h, hs));
       RUN(dec_dense_a2(w->dd, ab_h, nc, i, ts_h, qc_h, hs, cur, cur_n));
       RUN(dec_cross_attn(st, qc_h, mkv_h, ab_h, hs));
-      RUN(dec_dense_b(w->dd, ab_h, nc, i, ts_h, la_h, tok_h, forced_h, hs, cur, cur_n, mask_h));
+      RUN(dec_dense_b(w->dd, ab_h, nc, i, ts_h, la_h, tok_h, forced_h, hs, cur, cur_n, mask_h, lex_h.root ? &lex_h : nullptr,
+                      i == 0));
       if (early && i + 1 < L)
         RUN(dec_compact(cur, cur_n, nc, tok_h, L, i + 1, pd.eos_id, act + static_cast<size_t>((i + 1) & 1) * n + c0, cnt + i + 1, hs));
       return cudaSuccess;
@@ -489,12 +496,14 @@ cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const
       RUN(stream_tail(st, n, logits_ar + static_cast<size_t>(i) * NC, L * NC));
       if (i + 1 < L)
         RUN(argmax_rows(logits_ar + static_cast<size_t>(i) * NC, n, pd.n_cls, L * NC, nullptr, 0, tokens + i + 1, L,
-                        forced ? forced + i : nullptr, L - 1, s, mask_dev, 1));
+                        forced ? forced + i : nullptr, L - 1, s, mask_dev, 1, forced ? nullptr : lex, i == 0));
     }
   }
   DecoderStep st{n, D, pd.dec_heads, L, 0, L, 1};
   RUN(stream_tail(st, R, logits, NC));
-  if (pmax_dev)   // scores requested: the same ids plus each position's largest softmax probability, in the same launch
+  if (lex)   // lexicons: each crop walks its positions in order from its root (the ids, and pmax when requested)
+    RUN(lexicon_walk(logits, n, L, pd.n_cls, NC, *lex, ids, pmax_dev, s));
+  else if (pmax_dev)   // scores requested: the same ids plus each position's largest softmax probability, in the same launch
     RUN(argmax_conf_rows(logits, R, pd.n_cls, NC, ids, pmax_dev, s, mask_dev, L));
   else
     RUN(argmax_rows(logits, R, pd.n_cls, NC, ids, 1, nullptr, 0, nullptr, 0, s, mask_dev, L));
@@ -525,6 +534,7 @@ DeviceCtx::~DeviceCtx() {
   cudaSetDevice(device);
   post_workspace_free(&post);
   if (patch_buf) cudaFree(patch_buf);
+  if (lex_buf) cudaFree(lex_buf);
   if (pinned) cudaFreeHost(pinned);
   if (ev_fork) cudaEventDestroy(ev_fork);
   if (ev_join) cudaEventDestroy(ev_join);

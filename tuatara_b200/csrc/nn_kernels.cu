@@ -13,6 +13,7 @@
 #include "common.h"
 #include "epi_math.cuh"
 #include "gemm_tc.cuh"
+#include "lexicon.cuh"
 #include "ptx.cuh"
 #include "trace.h"
 
@@ -969,21 +970,62 @@ __global__ void __launch_bounds__(128) k_dec_attn_refine(const void* __restrict_
     }
 }
 
-// MASK: only the classes whose bit is set in the row's class mask compete (mask [rows / rows_per_mask][4], bit c & 31 of
-// word c >> 5).  Lane `lane` visits classes lane + 32 k, so its bit of word k is bit `lane`.
-template <bool MASK>
+// MM (MASK_NONE / MASK_CROP / MASK_STATE, lexicon.cuh): only the classes whose bit is set in the row's class mask
+// compete.  MASK_CROP: mask [rows / rows_per_mask][4], bit c & 31 of word c >> 5.  MASK_STATE (row = crop, the unfused AR
+// step): the allow row of the crop's state st_in[row]; an all-NaN row takes the lowest allowed class, and lx.state[row]
+// becomes the chosen class's successor.  Lane `lane` visits classes lane + 32 k, so its bit of word k is bit `lane`.
+template <int MM>
 __global__ void k_argmax(const float* __restrict__ logits, int rows, int n_cls, int ld, int* __restrict__ ids,
                          int ids_stride, int* __restrict__ next, int next_stride, const int* __restrict__ forced,
-                         int forced_stride, const uint32_t* __restrict__ mask, int rows_per_mask) {
+                         int forced_stride, const uint32_t* __restrict__ mask, int rows_per_mask, LexDev lx,
+                         const int* __restrict__ st_in) {
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (row >= rows) return;
   const float* l = logits + static_cast<long long>(row) * ld;
   uint4 mw = make_uint4(~0u, ~0u, ~0u, ~0u);
-  if constexpr (MASK) mw = *reinterpret_cast<const uint4*>(mask + static_cast<long long>(row / rows_per_mask) * 4);
+  int st = 0;
+  if constexpr (MM == MASK_CROP) mw = *reinterpret_cast<const uint4*>(mask + static_cast<long long>(row / rows_per_mask) * 4);
+  if constexpr (MM == MASK_STATE) {
+    st = st_in[row];
+    mw = lx.allow[st];
+  }
   const uint32_t mws[4] = {mw.x, mw.y, mw.z, mw.w};
   float best = -INFINITY;
   int bi = 0x7fffffff;
+  for (int c = lane, k = 0; c < n_cls; c += 32, ++k) {
+    const float v = l[c];
+    if ((MM == MASK_NONE || ((mws[k & 3] >> lane) & 1u)) && v > best) { best = v; bi = c; }  // strictly greater: first max per lane
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    const float ov = __shfl_xor_sync(0xffffffffu, best, o);
+    const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+    if (ov > best || (ov == best && oi < bi)) { best = ov; bi = oi; }  // ties -> lowest index (at::max on CPU)
+  }
+  if (bi >= n_cls) bi = MM == MASK_STATE ? lowest_class(mws) : 0;  // all-NaN row: no comparison succeeded (the id is used as a table index downstream)
+  if (lane == 0) {
+    if (ids != nullptr) ids[static_cast<long long>(row) * ids_stride] = bi;
+    if (next != nullptr) next[static_cast<long long>(row) * next_stride] = forced ? forced[static_cast<long long>(row) * forced_stride] : bi;
+    if constexpr (MM == MASK_STATE) lx.state[row] = lx.next[lx.first[st] + classes_below(mws, bi)];
+  }
+}
+
+// One row of the refinement head with scores: the argmax of k_argmax (same per-lane and cross-lane rules, so the ids are
+// bit-identical) and the sum whose inverse is the row's largest softmax probability, p = 1 / sum_c exp(l[c] - max),
+// summed per lane in class order and then over a fixed xor butterfly (every lane ends with the same bits), accurate
+// expf: p is deterministic.  A row with a NaN gets p = NaN.  The second pass re-reads the row from L1.  MASK: the argmax
+// and the sum both skip the classes whose bit is clear (p renormalised over the allowed classes); a mask that allows
+// every class gives the bits of MASK = false.  `none`: the id of a row where no allowed class compares (all NaN).
+// k_argmax_conf and k_lexicon_walk share it, so a one-state automaton gives k_argmax_conf's bits.
+struct RowChoice {
+  int id;
+  float sum;
+};
+template <bool MASK>
+__device__ __forceinline__ RowChoice argmax_conf_row(const float* l, int n_cls, int lane,
+                                                     const uint32_t (&mws)[4], int none) {
+  int bi = 0x7fffffff;
+  float best = -INFINITY;
   for (int c = lane, k = 0; c < n_cls; c += 32, ++k) {
     const float v = l[c];
     if ((!MASK || ((mws[k & 3] >> lane) & 1u)) && v > best) { best = v; bi = c; }  // strictly greater: first max per lane
@@ -993,18 +1035,15 @@ __global__ void k_argmax(const float* __restrict__ logits, int rows, int n_cls, 
     const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
     if (ov > best || (ov == best && oi < bi)) { best = ov; bi = oi; }  // ties -> lowest index (at::max on CPU)
   }
-  if (bi >= n_cls) bi = 0;  // all-NaN row: no comparison succeeded (the id is used as a table index downstream)
-  if (lane == 0) {
-    if (ids != nullptr) ids[static_cast<long long>(row) * ids_stride] = bi;
-    if (next != nullptr) next[static_cast<long long>(row) * next_stride] = forced ? forced[static_cast<long long>(row) * forced_stride] : bi;
-  }
+  if (bi >= n_cls) bi = none;  // all-NaN row
+  float sum = 0.f;
+  for (int c = lane, k = 0; c < n_cls; c += 32, ++k)
+    if (!MASK || ((mws[k & 3] >> lane) & 1u)) sum += expf(l[c] - best);
+  for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
+  return RowChoice{bi, sum};
 }
 
-// Refinement head with scores: the argmax of k_argmax (same per-lane and cross-lane rules, so the ids are bit-identical)
-// and the row's largest softmax probability p = 1 / sum_c exp(l[c] - max), summed per lane in class order and then over
-// a fixed xor butterfly (every lane ends with the same bits), accurate expf: p is deterministic.  A row with a NaN
-// gets p = NaN.  The second pass re-reads the row from L1.  MASK: the argmax and the sum both skip the classes whose bit
-// is clear (p renormalised over the allowed classes); a mask that allows every class gives the bits of MASK = false.
+// Refinement head with scores (argmax_conf_row per row); an all-NaN row gets id 0.
 template <bool MASK>
 __global__ void k_argmax_conf(const float* __restrict__ logits, int rows, int n_cls, int ld, int* __restrict__ ids,
                               float* __restrict__ pmax, const uint32_t* __restrict__ mask, int rows_per_mask) {
@@ -1015,25 +1054,32 @@ __global__ void k_argmax_conf(const float* __restrict__ logits, int rows, int n_
   uint4 mw = make_uint4(~0u, ~0u, ~0u, ~0u);
   if constexpr (MASK) mw = *reinterpret_cast<const uint4*>(mask + static_cast<long long>(row / rows_per_mask) * 4);
   const uint32_t mws[4] = {mw.x, mw.y, mw.z, mw.w};
-  float best = -INFINITY;
-  int bi = 0x7fffffff;
-  for (int c = lane, k = 0; c < n_cls; c += 32, ++k) {
-    const float v = l[c];
-    if ((!MASK || ((mws[k & 3] >> lane) & 1u)) && v > best) { best = v; bi = c; }  // strictly greater: first max per lane
-  }
-  for (int o = 16; o > 0; o >>= 1) {
-    const float ov = __shfl_xor_sync(0xffffffffu, best, o);
-    const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-    if (ov > best || (ov == best && oi < bi)) { best = ov; bi = oi; }  // ties -> lowest index (at::max on CPU)
-  }
-  if (bi >= n_cls) bi = 0;  // all-NaN row
-  float sum = 0.f;
-  for (int c = lane, k = 0; c < n_cls; c += 32, ++k)
-    if (!MASK || ((mws[k & 3] >> lane) & 1u)) sum += expf(l[c] - best);
-  for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
+  const RowChoice r = argmax_conf_row<MASK>(l, n_cls, lane, mws, 0);
   if (lane == 0) {
-    ids[row] = bi;
-    pmax[row] = 1.f / sum;
+    ids[row] = r.id;
+    pmax[row] = 1.f / r.sum;
+  }
+}
+
+// Refinement head of a lexicon request: one warp per crop walks its L rows in order from the crop's root, each row's
+// choice being argmax_conf_row under the current state's allow row (an all-NaN row takes the lowest allowed class); the
+// state then advances by the chosen class.  ids [n][L]; pmax (nullable) [n][L].
+__global__ void k_lexicon_walk(const float* __restrict__ logits, int n, int L, int n_cls, int ld, LexDev lx,
+                               int* __restrict__ ids, float* __restrict__ pmax) {
+  const int crop = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (crop >= n) return;
+  int st = lx.root[crop];
+  for (int t = 0; t < L; ++t) {
+    const long long row = static_cast<long long>(crop) * L + t;
+    const uint4 mw = lx.allow[st];
+    const uint32_t mws[4] = {mw.x, mw.y, mw.z, mw.w};
+    const RowChoice r = argmax_conf_row<true>(logits + row * ld, n_cls, lane, mws, lowest_class(mws));
+    if (lane == 0) {
+      ids[row] = r.id;
+      if (pmax != nullptr) pmax[row] = 1.f / r.sum;
+    }
+    st = lx.next[lx.first[st] + classes_below(mws, r.id)];
   }
 }
 
@@ -1253,14 +1299,17 @@ cudaError_t tokens_init(int* tokens, int n, int L, int bos, int pad, cudaStream_
 
 cudaError_t argmax_rows(const float* logits, int rows, int n_cls, int ld, int* ids, int ids_stride, int* next,
                         int next_stride, const int* forced, int forced_stride, cudaStream_t s, const uint32_t* mask,
-                        int rows_per_mask) {
+                        int rows_per_mask, const LexDev* lex, bool first_step) {
   if (rows <= 0) return cudaSuccess;
-  if (mask)
-    k_argmax<true><<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, ids_stride, next, next_stride, forced,
-                                                  forced_stride, mask, rows_per_mask);
+  if (lex)
+    k_argmax<MASK_STATE><<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, ids_stride, next, next_stride, forced,
+                                                        forced_stride, nullptr, 1, *lex, first_step ? lex->root : lex->state);
+  else if (mask)
+    k_argmax<MASK_CROP><<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, ids_stride, next, next_stride, forced,
+                                                       forced_stride, mask, rows_per_mask, LexDev{}, nullptr);
   else
-    k_argmax<false><<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, ids_stride, next, next_stride, forced,
-                                                   forced_stride, nullptr, 1);
+    k_argmax<MASK_NONE><<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, ids_stride, next, next_stride, forced,
+                                                       forced_stride, nullptr, 1, LexDev{}, nullptr);
   TT_LAUNCH_CHECK();
   return cudaSuccess;
 }
@@ -1272,6 +1321,14 @@ cudaError_t argmax_conf_rows(const float* logits, int rows, int n_cls, int ld, i
     k_argmax_conf<true><<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, pmax, mask, rows_per_mask);
   else
     k_argmax_conf<false><<<(rows + 7) / 8, 256, 0, s>>>(logits, rows, n_cls, ld, ids, pmax, nullptr, 1);
+  TT_LAUNCH_CHECK();
+  return cudaSuccess;
+}
+
+cudaError_t lexicon_walk(const float* logits, int n, int L, int n_cls, int ld, const LexDev& lex, int* ids, float* pmax,
+                         cudaStream_t s) {
+  if (n <= 0) return cudaSuccess;
+  k_lexicon_walk<<<(n + 7) / 8, 256, 0, s>>>(logits, n, L, n_cls, ld, lex, ids, pmax);
   TT_LAUNCH_CHECK();
   return cudaSuccess;
 }

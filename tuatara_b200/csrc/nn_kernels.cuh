@@ -19,6 +19,15 @@ cudaError_t maxpool3x3s1(const __nv_bfloat16* in, __nv_bfloat16* out, int B, int
 // F.interpolate(scale 2, bilinear, align_corners=False): [B][H][W][C] -> [B][2H][2W][C]
 cudaError_t upsample2x(const __nv_bfloat16* in, __nv_bfloat16* out, int B, int H, int W, int C, cudaStream_t s);
 
+// A request's lexicon automata on the device (lexicon.h: state 0 is the done state) and the walk state of its crops.
+struct LexDev {
+  const uint4* allow = nullptr;   // [S] class mask of each state
+  const int* first = nullptr;     // [S] index of the state's first successor in next
+  const int* next = nullptr;      // [E] successor of the state's k-th allowed class at next[first + k]
+  const int* root = nullptr;      // [n] root state of each crop
+  int* state = nullptr;           // [n] each crop's current state in the AR loop
+};
+
 // ---- PARSeq ------------------------------------------------------------------------------
 // LayerNorm over the last dim D (multiple of 32, <= 1024) of fp32 rows -> bf16 (and/or fp32) rows.
 // rows_mod > 0: input row = row % rows_mod (broadcast table, e.g. pos_queries).
@@ -64,14 +73,23 @@ cudaError_t dec_cross_attn(const DecoderStep& st, const __nv_bfloat16* q, const 
 // `forced` != null the value written to next_tokens comes from forced instead of the argmax.
 // mask (nullable, device [rows / rows_per_mask][4] uint32, 16-byte aligned): the class mask of each group of
 // rows_per_mask consecutive rows (1: row = crop; L: row = crop * L + t); only classes whose bit is set compete.
+// lex (nullable, rows = crops; mask is then unused): the allowed classes of crop c are the allow row of its state
+// (lex->root[c] when first_step, else lex->state[c]); lex->state[c] becomes the chosen class's successor.  An all-NaN row
+// takes the state's lowest allowed class.
 cudaError_t argmax_rows(const float* logits, int rows, int n_cls, int ld, int* ids, int ids_stride,
                         int* next_tokens, int next_stride, const int* forced, int forced_stride, cudaStream_t s,
-                        const uint32_t* mask = nullptr, int rows_per_mask = 1);
+                        const uint32_t* mask = nullptr, int rows_per_mask = 1, const LexDev* lex = nullptr,
+                        bool first_step = false);
 // argmax_rows' ids (same tie and NaN rules, bit-identical) fused with the largest softmax probability of the row,
 // pmax[row] = 1 / sum_c exp(logits[row][c] - max) in fp32 (deterministic; NaN for a row holding a NaN).  ids, pmax [rows].
 // mask as in argmax_rows: the max and the sum run over the allowed classes only.
 cudaError_t argmax_conf_rows(const float* logits, int rows, int n_cls, int ld, int* ids, float* pmax, cudaStream_t s,
                              const uint32_t* mask = nullptr, int rows_per_mask = 1);
+// Refinement head of a lexicon request (INTEGRATION.md section 9): per crop, a walk over its L rows of logits [n][L][ld]
+// from lex.root[crop]; each row's id is the argmax over its state's allowed classes (argmax_conf_rows' rules; an all-NaN
+// row takes the lowest allowed class) and p the probability renormalised over them.  ids [n][L], pmax (nullable) [n][L].
+cudaError_t lexicon_walk(const float* logits, int n, int L, int n_cls, int ld, const LexDev& lex, int* ids, float* pmax,
+                         cudaStream_t s);
 // u8 crops [n][32][128][3] -> bf16 patch rows [n*128][96] (raw 0..255), k = c*32 + (y%4)*8 + x%8
 cudaError_t tokens_init(int* tokens, int n, int L, int bos, int pad, cudaStream_t s);
 // AR early exit: the crops of (active_in, *n_in) -- null: all n crops -- whose token at position `pos` is not EOS, in the
