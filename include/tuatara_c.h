@@ -288,6 +288,11 @@ TT_API int tt_linear_dev(const void* A, int lda, int M, int K, const void* W, in
 TT_API int tt_linear_ln_pair_dev(const void* A, int M, int K1, const void* W1, const float* b1, int D, void* x_hi, void* x_lo,
                           float* stats, const void* W2f, const float* c0, const float* c1, int N2, int act, float eps,
                           void* out, void* stream);
+/* The LayerNorm-consumer GEMM alone (the second half of tt_linear_ln_pair_dev): out = LN(x) W^T + b from A = bf16(x)
+ * [M][K], stats fp32 [M][parts][2] (1 <= parts <= 4 partial (sum x, sum x^2) pairs per row), Wf = W * gamma bf16 [N][K],
+ * c0 / c1 fp32 [N] as above; out bf16 [M][N].  All device pointers. */
+TT_API int tt_linear_ln_dev(const void* A, int M, int K, const void* Wf, const float* c0, const float* c1, int N, const float* stats,
+                            int parts, float eps, void* out, void* stream);
 /* Kernel test of the fused second half of a PARSeq-base encoder block (timm Block, reached by the reference through
  * TorchScript at tuatara.cpp:307):  x += att Wp^T + bp  (the attention output projection; skipped when att is NULL), then
  * x += fc2(GELU(fc1(LN2(x)))) -- one kernel, neither x1 nor the hidden activations leave the SM.  The residual stream is the
@@ -297,6 +302,13 @@ TT_API int tt_linear_ln_pair_dev(const void* A, int M, int K1, const void* W1, c
  * All device pointers. */
 TT_API int tt_enc_mlp_dev(void* x_hi, void* x_lo, float* stats, long long M, const void* att, const void* Wp, const float* bp,
                    const void* W1f, const float* c0, const float* c1, const void* W2, const float* b2, float eps, void* stream);
+/* Kernel test of the fused first half of a PARSeq encoder block: qkv = LN1(x) Wqkv^T + b (LayerNorm applied to the
+ * accumulators, as tt_linear_ln_pair_dev's second GEMM does) and the self attention of tt_attn_enc_dev (one-pass), in one
+ * kernel -- qkv never leaves the SM.  x_hi bf16 [crops*128][D] (D = 384 or 192, heads = D / 64), stats fp32 [crops*128]
+ * [parts][2] (1 <= parts <= 4 partial (sum x, sum x^2) pairs per row), Wf = Wqkv * gamma bf16 [3D][D], c0 / c1 fp32 [3D]
+ * (16-byte aligned), att bf16 [crops*128][D].  All device pointers. */
+TT_API int tt_enc_qkv_attn_dev(const void* x_hi, const float* stats, int parts, const void* Wf, const float* c0, const float* c1,
+                               void* att, int crops, int D, int heads, float eps, void* stream);
 /* NHWC bf16 stride-1 "same" convolution as implicit GEMM; src1 may be NULL (else channel concat).
  * weight bf16 [Cout][taps][C0+C1]; out bf16 [batch][H][W][Cout]. */
 TT_API int tt_conv_dev(const void* src0, int C0, const void* src1, int C1, int batch, int H, int W, int taps, int dil,

@@ -112,7 +112,9 @@ SIGNATURES = {
     "tt_rect_to_bbox": (_I, [_P, _P]),
     "tt_linear_dev": (_I, [_P, _I, _I, _I, _P, _I, _P, _I, _P, _I, _I, _P, _I, _I, _I, _I, _P]),
     "tt_linear_ln_pair_dev": (_I, [_P, _I, _I, _P, _P, _I, _P, _P, _P, _P, _P, _P, _I, _I, C.c_float, _P, _P]),
+    "tt_linear_ln_dev": (_I, [_P, _I, _I, _P, _P, _P, _I, _P, _I, C.c_float, _P, _P]),
     "tt_enc_mlp_dev": (_I, [_P, _P, _P, C.c_longlong, _P, _P, _P, _P, _P, _P, _P, _P, C.c_float, _P]),
+    "tt_enc_qkv_attn_dev": (_I, [_P, _P, _I, _P, _P, _P, _P, _I, _I, _I, C.c_float, _P]),
     "tt_conv_dev": (_I, [_P, _I, _P, _I, _I, _I, _I, _I, _I, _P, _P, _I, _I, _P, _I, _I, _P]),
     "tt_attn_enc_dev": (_I, [_P, _P, _I, _I, _I, _I, _P]),
     "tt_dec_score_table_dev": (_I, [_P, _P, _I, _I, _I, _I, _P, _P]),

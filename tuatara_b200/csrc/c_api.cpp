@@ -10,6 +10,7 @@
 #include "common.h"
 #include "detect.h"
 #include "enc_mlp.cuh"
+#include "enc_qkv_attn.cuh"
 #include "engine.h"
 #include "lexicon.h"
 #include "gemm_tc.cuh"
@@ -417,6 +418,19 @@ int tt_linear_ln_pair_dev(const void* A, int M, int K1, const void* W1, const fl
   });
 }
 
+int tt_linear_ln_dev(const void* A, int M, int K, const void* Wf, const float* c0, const float* c1, int N, const float* stats,
+                     int parts, float eps, void* out, void* stream) {
+  return guarded([&]() -> int {
+    LinearProblem l;
+    l.A = static_cast<const __nv_bfloat16*>(A); l.lda = K; l.M = M; l.K = K;
+    l.W = static_cast<const __nv_bfloat16*>(Wf); l.N = N;
+    Epilogue e;
+    e.bias = c0; e.out = out; e.out_type = OUT_BF16; e.ldc = N;
+    e.ln_stats_in = stats; e.ln_c1 = c1; e.ln_parts = parts; e.ln_dim = K; e.ln_eps = eps;
+    return linear_forward(l, e, static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : 1;
+  });
+}
+
 int tt_enc_mlp_dev(void* x_hi, void* x_lo, float* stats, long long M, const void* att, const void* Wp, const float* bp,
                    const void* W1f, const float* c0, const float* c1, const void* W2, const float* b2, float eps, void* stream) {
   return guarded([&]() -> int {
@@ -427,6 +441,15 @@ int tt_enc_mlp_dev(void* x_hi, void* x_lo, float* stats, long long M, const void
     pj.att = static_cast<const __nv_bfloat16*>(att); pj.wp = static_cast<const __nv_bfloat16*>(Wp); pj.bp = bp;
     return enc_mlp_forward(w, static_cast<__nv_bfloat16*>(x_hi), static_cast<__nv_bfloat16*>(x_lo), stats, 2, M, 384, 1536, eps,
                            static_cast<cudaStream_t>(stream), att ? &pj : nullptr) == cudaSuccess ? 0 : 1;
+  });
+}
+
+int tt_enc_qkv_attn_dev(const void* x_hi, const float* stats, int parts, const void* Wf, const float* c0, const float* c1, void* att,
+                        int crops, int D, int heads, float eps, void* stream) {
+  return guarded([&]() -> int {
+    return enc_qkv_attn_forward(static_cast<const __nv_bfloat16*>(x_hi), stats, parts, static_cast<const __nv_bfloat16*>(Wf), c0, c1,
+                                static_cast<__nv_bfloat16*>(att), crops, D, heads, eps, static_cast<cudaStream_t>(stream)) == cudaSuccess
+               ? 0 : 1;
   });
 }
 

@@ -13,6 +13,7 @@
 #include "common.h"
 #include "dec_fused.cuh"
 #include "enc_mlp.cuh"
+#include "enc_qkv_attn.cuh"
 #include "engine.h"
 #include "gemm_tc.cuh"
 #include "nn_kernels.cuh"
@@ -243,10 +244,26 @@ cudaError_t DeviceCtx::craft_forward(const uint8_t* in, int B, int H, int W, flo
 }
 
 // ---------------------------------------------------------------------------------- PARSeq
+// LayerNorm fused away (see parseq_forward); TT_ENC_LNFUSE=0 keeps the standalone LayerNorm.  Read per call: the parity
+// test flips it in-process.
+static bool enc_ln_fused(const WeightFile& wf) {
+  const char* e = std::getenv("TT_ENC_LNFUSE");
+  return !(e && std::atoi(e) == 0) && wf.has("b0.qkv.wf") && wf.has("dec.ca.kvf.wf");
+}
+static bool enc_attn_onepass() {   // TT_ATTN_ONEPASS=0: the two-pass encoder attention (A/B runs)
+  static const bool v = !(std::getenv("TT_ATTN_ONEPASS") && std::atoi(std::getenv("TT_ATTN_ONEPASS")) == 0);
+  return v;
+}
+// qkv projection + attention as one kernel (enc_qkv_attn.cu): the LayerNorm-fused stream only, no qkv buffer then
+static bool enc_qkv_attn_fused(const WeightFile& wf, const ParseqDims& pd) {
+  return enc_ln_fused(wf) && enc_attn_onepass() && enc_qkv_attn_supported(pd.D, pd.enc_heads);
+}
+
 size_t DeviceCtx::parseq_bytes(int n) const {
   const ParseqDims& pd = w->pd;
   const size_t M = static_cast<size_t>(n) * 128, D = pd.D;
-  size_t b = M * D * 4 + M * D * 2 + M * 3 * D * 2 + M * D * 2 + M * pd.mlp * 2 + M * D * 2 + M * 32 + M * 2 * D * 2;  // encoder
+  const size_t qkv = enc_qkv_attn_fused(w->parseq, pd) ? 0 : M * 3 * D * 2;
+  size_t b = M * D * 4 + M * D * 2 + qkv + M * D * 2 + M * pd.mlp * 2 + M * D * 2 + M * 32 + M * 2 * D * 2;  // encoder
   const size_t R = static_cast<size_t>(n) * pd.L;
   b += R * 4 + R * D * (4 + 2 + 2 + 2) + R * pd.mlp * 2 + 2 * R * pd.n_cls_pad * 4 + 2 * R * 4;
   b += dec_dense_scratch_floats(n, pd.D) * 4;
@@ -287,19 +304,21 @@ cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const
   // fp32 and emit the rows' (sum, sum of squares); qkv / fc1 / the memory K|V projection read `hi` (= bf16(x)) with
   // gamma folded into their weights and apply (mean, rstd) in the epilogue.  Needs the folded tensors of the current
   // weights.py; TT_ENC_LNFUSE=0 keeps the fp32 stream and the standalone LayerNorm kernel (A/B runs, parity test).
-  const char* lnf_env = std::getenv("TT_ENC_LNFUSE");
-  const bool lnf = !(lnf_env && std::atoi(lnf_env) == 0) && wf.has("b0.qkv.wf") && wf.has("dec.ca.kvf.wf");
+  const bool lnf = enc_ln_fused(wf);
+  // LN1 + qkv + attention in one kernel whenever the stream is LayerNorm-fused: qkv never reaches HBM (enc_qkv_attn.cu)
+  const bool qkv_attn = enc_qkv_attn_fused(wf, pd);
   // fc1 + GELU + fc2 + residual as one kernel (enc_mlp.cu; PARSeq-base dims, split stream): the hidden activations stay
   // on the SM.  TT_ENC_MLPFUSE=0 keeps the two GEMM launches (A/B runs, parity test); PARSeq-tiny always takes them.
   const char* mf_env = std::getenv("TT_ENC_MLPFUSE");   // read per call: the parity test flips it in-process
   const bool mlp_fuse = lnf && !(mf_env && std::atoi(mf_env) == 0) && enc_mlp_supported(D, pd.mlp);
   const char* pf_env = std::getenv("TT_ENC_PROJFUSE");   // 0: the attention output projection stays a GEMM launch (A/B runs)
   const bool proj_fuse = !(pf_env && std::atoi(pf_env) == 0);
-  static const bool attn_onepass = !(std::getenv("TT_ATTN_ONEPASS") && std::atoi(std::getenv("TT_ATTN_ONEPASS")) == 0);  // 0: A/B runs
+  const bool attn_onepass = enc_attn_onepass();
   ARENA_GET(x, float, Mc * D);       // fp32 residual stream (unfused) / the lo half of the split stream (fused; first half of the buffer)
   ARENA_GET(h, bf, Mc * D);          // LayerNorm output (unfused) / the hi half of the split stream = bf16(x) (fused)
   bf* const x_lo = reinterpret_cast<bf*>(x);
-  ARENA_GET(qkv, bf, Mc * 3 * D);
+  bf* qkv = nullptr;
+  if (!qkv_attn) { ARENA_GET(qkv_buf, bf, Mc * 3 * D); qkv = qkv_buf; }
   ARENA_GET(att, bf, Mc * D);
   ARENA_GET(hid, bf, Mc * pd.mlp);
   ARENA_GET(mem, bf, Mc * D);
@@ -347,8 +366,13 @@ cudaError_t DeviceCtx::parseq_forward(const __nv_bfloat16* patches, int n, const
     for (int i = 0; i < pd.depth; ++i) {
       const std::string p = "b" + std::to_string(i) + ".";
       if (!lnf) RUN(layernorm(x, Mi, D, wf.f32(p + "ln1.g"), wf.f32(p + "ln1.b"), 1e-6f, h, nullptr, 0, s));
-      RUN(ln_gemm(p + "qkv", Mi, 3 * D, ACT_NONE, qkv));
-      RUN(attention_enc(qkv, att, nc, D, pd.enc_heads, attn_onepass, s));
+      if (qkv_attn) {
+        RUN(enc_qkv_attn_forward(h, lnstats, ln_parts, wf.bf(p + "qkv.wf"), wf.f32(p + "qkv.c0"), wf.f32(p + "qkv.c1"), att, nc, D,
+                                 pd.enc_heads, 1e-6f, s));
+      } else {
+        RUN(ln_gemm(p + "qkv", Mi, 3 * D, ACT_NONE, qkv));
+        RUN(attention_enc(qkv, att, nc, D, pd.enc_heads, attn_onepass, s));
+      }
       if (mlp_fuse && proj_fuse) {
         // proj + residual + fc1 -> GELU -> fc2 + residual in one kernel: x1 never leaves the SM either (enc_mlp.cu)
         EncMlpWeights mw;

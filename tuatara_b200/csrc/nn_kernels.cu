@@ -10,6 +10,7 @@
 
 #include <cstdlib>
 
+#include "attn_softmax.cuh"
 #include "common.h"
 #include "epi_math.cuh"
 #include "gemm_tc.cuh"
@@ -395,45 +396,8 @@ __global__ void __launch_bounds__(128, ONEPASS ? 3 : 4) k_attn_enc(const __grid_
   const uint32_t t_row = tmem + (static_cast<uint32_t>(warp * 32) << 16);
   float sum = 0.f;
   const int r = tid;
-  // P as the A operand of the second MMA: K-major SWIZZLE_128B, keys [64b, 64b+64) in atom block b
-  auto store_p16 = [&](int ch, const float (&p)[16]) {
-    uint8_t* blk = sP + (ch >> 2) * 16384 + r * 128;
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      const int chunk = ((ch & 3) * 2 + h) ^ (r & 7);
-      uint4 u;
-      u.x = pack_bf16(p[8 * h + 0], p[8 * h + 1]); u.y = pack_bf16(p[8 * h + 2], p[8 * h + 3]);
-      u.z = pack_bf16(p[8 * h + 4], p[8 * h + 5]); u.w = pack_bf16(p[8 * h + 6], p[8 * h + 7]);
-      *reinterpret_cast<uint4*>(blk + chunk * 16) = u;
-    }
-  };
   if constexpr (ONEPASS) {
-    uint32_t raw[4][32];
-#pragma unroll
-    for (int b = 0; b < 4; ++b) ptx::tmem_ld<32>(t_row + b * 32, raw[b]);
-#pragma unroll
-    for (int b = 0; b < 4; ++b) ptx::tmem_ld_wait(raw[b]);
-    float m4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-#pragma unroll
-    for (int b = 0; b < 4; ++b)
-#pragma unroll
-      for (int i = 0; i < 32; ++i) m4[i & 3] = fmaxf(m4[i & 3], __uint_as_float(raw[b][i]));
-    const float mx = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3]));
-    const float nms = -mx * scale_log2e;
-    float s4[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-    for (int ch = 0; ch < 8; ++ch) {
-      float p[16];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        // exp2((s - mx) * scale) as one FFMA + one MUFU (arguments <= 0: no range fix-up needed)
-        const float a = fmaf(__uint_as_float(raw[ch >> 1][(ch & 1) * 16 + i]), scale_log2e, nms);
-        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(p[i]) : "f"(a));
-        s4[i & 3] += p[i];
-      }
-      store_p16(ch, p);
-    }
-    sum = (s4[0] + s4[1]) + (s4[2] + s4[3]);
+    sum = attn_softmax_onepass(t_row, sP, r, scale_log2e);
   } else {
     float mx = -INFINITY;
 #pragma unroll
@@ -455,7 +419,7 @@ __global__ void __launch_bounds__(128, ONEPASS ? 3 : 4) k_attn_enc(const __grid_
         p[i] = exp2f((__uint_as_float(raw[i]) - mx) * scale_log2e);
         sum += p[i];
       }
-      store_p16(ch, p);
+      attn_store_p16(sP, r, ch, p);
     }
   }
   // generic-proxy smem writes -> visible to the tensor core (async proxy); all S reads retired

@@ -52,6 +52,18 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
       : "memory");
   return ok != 0;
 }
+// Non-blocking probe (try_wait may suspend the thread for a while; a thread that polls several barriers must not be)
+__device__ __forceinline__ bool mbar_test_wait(uint64_t* bar, uint32_t parity) {
+  uint32_t ok;
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+      "selp.u32 %0, 1, 0, p;\n\t}"
+      : "=r"(ok)
+      : "r"(smem_u32(bar)), "r"(parity)
+      : "memory");
+  return ok != 0;
+}
 // Bounded wait: a protocol bug traps (-> launch error the host reports) instead of hanging the GPU.  The bound
 // is wall time (%globaltimer): 4 s, orders of magnitude above any legitimate wait in these kernels.
 __device__ __forceinline__ uint64_t globaltimer_ns() {
