@@ -100,6 +100,14 @@ class Lexicon {
   std::string err_ = "empty lexicon";
 };
 
+// The contrast re-read (tt_ocr_pages_contrast, INTEGRATION.md section 10): a word read with a confidence below
+// contrast_ths from a low-contrast crop is read again from a contrast-stretched crop, and the more confident read is kept.
+// The defaults are EasyOCR's readtext defaults.
+struct Contrast {
+  float contrast_ths = 0.1f;
+  float adjust_contrast = 0.5f;
+};
+
 namespace detail {
 inline tt_engine* engine_for(const std::string& weights_dir) {
   static std::mutex mu;
@@ -122,14 +130,15 @@ inline tt_engine* engine_for(const std::string& weights_dir) {
 
 namespace detail {
 // The one path of every entry point: the checks, the soft failures ({} after printing the reason), one
-// tt_ocr_pages_lexicon call and the walk over its result.  Each item's scores are fetched when `scores`, its angle when
+// tt_ocr_pages_contrast call and the walk over its result.  Each item's scores are fetched when `scores`, its angle when
 // rotation_info is not empty.  filters: none (empty), one for every page, or one per page.  lexicons (tt_lexicon
-// handles): likewise; a null entry is a page without lexicon.
+// handles): likewise; a null entry is a page without lexicon.  contrast: off (contrast_ths 0) unless given.
 inline std::vector<std::vector<ScoredItem>> ocr_pages(const std::vector<ImageView>& images, const std::string& weights_dir,
                                                       const std::string& outputs_dir, bool scores,
                                                       const std::vector<CharFilter>& filters,
                                                       const std::vector<int>& rotation_info = {},
-                                                      const std::vector<const tt_lexicon*>& lexicons = {}) {
+                                                      const std::vector<const tt_lexicon*>& lexicons = {},
+                                                      const Contrast& contrast = Contrast{0.f, 0.5f}) {
   std::vector<std::vector<ScoredItem>> out;
   if (weights_dir.empty()) { std::cerr << "Please provide a value for weights_dir" << std::endl; return out; }
   if (outputs_dir.empty()) { std::cerr << "Please provide a value for outputs_dir" << std::endl; return out; }
@@ -146,9 +155,9 @@ inline std::vector<std::vector<ScoredItem>> ocr_pages(const std::vector<ImageVie
   tt_ocr_options opt = {};
   opt.with_scores = scores ? 1 : 0;
   tt_result* r = nullptr;
-  if (tt_ocr_pages_lexicon(e, pages.data(), static_cast<int>(pages.size()), &opt, f.data(), static_cast<int>(f.size()),
-                           rotation_info.data(), static_cast<int>(rotation_info.size()), lexicons.data(),
-                           static_cast<int>(lexicons.size()), &r) != 0) {
+  if (tt_ocr_pages_contrast(e, pages.data(), static_cast<int>(pages.size()), &opt, f.data(), static_cast<int>(f.size()),
+                            rotation_info.data(), static_cast<int>(rotation_info.size()), lexicons.data(),
+                            static_cast<int>(lexicons.size()), contrast.contrast_ths, contrast.adjust_contrast, &r) != 0) {
     std::cerr << "tuatara: " << tt_last_error() << std::endl;
     return out;
   }
@@ -319,6 +328,43 @@ inline std::vector<ScoredItem> image_to_data_oriented(const ImageView& image, co
   return pages.empty() ? std::vector<ScoredItem>{} : pages[0];
 }
 
+// The contrast re-read (tt_ocr_pages_contrast, INTEGRATION.md section 10) on every page; Contrast() is EasyOCR's
+// defaults.  Same soft failures; an invalid value prints the error and returns {}.
+inline std::vector<std::vector<OutputItem>> image_to_data_batch(const std::vector<ImageView>& images,
+                                                                const std::string& weights_dir,
+                                                                const std::string& outputs_dir, const Contrast& contrast) {
+  return detail::unscored(detail::ocr_pages(images, weights_dir, outputs_dir, false, {}, {}, {}, contrast));
+}
+
+inline std::vector<std::vector<ScoredItem>> image_to_data_scored_batch(const std::vector<ImageView>& images,
+                                                                       const std::string& weights_dir,
+                                                                       const std::string& outputs_dir,
+                                                                       const Contrast& contrast) {
+  return detail::ocr_pages(images, weights_dir, outputs_dir, true, {}, {}, {}, contrast);
+}
+
+inline std::vector<ScoredItem> image_to_data_scored(const ImageView& image, const std::string& weights_dir,
+                                                    const std::string& outputs_dir, const Contrast& contrast) {
+  std::vector<std::vector<ScoredItem>> pages = image_to_data_scored_batch({image}, weights_dir, outputs_dir, contrast);
+  return pages.empty() ? std::vector<ScoredItem>{} : pages[0];
+}
+
+inline std::vector<std::vector<ScoredItem>> image_to_data_oriented_batch(const std::vector<ImageView>& images,
+                                                                         const std::string& weights_dir,
+                                                                         const std::string& outputs_dir,
+                                                                         const std::vector<int>& rotation_info,
+                                                                         const Contrast& contrast) {
+  return detail::ocr_pages(images, weights_dir, outputs_dir, true, {}, rotation_info, {}, contrast);
+}
+
+inline std::vector<ScoredItem> image_to_data_oriented(const ImageView& image, const std::string& weights_dir,
+                                                      const std::string& outputs_dir, const std::vector<int>& rotation_info,
+                                                      const Contrast& contrast) {
+  std::vector<std::vector<ScoredItem>> pages =
+      image_to_data_oriented_batch({image}, weights_dir, outputs_dir, rotation_info, contrast);
+  return pages.empty() ? std::vector<ScoredItem>{} : pages[0];
+}
+
 }  // namespace tuatara
 
 inline std::vector<OutputItem> image_to_data(const tuatara::ImageView& image, std::string weights_dir,
@@ -338,6 +384,13 @@ inline std::vector<OutputItem> image_to_data(const tuatara::ImageView& image, st
 inline std::vector<OutputItem> image_to_data(const tuatara::ImageView& image, std::string weights_dir,
                                              std::string outputs_dir, const tuatara::Lexicon& lexicon) {
   auto pages = tuatara::image_to_data_batch({image}, weights_dir, outputs_dir, lexicon);
+  return pages.empty() ? std::vector<OutputItem>{} : pages[0];
+}
+
+// image_to_data with the contrast re-read: a low-confidence word on a low-contrast crop is read again, stretched.
+inline std::vector<OutputItem> image_to_data(const tuatara::ImageView& image, std::string weights_dir,
+                                             std::string outputs_dir, const tuatara::Contrast& contrast) {
+  auto pages = tuatara::image_to_data_batch({image}, weights_dir, outputs_dir, contrast);
   return pages.empty() ? std::vector<OutputItem>{} : pages[0];
 }
 

@@ -172,6 +172,21 @@ TT_API int tt_lexicon_info(const tt_lexicon* lex, int* n_words, int* n_states);
 TT_API int tt_ocr_pages_lexicon(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
                                 const tt_char_filter* filters, int n_filters, const int* rotation_info, int n_rotations,
                                 const tt_lexicon* const* lexicons, int n_lexicons, tt_result** out);
+/* The contrast re-read (INTEGRATION.md section 10, EasyOCR's readtext(contrast_ths, adjust_contrast)): tt_ocr_pages_lexicon
+ * where a word whose first read has conf (tt_item_scores, under its page's filter or lexicon) below contrast_ths and whose
+ * 128 x 32 crop has low contrast is read again from a contrast-stretched crop.  On the crop (the winning rotation candidate,
+ * rectify 0 or 1): grey = cv2 BGR2GRAY of its channels in the caller's order, low / high = np.percentile(grey, 10 / 90),
+ * contrast = (high - low) / max(10, high + low); low contrast iff contrast < adjust_contrast.  Then every channel value v
+ * becomes uint8(clip((v - low + 25) * 200 / max(10, high - low), 0, 255)) in double (EasyOCR's adjust_contrast_grey, one
+ * map for all three channels), and the crop is decoded again under the same filter or lexicon, at the same angle.  The
+ * second read replaces the first only when its conf is strictly greater (ties and NaN keep the first; EasyOCR gives ties
+ * to the second).  text, and with with_scores conf and char_conf, are the winner's; bbox, det_score, angle and item order
+ * do not change.  contrast_ths: finite, >= 0 (0 = off: exactly tt_ocr_pages_lexicon); adjust_contrast: finite, in (0, 1]
+ * (EasyOCR's defaults are 0.1 and 0.5).  Any other value is an error that names it, reported before any device work. */
+TT_API int tt_ocr_pages_contrast(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
+                                 const tt_char_filter* filters, int n_filters, const int* rotation_info, int n_rotations,
+                                 const tt_lexicon* const* lexicons, int n_lexicons, float contrast_ths, float adjust_contrast,
+                                 tt_result** out);
 /* The angle (0, 90, 180 or 270) of the candidate that was read for item `item` of page `page`, -1 when the item was not
  * recognised (detect_only).  An error on a result not made by tt_ocr_pages_oriented with n_rotations > 0. */
 TT_API int tt_item_angle(const tt_result* r, int page, int item, int* angle);
@@ -254,6 +269,10 @@ TT_API int tt_parseq_forward_masked(tt_engine* e, const uint8_t* crops, int n, c
  * forwards).  Every output pointer may be NULL. */
 TT_API int tt_parseq_forward_lexicon(tt_engine* e, const uint8_t* crops, int n, const int32_t* forced_tokens,
                                      const tt_lexicon* lex, float* logits_out, int32_t* ids_out, float* pmax_out);
+/* The contrast stretch of tt_ocr_pages_contrast on host crops [n][32][128][3] (tt_crop_resize's layout): out [n][32][128][3]
+ * holds each crop stretched when it has low contrast for adjust_contrast (in (0, 1]), else unchanged; stretched
+ * (nullable) [n] is 1 for a stretched crop, else 0.  Runs the kernels the engine runs. */
+TT_API int tt_contrast_adjust(const uint8_t* crops, int n, float adjust_contrast, uint8_t* out, int32_t* stretched);
 /* Tokenizer::decode + truncation (tuatara.cpp:61-116, :497-502). ids [n][len]; out [n][out_stride] chars. */
 TT_API int tt_decode(const int32_t* ids, int n, int len, char* out, int out_stride);
 /* tt_decode with the scores of tt_item_scores (host only).  pmax [n][len]; conf_out (nullable) [n];
@@ -340,6 +359,10 @@ TT_API int tt_dec_cross_attn_dev(int n_crops, int D, int heads, int L, int p0, i
  * pmax_out [n_words][26] (nullable) and angle_out [n_words].  Device pointers except angles. */
 TT_API int tt_orient_select_dev(const int32_t* ids, const float* pmax, int n_words, const int32_t* angles, int n_candidates,
                                 int32_t* ids_out, float* pmax_out, int32_t* angle_out, void* stream);
+/* Kernel test of the contrast re-read's choice: for i < n_listed, the second read ids2 int32 / pmax2 fp32 [n_listed][26]
+ * replaces ids / pmax [.][26] of word list[i] in place when its conf is strictly greater.  Device pointers. */
+TT_API int tt_contrast_select_dev(int32_t* ids, float* pmax, const int32_t* list, int n_listed, const int32_t* ids2,
+                                  const float* pmax2, void* stream);
 /* Kernel test of the lexicon refinement head: the walk of lex's trie over device logits fp32 [n][26][95], every crop from
  * the root.  Writes ids_out int32 [n][26] and pmax_out fp32 [n][26] (nullable), device pointers. */
 TT_API int tt_lexicon_walk_dev(const tt_lexicon* lex, const float* logits, int n, int32_t* ids_out, float* pmax_out,

@@ -17,7 +17,7 @@ from ._native import TuataraError, check, lib, ptr
 
 __all__ = [
     "TuataraError", "Engine", "image_to_data", "images_to_data", "image_to_data_scored", "images_to_data_scored",
-    "default_config", "resize_plan", "preprocess", "postprocess", "crop_resize", "decode_ids", "decode_scores", "tokenizer_table",
+    "default_config", "resize_plan", "preprocess", "postprocess", "crop_resize", "contrast_adjust", "decode_ids", "decode_scores", "tokenizer_table",
     "char_filter_mask", "Lexicon", "min_area_rect", "convex_hull",
     "rect_points", "rect_bounding", "adjust_rect", "rect_to_bbox", "launch_count",
 ]
@@ -278,6 +278,20 @@ def crop_resize(image: np.ndarray, rects_xywh, angles=None) -> np.ndarray:
     return out
 
 
+def contrast_adjust(crops, adjust_contrast: float = 0.5):
+    """The contrast stretch of the contrast re-read (tt_contrast_adjust, INTEGRATION.md section 10) on the GPU.  crops:
+    uint8 [n, 32, 128, 3] (crop_resize's output) -> (uint8 [n, 32, 128, 3], stretched bool [n]): each crop whose grey
+    contrast is below adjust_contrast stretched by EasyOCR's adjust_contrast_grey map on all three channels, the rest
+    unchanged."""
+    x = np.ascontiguousarray(crops, np.uint8)
+    if x.ndim != 4 or x.shape[1:] != (32, 128, 3):
+        raise ValueError(f"contrast_adjust: expected crops of shape (n, 32, 128, 3), got {x.shape}")
+    out = np.empty_like(x)
+    flags = np.empty(len(x), np.int32)
+    check(lib().tt_contrast_adjust(ptr(x), len(x), float(adjust_contrast), ptr(out), ptr(flags)), "tt_contrast_adjust")
+    return out, flags.astype(bool)
+
+
 def rect_to_quad(rect) -> np.ndarray:
     """The quadrilateral tt_config.rectify warps for a RotatedRect: float32 [4, 2] (tl, tr, br, bl)."""
     out = np.zeros(8, np.float32)
@@ -320,7 +334,7 @@ class Engine:
 
     def ocr_pages(self, images: list, score_override: list | None = None, detect_only: bool = False,
                   scores: bool = False, *, allowlist=None, blocklist=None, rotation_info=None,
-                  lexicon=None) -> list[list[dict]]:
+                  lexicon=None, contrast_ths: float = 0.0, adjust_contrast: float = 0.5) -> list[list[dict]]:
         """images: uint8 [H,W,3] numpy arrays (host) or torch CUDA tensors (already on the device).
         score_override: optional per-page float32 [h32/2, w32/2, 2] maps (numpy or CUDA tensors, or
         None entries) that replace CRAFT's output after CRAFT has run (benchmark / parity tests).
@@ -332,7 +346,10 @@ class Engine:
         that many degrees counter-clockwise and the candidate with the highest word confidence wins; every item then
         carries "angle" (0, 90, 180 or 270; -1 when not recognised).  An empty iterable reads every word upright.
         lexicon: every recognised word is one of a word list (INTEGRATION.md section 9): a Lexicon or an iterable of
-        str for every page, or a list with one Lexicon or None per page (None: the page decodes as without lexicon)."""
+        str for every page, or a list with one Lexicon or None per page (None: the page decodes as without lexicon).
+        contrast_ths / adjust_contrast: a word whose confidence is below contrast_ths and whose crop's contrast is below
+        adjust_contrast is read again from a contrast-stretched crop and the more confident read is kept (INTEGRATION.md
+        section 10; 0 = off, EasyOCR's readtext uses 0.1 and 0.5)."""
         n = len(images)
         on_dev = n > 0 and not isinstance(images[0], np.ndarray)
         if on_dev:
@@ -361,7 +378,13 @@ class Engine:
         filters = _filters(allowlist, blocklist, n)
         rot = None if rotation_info is None else _rotations(rotation_info)
         lex = _lexicon_arg(lexicon, n, strict=True)
-        if lex is None:
+        if contrast_ths != 0.0 or adjust_contrast != 0.5:
+            handles = None if lex is None else (C.c_void_p * len(lex))(*[None if x is None else x._h.value for x in lex])
+            check(lib().tt_ocr_pages_contrast(self._h, arr, n, C.byref(opt), filters or None, len(filters) if filters else 0,
+                                              rot, len(rot) if rot is not None else 0, handles, len(lex) if lex else 0,
+                                              float(contrast_ths), float(adjust_contrast), C.byref(res)),
+                  "tt_ocr_pages_contrast")
+        elif lex is None:
             check(lib().tt_ocr_pages_oriented(self._h, arr, n, C.byref(opt), filters or None, len(filters) if filters else 0,
                                               rot, len(rot) if rot is not None else 0, C.byref(res)), "tt_ocr_pages_oriented")
         else:
@@ -493,44 +516,54 @@ def _engine_for(weights_dir: str) -> Engine:
 
 
 def image_to_data(image: np.ndarray, weights_dir: str, outputs_dir: str, *, allowlist: str | None = None,
-                  blocklist: str | None = None, rotation_info=None, lexicon=None) -> list[dict]:
+                  blocklist: str | None = None, rotation_info=None, lexicon=None, contrast_ths: float = 0.0,
+                  adjust_contrast: float = 0.5) -> list[dict]:
     """Same call as the reference's ``pytuatara.image_to_data`` (bindings/python.cpp:43-57):
     uint8 [H, W, 3] in, list of ``dict(text=str, bbox=[4 floats])`` out.  Empty directory
     strings print to stderr and return [] like tuatara.cpp:315-323.  allowlist / blocklist: recognition only produces
     characters in allowlist and not in blocklist (INTEGRATION.md section 7).  rotation_info: angles from {90, 180, 270}
     at which each word is also read; items then carry "angle" (INTEGRATION.md section 8).  lexicon: a Lexicon or an
-    iterable of str; every recognised word is one of its words (INTEGRATION.md section 9)."""
+    iterable of str; every recognised word is one of its words (INTEGRATION.md section 9).  contrast_ths /
+    adjust_contrast: low-confidence words on low-contrast crops are read again from a stretched crop (INTEGRATION.md
+    section 10; 0 = off)."""
     return _one_page(image, weights_dir, outputs_dir, allowlist=allowlist, blocklist=blocklist,
-                     rotation_info=rotation_info, lexicon=lexicon)
+                     rotation_info=rotation_info, lexicon=lexicon, contrast_ths=contrast_ths,
+                     adjust_contrast=adjust_contrast)
 
 
 def images_to_data(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".", *, allowlist=None,
-                   blocklist=None, rotation_info=None, lexicon=None) -> list[list[dict]]:
+                   blocklist=None, rotation_info=None, lexicon=None, contrast_ths: float = 0.0,
+                   adjust_contrast: float = 0.5) -> list[list[dict]]:
     """Additive batch API: one call, many pages (sharded over the engine's GPUs).  allowlist / blocklist: None, a str
     for every page, or a list with one str or None per page.  lexicon: a Lexicon or an iterable of str for every page,
     or a list with one entry per page, each None, a Lexicon or an iterable of str."""
     images = list(images)
     return _engine_for(weights_dir).ocr_pages(images, allowlist=allowlist, blocklist=blocklist,
                                               rotation_info=rotation_info,
-                                              lexicon=_engine_lexicon(lexicon, len(images)))
+                                              lexicon=_engine_lexicon(lexicon, len(images)), contrast_ths=contrast_ths,
+                                              adjust_contrast=adjust_contrast)
 
 
 def image_to_data_scored(image: np.ndarray, weights_dir: str, outputs_dir: str, *, allowlist: str | None = None,
-                         blocklist: str | None = None, rotation_info=None, lexicon=None) -> list[dict]:
+                         blocklist: str | None = None, rotation_info=None, lexicon=None, contrast_ths: float = 0.0,
+                         adjust_contrast: float = 0.5) -> list[dict]:
     """image_to_data whose items also carry ``conf`` (word confidence 0..1), ``det_score`` (the detection score of the
     box) and ``char_conf`` (one probability per character of ``text``).  Same inputs, errors and soft failures;
     ``text`` and ``bbox`` are what image_to_data returns."""
     return _one_page(image, weights_dir, outputs_dir, scores=True, allowlist=allowlist, blocklist=blocklist,
-                     rotation_info=rotation_info, lexicon=lexicon)
+                     rotation_info=rotation_info, lexicon=lexicon, contrast_ths=contrast_ths,
+                     adjust_contrast=adjust_contrast)
 
 
 def images_to_data_scored(images: list[np.ndarray], weights_dir: str, outputs_dir: str = ".", *, allowlist=None,
-                          blocklist=None, rotation_info=None, lexicon=None) -> list[list[dict]]:
+                          blocklist=None, rotation_info=None, lexicon=None, contrast_ths: float = 0.0,
+                          adjust_contrast: float = 0.5) -> list[list[dict]]:
     """Batch variant of image_to_data_scored."""
     images = list(images)
     return _engine_for(weights_dir).ocr_pages(images, scores=True, allowlist=allowlist, blocklist=blocklist,
                                               rotation_info=rotation_info,
-                                              lexicon=_engine_lexicon(lexicon, len(images)))
+                                              lexicon=_engine_lexicon(lexicon, len(images)), contrast_ths=contrast_ths,
+                                              adjust_contrast=adjust_contrast)
 
 
 def _one_page(image: np.ndarray, weights_dir: str, outputs_dir: str, **kw) -> list[dict]:

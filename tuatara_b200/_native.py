@@ -75,6 +75,8 @@ SIGNATURES = {
     "tt_lexicon_info": (_I, [_P, _PI, _PI]),
     "tt_ocr_pages_lexicon": (_I, [_P, C.POINTER(tt_image), _I, C.POINTER(tt_ocr_options), C.POINTER(tt_char_filter), _I,
                                   _P, _I, C.POINTER(_P), _I, C.POINTER(C.POINTER(tt_result))]),
+    "tt_ocr_pages_contrast": (_I, [_P, C.POINTER(tt_image), _I, C.POINTER(tt_ocr_options), C.POINTER(tt_char_filter), _I,
+                                   _P, _I, C.POINTER(_P), _I, _F, _F, C.POINTER(C.POINTER(tt_result))]),
     "tt_item_angle": (_I, [C.POINTER(tt_result), _I, _I, _PI]),
     "tt_item_scores": (_I, [C.POINTER(tt_result), _I, _I, _PF, _PF, C.POINTER(_PF), _PI]),
     "tt_launch_count": (C.c_ulonglong, []),
@@ -92,6 +94,7 @@ SIGNATURES = {
     "tt_postprocess": (_I, [_P, _I, _I, C.POINTER(tt_config), _P, _P, _I, _PI, _P, _P, _I, _PI]),
     "tt_crop_resize": (_I, [C.POINTER(tt_image), _P, _I, _P]),
     "tt_crop_resize_rotated": (_I, [C.POINTER(tt_image), _P, _P, _I, _P]),
+    "tt_contrast_adjust": (_I, [_P, _I, _F, _P, _P]),
     "tt_craft_tap": (_I, [_P, C.c_char_p, _P, C.c_longlong, _P]),
     "tt_crop_warp": (_I, [C.POINTER(tt_image), _P, _I, _P]),
     "tt_rect_to_quad": (_I, [_P, _P]),
@@ -121,6 +124,7 @@ SIGNATURES = {
     "tt_dec_self_attn_dev": (_I, [_I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _I, _I, _P, _P]),
     "tt_dec_cross_attn_dev": (_I, [_I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P]),
     "tt_orient_select_dev": (_I, [_P, _P, _I, _P, _I, _P, _P, _P, _P]),
+    "tt_contrast_select_dev": (_I, [_P, _P, _P, _I, _P, _P, _P]),
     "tt_lexicon_walk_dev": (_I, [_P, _P, _I, _P, _P, _P]),
     "tt_postprocess_dev": (_I, [_P, _P, _I, _I, _I, _PI, _P]),
 }

@@ -144,14 +144,16 @@ static py::dict item_to_dict(const tuatara::ScoredItem& item, bool scored, bool 
 // The four functions' one path -> a list of pages of item dicts.  batch: allowlist / blocklist may hold one entry per page.
 static py::list ocr_pages(const std::vector<tuatara::ImageView>& views, bool batch, const std::string& weights_dir,
                           const std::string& output_dir, const py::object& allowlist, const py::object& blocklist,
-                          const py::object& rotation_info, const py::object& lexicon, bool scored) {
+                          const py::object& rotation_info, const py::object& lexicon, float contrast_ths,
+                          float adjust_contrast, bool scored) {
   const FilterArgs fa = filter_args(allowlist, blocklist, views.size(), batch);
   const RotationArgs ra = rotation_args(rotation_info);
   const LexiconArgs la = lexicon_args(lexicon, views.size(), batch);
   std::vector<std::vector<tuatara::ScoredItem>> pages;
   {
     py::gil_scoped_release release;
-    pages = tuatara::detail::ocr_pages(views, weights_dir, output_dir, scored, fa.filters, ra.angles, la.handles);
+    pages = tuatara::detail::ocr_pages(views, weights_dir, output_dir, scored, fa.filters, ra.angles, la.handles,
+                                       tuatara::Contrast{contrast_ths, adjust_contrast});
   }
   py::list result;
   for (const auto& page : pages) {
@@ -165,19 +167,22 @@ static py::list ocr_pages(const std::vector<tuatara::ImageView>& views, bool bat
 // image_to_data / image_to_data_scored: page 0, or [] after a soft failure
 template <bool kScored>
 static py::list image_wrapper(Image image_data, std::string weights_dir, std::string output_dir, py::object allowlist,
-                              py::object blocklist, py::object rotation_info, py::object lexicon) {
+                              py::object blocklist, py::object rotation_info, py::object lexicon, float contrast_ths,
+                              float adjust_contrast) {
   py::list pages = ocr_pages({buffer_to_view(image_data)}, false, weights_dir, output_dir, allowlist, blocklist,
-                             rotation_info, lexicon, kScored);
+                             rotation_info, lexicon, contrast_ths, adjust_contrast, kScored);
   return pages.empty() ? py::list() : py::list(pages[0]);
 }
 
 // images_to_data / images_to_data_scored
 template <bool kScored>
 static py::list images_wrapper(std::vector<Image> images, std::string weights_dir, std::string output_dir,
-                               py::object allowlist, py::object blocklist, py::object rotation_info, py::object lexicon) {
+                               py::object allowlist, py::object blocklist, py::object rotation_info, py::object lexicon,
+                               float contrast_ths, float adjust_contrast) {
   std::vector<tuatara::ImageView> views;
   for (auto& a : images) views.push_back(buffer_to_view(a));
-  return ocr_pages(views, true, weights_dir, output_dir, allowlist, blocklist, rotation_info, lexicon, kScored);
+  return ocr_pages(views, true, weights_dir, output_dir, allowlist, blocklist, rotation_info, lexicon, contrast_ths,
+                   adjust_contrast, kScored);
 }
 
 PYBIND11_MODULE(pytuatara, m) {
@@ -185,20 +190,22 @@ PYBIND11_MODULE(pytuatara, m) {
   // allowlist / blocklist (keyword only): recognition only produces characters in allowlist and not in blocklist.
   // rotation_info (keyword only): angles from {90, 180, 270} at which each word is also read; items then carry "angle".
   // lexicon (keyword only): every recognised word is one of a word list (a tuatara_b200.Lexicon or an iterable of str).
+  // contrast_ths / adjust_contrast (keyword only): a word read with a confidence below contrast_ths from a crop whose
+  // contrast is below adjust_contrast is read again from a contrast-stretched crop (0 = off; EasyOCR uses 0.1 / 0.5).
   m.def("image_to_data", &image_wrapper<false>, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"), py::kw_only(),
         py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
-        py::arg("lexicon") = py::none(),
+        py::arg("lexicon") = py::none(), py::arg("contrast_ths") = 0.0f, py::arg("adjust_contrast") = 0.5f,
         "Extract text and bounding boxes from an image");
   m.def("images_to_data", &images_wrapper<false>, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"), py::kw_only(),
         py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
-        py::arg("lexicon") = py::none(),
+        py::arg("lexicon") = py::none(), py::arg("contrast_ths") = 0.0f, py::arg("adjust_contrast") = 0.5f,
         "Batch variant: list of images -> list of per-page results");
   m.def("image_to_data_scored", &image_wrapper<true>, py::arg("image"), py::arg("weights_dir"), py::arg("outputs_dir"),
         py::kw_only(), py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
-        py::arg("lexicon") = py::none(),
+        py::arg("lexicon") = py::none(), py::arg("contrast_ths") = 0.0f, py::arg("adjust_contrast") = 0.5f,
         "image_to_data whose items also carry conf (word confidence 0..1, None when not recognised), det_score and char_conf");
   m.def("images_to_data_scored", &images_wrapper<true>, py::arg("images"), py::arg("weights_dir"), py::arg("outputs_dir"),
         py::kw_only(), py::arg("allowlist") = py::none(), py::arg("blocklist") = py::none(), py::arg("rotation_info") = py::none(),
-        py::arg("lexicon") = py::none(),
+        py::arg("lexicon") = py::none(), py::arg("contrast_ths") = 0.0f, py::arg("adjust_contrast") = 0.5f,
         "Batch variant of image_to_data_scored");
 }

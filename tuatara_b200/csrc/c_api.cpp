@@ -3,11 +3,14 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
+#include <cstdio>
 #include <cstring>
 #include <string>
 #include <vector>
 
 #include "common.h"
+#include "contrast.cuh"
 #include "detect.h"
 #include "enc_mlp.cuh"
 #include "enc_qkv_attn.cuh"
@@ -276,6 +279,42 @@ int tt_crop_warp(const tt_image* image, const float* quads, int n, uint8_t* out)
   });
 }
 
+int tt_contrast_adjust(const uint8_t* crops, int n, float adjust_contrast, uint8_t* out, int32_t* stretched) {
+  return guarded([&]() -> int {
+    if (!std::isfinite(adjust_contrast) || !(adjust_contrast > 0.f) || adjust_contrast > 1.f) {
+      char v[32];
+      std::snprintf(v, sizeof v, "%g", adjust_contrast);
+      set_error(std::string("tt_contrast_adjust: adjust_contrast is ") + v + "; it must be finite and in (0, 1]");
+      return 1;
+    }
+    if (n < 0 || (n > 0 && (!crops || !out))) { set_error("tt_contrast_adjust: null crops or output, or n < 0"); return 1; }
+    if (n == 0) return 0;
+    const size_t bytes = static_cast<size_t>(n) * 32 * 128 * 3;
+    DevBuf din, dpatch, dflag, dlr, dlist, dcount, dout;
+    TT_CUDA_INT(din.alloc(bytes));
+    TT_CUDA_INT(dout.alloc(bytes));
+    TT_CUDA_INT(dpatch.alloc(static_cast<size_t>(n) * 128 * 96 * sizeof(__nv_bfloat16)));
+    TT_CUDA_INT(dflag.alloc(sizeof(int) * n));
+    TT_CUDA_INT(dlr.alloc(sizeof(double2) * n));
+    TT_CUDA_INT(dlist.alloc(sizeof(int) * n));
+    TT_CUDA_INT(dcount.alloc(sizeof(int)));
+    TT_CUDA_INT(cudaMemcpy(din.p, crops, bytes, cudaMemcpyHostToDevice));
+    TT_CUDA_INT(cudaMemcpy(dout.p, din.p, bytes, cudaMemcpyDeviceToDevice));   // crops that are not stretched stay as given
+    const OrientSet upright{1, {0, 0, 0, 0}};
+    TT_TRY_INT(patchify_u8(din.as<uint8_t>(), n, dpatch.as<__nv_bfloat16>(), 0));
+    TT_TRY_INT(contrast_stats(nullptr, nullptr, n, TT_MAX_LABEL_LEN, 0.f, adjust_contrast, dpatch.as<__nv_bfloat16>(), 1,
+                              nullptr, upright, dflag.as<int>(), dlr.as<double2>(), 0));
+    TT_TRY_INT(contrast_compact(dflag.as<int>(), n, dlist.as<int>(), dcount.as<int>(), 0));
+    int m = 0;
+    TT_CUDA_INT(cudaMemcpy(&m, dcount.p, sizeof(int), cudaMemcpyDeviceToHost));
+    TT_TRY_INT(contrast_apply(dlist.as<int>(), m, dpatch.as<__nv_bfloat16>(), 1, nullptr, upright, dlr.as<double2>(), nullptr,
+                              dout.as<uint8_t>(), nullptr, nullptr, nullptr, nullptr, 0));
+    TT_CUDA_INT(cudaMemcpy(out, dout.p, bytes, cudaMemcpyDeviceToHost));
+    if (stretched) TT_CUDA_INT(cudaMemcpy(stretched, dflag.p, sizeof(int) * n, cudaMemcpyDeviceToHost));
+    return 0;
+  });
+}
+
 int tt_rect_to_quad(const float rect[5], float quad_out[8]) {
   return guarded([&]() -> int {
     Pt2f q[4];
@@ -508,6 +547,18 @@ int tt_orient_select_dev(const int32_t* ids, const float* pmax, int n_words, con
     for (int r = 0; r < n_candidates; ++r) set.angle[r] = angles[r];
     return orient_select(ids, pmax, n_words, TT_MAX_LABEL_LEN, set, ids_out, pmax_out, angle_out,
                          static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : 1;
+  });
+}
+
+int tt_contrast_select_dev(int32_t* ids, float* pmax, const int32_t* list, int n_listed, const int32_t* ids2, const float* pmax2,
+                           void* stream) {
+  return guarded([&]() -> int {
+    if (n_listed < 0 || (n_listed > 0 && (!ids || !pmax || !list || !ids2 || !pmax2))) {
+      set_error("tt_contrast_select_dev: null argument or n_listed < 0");
+      return 1;
+    }
+    return contrast_select(ids, pmax, TT_MAX_LABEL_LEN, list, n_listed, ids2, pmax2, static_cast<cudaStream_t>(stream)) ==
+                   cudaSuccess ? 0 : 1;
   });
 }
 

@@ -8,11 +8,14 @@
 #include <atomic>
 #include <map>
 #include <tuple>
+#include <cmath>
+#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <thread>
 
 #include "common.h"
+#include "contrast.cuh"
 #include "gemm_tc.cuh"
 #include "lexicon.h"
 #include "nn_kernels.cuh"
@@ -126,6 +129,8 @@ struct Request {
   std::vector<int> roots;                    // the root state of every page's automaton
   std::vector<uint32_t> lex_table;           // the request's automata, LexTableBuilder::words()
   int lex_states = 0;                        //   its number of states
+  float contrast_ths = 0.f;                  // the contrast re-read (INTEGRATION.md section 10); 0 = off
+  float adjust_contrast = 0.5f;
 };
 
 // The request's automaton table in the slot's lex_buf, uploaded at most once per slot per request; -> its device view.
@@ -309,6 +314,78 @@ int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const
   return 0;
 }
 
+// The contrast re-read's per-pass buffers in the arena, below the first read's end (so the second forward leaves them).
+struct ContrastBufs {
+  int* ids = nullptr;           // R == 1: the first read's ids [nw][L] (with R > 1 orient_select's output is kept)
+  int* flag = nullptr;          // [nw]
+  double2* lr = nullptr;        // [nw] (low, ratio)
+  int* list = nullptr;          // [nw] the words read again
+  int* count = nullptr;         //   their number
+  __nv_bfloat16* patches = nullptr;   // [nw * 128][96] their stretched crops
+  float* p2 = nullptr;          // [nw][L] the second read's pmax
+  uint32_t* mask = nullptr;     // [nw][4] with filters
+  int* root = nullptr;          // [nw] with lexicons, and as many walk states
+  int* state = nullptr;
+  int get(Arena& a, int nw, int L, bool own_ids, bool masked, bool lexed) {
+    const size_t n = static_cast<size_t>(nw);
+    if (own_ids) ids = a.get<int>(n * L);
+    flag = a.get<int>(n);
+    lr = a.get<double2>(n);
+    list = a.get<int>(n);
+    count = a.get<int>(1);
+    patches = a.get<__nv_bfloat16>(n * 128 * 96);
+    p2 = a.get<float>(n * L);
+    if (masked) mask = a.get<uint32_t>(4 * n);
+    if (lexed) {
+      root = a.get<int>(n);
+      state = a.get<int>(n);
+    }
+    if ((own_ids && !ids) || !flag || !lr || !list || !count || !patches || !p2 || (masked && !mask) ||
+        (lexed && (!root || !state))) {
+      set_error("arena exhausted (contrast)");
+      return 1;
+    }
+    return 0;
+  }
+};
+
+// The contrast re-read of one pass (INTEGRATION.md section 10): ids / pmax [nw][L] hold the first read of every word (the
+// winner of its candidates; angle [nw] its angle, null without rotation candidates) and end up holding the kept read.
+// mask / lex: the first forward's per-crop class masks or lexicon roots (null without).
+int reread_contrast(DeviceCtx& d, const Request& req, const __nv_bfloat16* patches, int nw, const int* angle,
+                    const uint32_t* mask, const LexDev* lex, const ContrastBufs& cb, size_t first_read_end, int* ids,
+                    float* pmax) {
+  const int L = d.w->pd.L, R = req.orient.n;
+  stage_begin(d.stream);
+  E_TRY(contrast_stats(ids, pmax, nw, L, req.contrast_ths, req.adjust_contrast, patches, R, angle, req.orient, cb.flag, cb.lr,
+                       d.stream));
+  E_TRY(contrast_compact(cb.flag, nw, cb.list, cb.count, d.stream));
+  E_CUDA(cudaMemcpyAsync(d.pinned, cb.count, sizeof(int), cudaMemcpyDeviceToHost, d.stream));
+  stage_end(d.stream, "contrast_stats", 0.0, static_cast<double>(nw) * (L * 8 + 16));
+  g_d2h_bytes += sizeof(int);
+  E_TRY(stream_sync(d.stream));
+  const int m = *reinterpret_cast<const int*>(d.pinned);
+  if (m == 0) return 0;
+  stage_begin(d.stream);
+  E_TRY(contrast_apply(cb.list, m, patches, R, angle, req.orient, cb.lr, cb.patches, nullptr, mask, cb.mask,
+                       lex ? lex->root : nullptr, cb.root, d.stream));
+  stage_end(d.stream, "contrast_apply", 0.0, static_cast<double>(m) * 128 * 96 * 4);
+  d.arena.reset_to(first_read_end);
+  LexDev lx2{};
+  if (lex) {
+    lx2 = *lex;
+    lx2.root = cb.root;
+    lx2.state = cb.state;
+  }
+  float* logits = nullptr;
+  int* ids2 = nullptr;
+  E_TRY(d.parseq_forward(cb.patches, m, nullptr, &logits, &ids2, cb.p2, mask ? cb.mask : nullptr, lex ? &lx2 : nullptr));
+  stage_begin(d.stream);
+  E_TRY(contrast_select(ids, pmax, L, cb.list, m, ids2, cb.p2, d.stream));
+  stage_end(d.stream, "contrast_select", 0.0, static_cast<double>(m) * L * 16);
+  return 0;
+}
+
 // PARSeq + tokenizer over the slot's recognition batch (tuatara.cpp:450-505), which holds R = req.orient.n crops per
 // word.  A pass takes whole words (at most kMaxCropsPerPass crops).  With scores the refinement head also writes each
 // position's largest softmax probability, copied back next to the ids and decoded into conf / char_conf.  With
@@ -316,7 +393,10 @@ int detect_unit(DeviceCtx& d, const tt_config& cfg, const tt_image* pages, const
 // the copy back is the same ids (and pmax with scores) per word plus its 4-byte angle.  With filters (req.masks) each
 // crop decodes under its page's class mask, uploaded per pass as [nc][4] words.  With lexicons (req.roots) each crop
 // walks its page's automaton instead: the table goes to the slot once per request (*lex_ready), the crops' roots with
-// each pass as [nc] words.
+// each pass as [nc] words.  With the contrast re-read (req.contrast_ths > 0) the refinement head always writes pmax, and
+// after the first read (and orient_select) the contrast kernels pick the low-confidence, low-contrast words on the device;
+// the host reads their 4-byte count, runs PARSeq once more on their stretched crops, and contrast_select leaves the more
+// confident read in the per-word ids / pmax, which then go back as without it.
 int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, const Request& req, bool* lex_ready) {
   const int n = static_cast<int>(pend->owner.size());
   const bool lexed = !req.roots.empty();
@@ -328,17 +408,24 @@ int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, const 
   if (lexed) lx = d.lex_view;
   const int L = d.w->pd.L, R = req.orient.n;
   const bool scores = req.opt.with_scores != 0;
+  const bool contrast = req.contrast_ths > 0.f;
   const int words_per_pass = kMaxCropsPerPass / R;
   for (int w0 = 0; w0 < n; w0 += words_per_pass) {
     const int nw = std::min(words_per_pass, n - w0);
     const int nc = nw * R;
     const size_t bytes = sizeof(int) * static_cast<size_t>(nw) * L;   // ids per word; with scores as many bytes of pmax
     const size_t angle_bytes = R > 1 ? sizeof(int) * static_cast<size_t>(nw) : 0;
-    const size_t pmax_bytes = scores || R > 1 ? sizeof(float) * static_cast<size_t>(nc) * L : 0;
+    const size_t pmax_bytes = scores || R > 1 || contrast ? sizeof(float) * static_cast<size_t>(nc) * L : 0;
     const size_t mask_bytes = req.masks.empty() ? 0 : sizeof(ClassMask) * nc;
     const size_t root_bytes = lexed ? sizeof(int) * static_cast<size_t>(nc) : 0;   // and as many for the walk state
+    // contrast: the first read's ids (R == 1), flag, (low, ratio), list, count, the second batch's patch rows, its pmax,
+    // class masks and roots / walk states -- at most nw words, so the second forward fits in parseq_bytes(nc)
+    const size_t contrast_bytes =
+        contrast ? (R == 1 ? bytes : 0) + static_cast<size_t>(nw) * (4 + 16 + 4 + 128 * 96 * 2 + 4 * L) + 4 +
+                       (req.masks.empty() ? 0 : sizeof(ClassMask) * nw) + (lexed ? 8 * static_cast<size_t>(nw) : 0)
+                 : 0;
     const size_t need = d.parseq_bytes(nc) + (4u << 20) + pmax_bytes + (R > 1 ? 2 * bytes + angle_bytes : 0) + mask_bytes +
-                        2 * root_bytes;
+                        2 * root_bytes + contrast_bytes;
     if (need > d.arena.capacity()) E_TRY(stream_sync(d.stream));
     E_TRY(d.arena.reserve(need));
     d.arena.reset();
@@ -374,16 +461,28 @@ int recognise(DeviceCtx& d, std::vector<PageOut>* results, Pending* pend, const 
       g_h2d_bytes += root_bytes;
       lx.root = roots;
     }
+    ContrastBufs cb{};
+    if (contrast && cb.get(d.arena, nw, L, R == 1, !req.masks.empty(), lexed)) return 1;
+    const size_t first_read_end = d.arena.offset();   // the second forward reuses the arena from here
+    const __nv_bfloat16* patches = d.patch_buf + static_cast<size_t>(w0) * R * 128 * 96;
     float* logits = nullptr;
     int* ids = nullptr;
-    E_TRY(d.parseq_forward(d.patch_buf + static_cast<size_t>(w0) * R * 128 * 96, nc, nullptr, &logits, &ids, pmax, mask,
-                           lexed ? &lx : nullptr));
+    E_TRY(d.parseq_forward(patches, nc, nullptr, &logits, &ids, pmax, mask, lexed ? &lx : nullptr));
     if (R > 1) {
       stage_begin(d.stream);
-      E_TRY(orient_select(ids, pmax, nw, L, req.orient, win_ids, scores ? win_p : nullptr, win_angle, d.stream));
+      E_TRY(orient_select(ids, pmax, nw, L, req.orient, win_ids, scores || contrast ? win_p : nullptr, win_angle, d.stream));
       stage_end(d.stream, "orient_select", 0.0, static_cast<double>(nc) * L * 8 + static_cast<double>(nw) * (L * 8 + 4));
       ids = win_ids;
       pmax = win_p;
+    }
+    if (contrast) {
+      if (R == 1) {   // the first read's ids live in the forward's arena space, which the second forward reuses
+        E_CUDA(cudaMemcpyAsync(cb.ids, ids, bytes, cudaMemcpyDeviceToDevice, d.stream));
+        ids = cb.ids;
+      }
+      if (reread_contrast(d, req, patches, nw, R > 1 ? win_angle : nullptr, mask, lexed ? &lx : nullptr, cb,
+                          first_read_end, ids, pmax))
+        return 1;
     }
     E_CUDA(cudaMemcpyAsync(d.pinned, ids, bytes, cudaMemcpyDeviceToHost, d.stream));
     if (R > 1) E_CUDA(cudaMemcpyAsync(d.pinned + bytes, win_angle, angle_bytes, cudaMemcpyDeviceToHost, d.stream));
@@ -456,12 +555,31 @@ void slot_worker(tt_engine& e, int g, int sidx, int want, const tt_image* pages,
   if (recognise(d, results, &pend, req, &lex_ready)) { *err = last_error(); *rc = 1; return; }
 }
 
+// The last check of make_request: the contrast re-read's two values.
+int set_contrast(const char* fn, float contrast_ths, float adjust_contrast, Request* req) {
+  char v[32];
+  if (!std::isfinite(contrast_ths) || contrast_ths < 0.f) {
+    std::snprintf(v, sizeof v, "%g", contrast_ths);
+    set_error(std::string(fn) + ": contrast_ths is " + v + "; it must be finite and >= 0");
+    return 1;
+  }
+  if (!std::isfinite(adjust_contrast) || !(adjust_contrast > 0.f) || adjust_contrast > 1.f) {
+    std::snprintf(v, sizeof v, "%g", adjust_contrast);
+    set_error(std::string(fn) + ": adjust_contrast is " + v + "; it must be finite and in (0, 1]");
+    return 1;
+  }
+  req->contrast_ths = contrast_ths;
+  req->adjust_contrast = adjust_contrast;
+  return 0;
+}
+
 // The argument checks of the tt_ocr_pages* entry points (fn: the one called, named in the messages), made before any
 // device work: the rotation candidates, then the filters, turned into one class mask per page, then the lexicons, turned
-// into one automaton per page with the page's filter folded in.  ocr_pages checks the engine and the pages.
+// into one automaton per page with the page's filter folded in, then the contrast values.  ocr_pages checks the engine
+// and the pages.
 int make_request(const char* fn, const tt_ocr_options* opt, const tt_char_filter* filters, int n_filters,
-                 const int* rotation_info, int n_rotations, const tt_lexicon* const* lexicons, int n_lexicons, int n_pages,
-                 Request* req) {
+                 const int* rotation_info, int n_rotations, const tt_lexicon* const* lexicons, int n_lexicons,
+                 float contrast_ths, float adjust_contrast, int n_pages, Request* req) {
   try {
     if (opt) req->opt = *opt;
     if (n_rotations < 0 || (n_rotations > 0 && !rotation_info)) {
@@ -494,7 +612,7 @@ int make_request(const char* fn, const tt_ocr_options* opt, const tt_char_filter
         char_filter_mask(f.allow, f.block, req->masks[i].data());
       }
     }
-    if (n_lexicons == 0) return 0;
+    if (n_lexicons == 0) return set_contrast(fn, contrast_ths, adjust_contrast, req);
     if (!lexicons) { set_error(std::string(fn) + ": lexicons is NULL but n_lexicons is " + std::to_string(n_lexicons)); return 1; }
     if (n_lexicons != 1 && n_lexicons != n_pages) {
       set_error(std::string(fn) + ": n_lexicons must be 0, 1 or n_pages (" + std::to_string(n_pages) + "), got " +
@@ -535,7 +653,7 @@ int make_request(const char* fn, const tt_ocr_options* opt, const tt_char_filter
     req->lex_table = table.words();
     req->lex_states = table.n_states();
     req->masks.clear();
-    return 0;
+    return set_contrast(fn, contrast_ths, adjust_contrast, req);
   } catch (const std::exception& ex) {
     set_error(std::string(fn) + ": " + ex.what());
     return 1;
@@ -639,14 +757,14 @@ int tt_ocr_pages(tt_engine* e, const tt_image* pages, int n_pages, tt_result** o
 
 int tt_ocr_pages_ex(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt, tt_result** out) {
   Request req;
-  return make_request("tt_ocr_pages_ex", opt, nullptr, 0, nullptr, 0, nullptr, 0, n_pages, &req)
+  return make_request("tt_ocr_pages_ex", opt, nullptr, 0, nullptr, 0, nullptr, 0, 0.f, 0.5f, n_pages, &req)
              ? 1 : ocr_pages(e, pages, n_pages, req, out);
 }
 
 int tt_ocr_pages_filtered(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
                           const tt_char_filter* filters, int n_filters, tt_result** out) {
   Request req;
-  return make_request("tt_ocr_pages_filtered", opt, filters, n_filters, nullptr, 0, nullptr, 0, n_pages, &req)
+  return make_request("tt_ocr_pages_filtered", opt, filters, n_filters, nullptr, 0, nullptr, 0, 0.f, 0.5f, n_pages, &req)
              ? 1 : ocr_pages(e, pages, n_pages, req, out);
 }
 
@@ -654,7 +772,8 @@ int tt_ocr_pages_oriented(tt_engine* e, const tt_image* pages, int n_pages, cons
                           const tt_char_filter* filters, int n_filters, const int* rotation_info, int n_rotations,
                           tt_result** out) {
   Request req;
-  return make_request("tt_ocr_pages_oriented", opt, filters, n_filters, rotation_info, n_rotations, nullptr, 0, n_pages, &req)
+  return make_request("tt_ocr_pages_oriented", opt, filters, n_filters, rotation_info, n_rotations, nullptr, 0, 0.f, 0.5f,
+                      n_pages, &req)
              ? 1 : ocr_pages(e, pages, n_pages, req, out);
 }
 
@@ -663,7 +782,17 @@ int tt_ocr_pages_lexicon(tt_engine* e, const tt_image* pages, int n_pages, const
                          const tt_lexicon* const* lexicons, int n_lexicons, tt_result** out) {
   Request req;
   return make_request("tt_ocr_pages_lexicon", opt, filters, n_filters, rotation_info, n_rotations, lexicons, n_lexicons,
-                      n_pages, &req)
+                      0.f, 0.5f, n_pages, &req)
+             ? 1 : ocr_pages(e, pages, n_pages, req, out);
+}
+
+int tt_ocr_pages_contrast(tt_engine* e, const tt_image* pages, int n_pages, const tt_ocr_options* opt,
+                          const tt_char_filter* filters, int n_filters, const int* rotation_info, int n_rotations,
+                          const tt_lexicon* const* lexicons, int n_lexicons, float contrast_ths, float adjust_contrast,
+                          tt_result** out) {
+  Request req;
+  return make_request("tt_ocr_pages_contrast", opt, filters, n_filters, rotation_info, n_rotations, lexicons, n_lexicons,
+                      contrast_ths, adjust_contrast, n_pages, &req)
              ? 1 : ocr_pages(e, pages, n_pages, req, out);
 }
 

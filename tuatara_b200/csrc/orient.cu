@@ -1,6 +1,7 @@
 #include "orient.cuh"
 
 #include "common.h"
+#include "word_conf.cuh"
 
 namespace tt {
 
@@ -15,12 +16,7 @@ __global__ void __launch_bounds__(128) k_orient_select(const int* __restrict__ i
   float best_conf = 0.f;
   for (int r = 0; r < set.n; ++r) {
     const size_t row = (static_cast<size_t>(w) * set.n + r) * L;
-    int end = L - 1;
-    for (int t = 0; t < L; ++t)
-      if (ids[row + t] == 0) { end = t; break; }
-    double prod = 1.0;
-    for (int t = 0; t <= end; ++t) prod = __dmul_rn(prod, static_cast<double>(pmax[row + t]));
-    const float conf = __double2float_rn(prod);
+    const float conf = word_conf(ids + row, pmax + row, L);
     if (r == 0 || conf > best_conf) { best = r; best_conf = conf; }
   }
   const size_t src = (static_cast<size_t>(w) * set.n + best) * L, dst = static_cast<size_t>(w) * L;
